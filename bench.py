@@ -4,6 +4,7 @@ one 15 s slot = 36 M complex samples through the full CIC+FIR decimation and FT8
 
   python bench.py --gpus N --steps K --warmup W                     this repository's CUDA path (one process per GPU)
   python bench.py --impl reference --gpus N --steps K --warmup W    the reference's own CPU implementation, all host cores
+  python bench.py ... --dump-outputs DIR                            + the spot records of the last timed step as DIR/*.npy
 
 A "step" is one pass of the whole hot path (decimate -> condition -> waterfall -> Costas sync/top-K ->
 LLR/LDPC/CRC/unpack -> spot table) over one batch of synthetic slots.  `value` times it with the batch already
@@ -378,6 +379,34 @@ def records_equal(a, b) -> bool:
     return bool(np.array_equal(np.asarray(a[1]), np.asarray(b[1])) and np.asarray(a[0]).tobytes() == np.asarray(b[0]).tobytes())
 
 
+DUMP_MAX_BYTES = 64_000_000   # all files together, .npy headers included
+DUMP_HEADER_BYTES = 256       # allowance per .npy header (numpy writes 128 bytes for these arrays)
+
+
+def dump_outputs(path: str, res, nres, result_dtype):
+    """Write what the caller of the timed path received in its last step -- per slot, the spot count and the decoder_results
+    records -- as float arrays under `path`, so two builds can be compared output for output on the same inputs.  Records past
+    a slot's count carry no result and are written as zeros.  Text fields are written one float32 per byte.  Where all slots
+    would not fit in DUMP_MAX_BYTES a fixed, seeded sample of slots is written; slot_index.npy names the slots either way."""
+    res = np.asarray(res).view(result_dtype)
+    nres = np.asarray(nres, np.int64)
+    n_slots, m = res.shape
+    slot_bytes = m * (8 + 8 + 4 * (result_dtype["call"].itemsize + result_dtype["loc"].itemsize)) + 16
+    budget = DUMP_MAX_BYTES - 6 * DUMP_HEADER_BYTES   # six files
+    idx = np.arange(n_slots)
+    if n_slots * slot_bytes > budget:
+        idx = np.sort(np.random.default_rng(0).choice(n_slots, budget // slot_bytes, replace=False))
+    res, nres = res[idx].copy(), nres[idx]
+    res[np.arange(m)[None, :] >= nres[:, None]] = np.zeros((), result_dtype)
+    os.makedirs(path, exist_ok=True)
+    arrays = {"slot_index": idx.astype(np.float64), "n_results": nres.astype(np.float64),
+              "freq": res["freq"].astype(np.float64), "snr": res["snr"].astype(np.float64)}
+    for name in ("call", "loc"):
+        arrays[name] = np.ascontiguousarray(res[name]).view(np.uint8).reshape(res.shape + (-1,)).astype(np.float32)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 # --------------------------------------------------------------------------------------------- main
 def main():
     ap = argparse.ArgumentParser()
@@ -399,7 +428,12 @@ def main():
                                                           "(records gathered by the library's own NCCL all-gather); not launched under torchrun")
     ap.add_argument("--chain-back", action="store_true", help="A/B: with an SM partition, back ends of consecutive batches run one at a time (ft8b200_pipe_set_back_chain)")
     ap.add_argument("--no-configs", action="store_true", help="skip the other BASELINE configurations (configs, e2e_slots, roofline_extra)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the spot records of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.cluster):
+        ap.error("--dump-outputs applies to the CUDA arm without --cluster")
     args.warmup = max(args.warmup, 3)
     # stdout carries exactly ONE line, the JSON: anything a library prints to fd 1 on the way (NCCL's version banner at
     # communicator creation, for one) is sent to stderr, and the JSON line is written to the original stdout at the end
@@ -493,10 +527,12 @@ def main():
     time.sleep(0.3)
     pipe.set_profiling(True)
     launches0 = pipe.launches()
-    ms, _, (t_wall0, t_wall1) = env.timed(lambda k: run_steps(env, pipe, submit_dev, k, args.chunks, Bc, gather), args.steps)
+    ms, last_step, (t_wall0, t_wall1) = env.timed(lambda k: run_steps(env, pipe, submit_dev, k, args.chunks, Bc, gather), args.steps)
     launches = pipe.launches() - launches0
     stage_acc, n_prof = pipe.stage_times()
     pipe.set_profiling(False)
+    if args.dump_outputs and rank == 0 and last_step is not None:
+        dump_outputs(args.dump_outputs, *last_step, pkg.result_dtype)
     value = world * B * args.steps / (ms * 1e-3)
     clocks = sampler.summary(t_wall0, t_wall1)
 

@@ -55,6 +55,17 @@ def _ptr(a, t=C.c_void_p):
     return a.ctypes.data_as(t)
 
 
+def reference_dir() -> str:
+    """Where oracle/Makefile looks for the reference's sources: $REF, else the Makefile's default."""
+    if os.environ.get("REF"):
+        return os.environ["REF"]
+    with open(os.path.join(HERE, "Makefile")) as f:
+        for line in f:
+            if line.startswith("REF") and "?=" in line:
+                return line.split("?=", 1)[1].strip()
+    raise RuntimeError("oracle/Makefile sets no REF")
+
+
 def build_restatement(force: bool = False) -> str:
     so = os.path.join(HERE, "libft8oracle.so")
     srcs = [os.path.join(HERE, f) for f in ("ft8_oracle.c", "ft8_oracle_codec.c", "ft8_oracle_synth.c", "ft8_oracle_report.c", "ft8_oracle.h", "ft8_tables.h")]

@@ -1,18 +1,20 @@
 """INTEGRATION.md, verified: the reference's own daemon (rtlsdr_ft8d.c) and ft8_lib's example decoder (decode_ft8.c), patched
 exactly as INTEGRATION.md sections 1 and 2 describe (tools/patch_reference_daemon.py, in a temp directory), compile against
 include/ft8b200.h NEXT TO the reference's own headers and link against libft8b200.so with the hot-path objects (decode.o, ldpc.o,
-unpack.o, kiss_fft) left out.  Needs /root/reference (build container only); nothing of it is copied into the repository."""
+unpack.o, kiss_fft) left out.  Needs the reference's sources where oracle/Makefile's REF points; nothing of them is copied into the repository."""
 import os
 import subprocess
 import sys
 
 import pytest
 
+from oracle.pyoracle import reference_dir
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+REF = reference_dir()
 LIBDIR = os.path.join(ROOT, "rtlsdr-ft8d_b200")
 
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "ft8_lib")), reason="the reference tree is only present in the build container")
+pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "ft8_lib")), reason="the reference's sources are not present (oracle/Makefile REF)")
 
 
 @pytest.fixture(scope="module")

@@ -1,22 +1,24 @@
-"""Pins the CPU restatement (oracle/ft8_oracle*.c) against the UNMODIFIED reference compiled from /root/reference
+"""Pins the CPU restatement (oracle/ft8_oracle*.c) against the UNMODIFIED reference compiled from its sources
 (oracle/_ref/libref_*.so, `make -C oracle ref`).  Skipped where the reference build is absent (the committed golden
 fixtures in tests/golden/ cover that case: tests/test_oracle_golden.py)."""
 import numpy as np
 import pytest
 
-from conftest import bits_equal
+from conftest import bits_equal, golden
 from oracle.pyoracle import Reference, ReferenceMonitor, cand_dtype
 from tools import ft8enc, synth
 
-pytestmark = pytest.mark.skipif(not (Reference.available("k120") and Reference.available("k500") and ReferenceMonitor.available()),
-                                reason="oracle/_ref not built (needs /root/reference)")
+needs_reference = pytest.mark.skipif(not (Reference.available("k120") and Reference.available("k500") and ReferenceMonitor.available()),
+                                     reason="oracle/_ref not built (make -C oracle ref needs the reference's sources)")
 
 
+@needs_reference
 def test_reference_selftest_runs():
     """decoderSelfTest() (rtlsdr_ft8d.c:913-972): the reference decodes its own 'CQ K1JT FN20QI' signal."""
     assert Reference("k120").lib.ref_selftest() == 1
 
 
+@needs_reference
 def test_decimator_streaming_vs_rtlsdr_callback(oracle):
     ref = Reference("k120", fresh=True)
     rng = np.random.default_rng(3)
@@ -37,6 +39,7 @@ def test_decimator_streaming_vs_rtlsdr_callback(oracle):
     assert bits_equal(ri[:n], i_s) and bits_equal(rq[:n], q_s)
 
 
+@needs_reference
 def test_buffer_stops_at_48000_but_filter_keeps_running(oracle):
     """rtlsdr_ft8d.c:196-200: outputs beyond 48000 are dropped; after the flip the state continues."""
     ref = Reference("k120", fresh=True)
@@ -63,6 +66,7 @@ def test_buffer_stops_at_48000_but_filter_keeps_running(oracle):
     assert n == more.size and bits_equal(ri[:n], more)
 
 
+@needs_reference
 @pytest.mark.parametrize("variant,n_sig,seed", [("k120", 1, 7), ("k120", 25, 5), ("k500", 60, 99), ("k120", 60, 1234), ("k120", 0, 11)])
 def test_subsystem_all_taps(oracle, variant, n_sig, seed):
     ref = Reference(variant)
@@ -86,6 +90,7 @@ def test_subsystem_all_taps(oracle, variant, n_sig, seed):
         assert d["msg"].tobytes() == r["dec_msg"][k].tobytes()
 
 
+@needs_reference
 def test_find_sync_on_random_waterfalls(oracle):
     """Heap eviction and tie-breaking paths: random bytes make thousands of positions pass min_score."""
     ref = Reference("k120")
@@ -95,6 +100,7 @@ def test_find_sync_on_random_waterfalls(oracle):
         assert np.array_equal(oracle.find_sync(mag, k, ms), ref.find_sync(mag, k, ms).view(cand_dtype))
 
 
+@needs_reference
 def test_bp_decode_fuzz(oracle):
     ref = Reference("k120")
     rng = np.random.default_rng(6)
@@ -111,6 +117,7 @@ def test_bp_decode_fuzz(oracle):
         assert eo == er and np.array_equal(po, pr)
 
 
+@needs_reference
 def test_unpack77_fuzz(oracle):
     """All message types the reference unpacks (0.0 free text, 0.5 telemetry, 1/2 standard, 4 nonstandard) + rejects."""
     ref = Reference("k120")
@@ -132,6 +139,7 @@ def test_unpack77_fuzz(oracle):
         assert oracle.unpack77(bytes(a)) == ref.unpack77(bytes(a))
 
 
+@needs_reference
 def test_unpack77_stratified_vs_reference(oracle):
     """tools/synth.py::payload_fuzz (the generator the GPU tests use for the device unpacker): every token class, flag, report
     form and reject path -- oracle == reference on 60 000 payloads."""
@@ -144,6 +152,7 @@ def test_unpack77_stratified_vs_reference(oracle):
         assert rc_o == rc_r and (rc_r < 0 or t_o == t_r), (lab, b.hex(), rc_o, t_o, rc_r, t_r)
 
 
+@needs_reference
 def test_spots_vs_reference_loop(oracle):
     """The duplicate table / CQ filter restated in orc_spots() against the reference's OWN loop (ft8_subsystem, rtlsdr_ft8d.c:
     1452-1523) fed hand-made candidates and ft8_decode() answers through the scripted taps of oracle/ref_harness.c: 2-token CQ
@@ -176,6 +185,7 @@ def test_spots_vs_reference_loop(oracle):
         assert n == o["n"] and res.tobytes() == o["results"].tobytes(), texts
 
 
+@needs_reference
 def test_gfsk_twin_vs_reference_synth_gfsk(oracle):
     """The synthesiser's GFSK mode (integer pulse table, closed-form phase; oracle/ft8_oracle_synth.c is the bit-identical twin
     of csrc/synth.cu) against ft8_lib's own synth_gfsk() (gen_ft8.c:49-102) at the same sample rate: the quadrature rail of the
@@ -205,6 +215,7 @@ def test_gfsk_twin_vs_reference_synth_gfsk(oracle):
     assert abs(float(p8.sum()) - 512.0) < 0.5 and abs(float(p4.sum()) - 576.0) < 0.5   # a pulse integrates to one symbol of deviation
 
 
+@needs_reference
 def test_oracle_pack77_vs_reference(oracle):
     """The restated pack77() (oracle/ft8_oracle_codec.c) against the reference's on 20 000 message texts."""
     ref = Reference("k120")
@@ -212,6 +223,7 @@ def test_oracle_pack77_vs_reference(oracle):
         assert oracle.pack77(m)[0] == ref.pack77(m), repr(m)
 
 
+@needs_reference
 def test_library_pack77_vs_reference(pkg):
     """ft8b200_pack77 (host code of the library) against the reference's own pack77() (pack.c:284-301) on 20 000 message texts:
     standard / free-text choice and every payload byte, quirks included ("FN20QI" packs as FN20, unchecked reports, 3DA0/3X)."""
@@ -224,6 +236,7 @@ def test_library_pack77_vs_reference(pkg):
     assert 5000 < n_std < 15000
 
 
+@needs_reference
 def test_encoder_and_crc_vs_reference(oracle):
     ref = Reference("k120")
     rng = np.random.default_rng(8)
@@ -239,6 +252,7 @@ def test_encoder_and_crc_vs_reference(oracle):
     assert oracle.pack_text("HELLO WORLD") == ref.pack77("HELLO WORLD")
 
 
+@needs_reference
 def test_fft_vs_kiss(oracle):
     mon = ReferenceMonitor()
     rng = np.random.default_rng(9)
@@ -247,6 +261,7 @@ def test_fft_vs_kiss(oracle):
         assert np.array_equal(oracle.fft_r2c(x).view(np.uint32), mon.fftr(x).view(np.uint32)), n
 
 
+@needs_reference
 def test_monitor_vs_reference(oracle):
     mon = ReferenceMonitor()
     sigs = [(ft8enc.tones(ft8enc.pack_std("CQ", "K1JT", "FN20")), 1200.0, 0.5, 0.1), (ft8enc.tones(ft8enc.pack_std("K1ABC", "W9XYZ", "-15")), 2100.0, 1.1, 0.05)]
@@ -286,6 +301,7 @@ def ft4_audio(seed, n=5):
     return synth.audio_12k(sigs, seed, n_samples=90_000, symbol_period=0.048), texts
 
 
+@needs_reference
 def test_ft4_vs_reference(oracle):
     """FT4 through the restatement == the unmodified reference at every tap: encoder tones, the 7.5 s / 576-sample
     monitor waterfall (kiss_fftr 1152), ft4_sync_score + heap order, 87x2 LLRs, LDPC, CRC, descrambling, text."""
@@ -321,30 +337,42 @@ def test_ft4_vs_reference(oracle):
     assert decoded_any >= 4, "the synthetic FT4 signals must actually decode"
 
 
-def test_decode_ft8_main_on_the_reference_recordings(oracle):
-    """The reference's own main() (`decode_ft8 file.wav`, stdout captured) on all 60 real-world recordings it ships ==
-    the restatement's chain (monitor waterfall -> find_sync -> decode -> unique-message table), line for line:
-    score, time, frequency and text of every decode, in order (981 lines)."""
-    import glob
+def stored_recordings(tmp_path):
+    """tests/golden/recordings_12k.npz -- three of the reference's own real-world recordings and the stdout lines of its
+    decode_ft8 on them -- written back as 16-bit mono WAV files: -> [(path, lines)]."""
+    import wave
+    g = golden("recordings_12k")
+    out = []
+    for k, (pcm, lines) in enumerate(zip(g["pcm"], g["lines"])):
+        path = str(tmp_path / f"rec{k}.wav")
+        with wave.open(path, "wb") as w:
+            w.setnchannels(1); w.setsampwidth(2); w.setframerate(12000)
+            w.writeframes(np.ascontiguousarray(pcm, np.int16).tobytes())
+        out.append((path, str(lines).split("\n")))
+    return out
+
+
+@needs_reference
+def test_decode_ft8_main_on_the_reference_recordings(oracle, tmp_path):
+    """The reference's own main() (`decode_ft8 file.wav`, stdout captured) on the stored real-world recordings == the
+    restatement's chain (monitor waterfall -> find_sync -> decode -> unique-message table), line for line: score, time,
+    frequency and text of every decode, in order -- and both == the lines stored with the recordings (47 lines)."""
     mon = ReferenceMonitor()
-    wavs = sorted(glob.glob("/root/reference/ft8_lib/tests/**/*.wav", recursive=True))
-    if not wavs:
-        pytest.skip("reference recordings not present")
     total = 0
-    for p in wavs:
+    for p, stored in stored_recordings(tmp_path):
         ref = mon.decode_ft8_stdout(p)
         sig, sr = mon.load_wav(p)
-        assert oracle.decode_ft8_lines(sig, sr) == ref, p
+        assert oracle.decode_ft8_lines(sig, sr) == ref == stored, p
         total += len(ref)
-    assert len(wavs) == 60 and total > 900
+    assert total == 47
 
 
+@needs_reference
 def test_file_loaders_vs_reference(pkg, oracle, tmp_path):
     """The library's host-side readers against the reference's readRawIQfile / readC2file / load_wav on the same files
     (the reference normalises on the host; the library returns unscaled samples + peak and scales on the device, so the
     comparison applies decoder()'s scale expression here)."""
     import ctypes as C
-    import glob
     ref = Reference("k120")
     i_s, q_s = synth.slot_f32([(ft8enc.tones(ft8enc.pack_std("CQ", "K1JT", "FN20")), 700.0, 0.5, -3.0)], 5)
     i_s *= 3.7; q_s *= 3.7
@@ -366,7 +394,7 @@ def test_file_loaders_vs_reference(pkg, oracle, tmp_path):
     assert pkg.read_c2_file(c2_path)[4:] == (14.074, 2, b"210101_0000.c2")
     assert pkg.read_iq_file(str(tmp_path / "missing.iq"))[2] == 0
     mon = ReferenceMonitor()
-    for p in sorted(glob.glob("/root/reference/ft8_lib/tests/*.wav"))[:3]:
+    for p, _ in stored_recordings(tmp_path):
         a, sr = pkg.load_wav(p)
         b, sr2 = mon.load_wav(p)
         assert sr == sr2 == 12000 and bits_equal(a, b)
