@@ -250,6 +250,27 @@ int ft8b200_decode(ft8b200_ctx_t *ctx, const uint8_t *d_mag, size_t slot_stride_
                    int time_osr, int freq_osr, const candidate_t *d_cand, const int *d_ncand, uint8_t *d_ok, uint8_t *d_stage,
                    decode_status_t *d_status, message_t *d_msg, uint8_t *d_plain, float *d_llr, void *stream);
 
+/* Ordered-statistics decoding (OSD, DESIGN.md section 2.4.1) of the candidates belief propagation leaves undecoded (stage 1: no zero
+ * syndrome, stage 2: CRC mismatch).  order: 0 = off (default), 1 = the most reliable basis' hard decisions and every single flip
+ * (92 codewords), 2 = also every pair among its 32 least reliable positions (588); anything else is FT8B200_EINVAL.  The least-metric
+ * codeword is accepted when its CRC holds, it differs from the hard decision in at most max_hard_errors bits and it unpacks.
+ * max_hard_errors < 0 selects FT8B200_OSD_DEFAULT_MAX_HARD: the largest cap that decoded at most 2 messages on 4096 noise-only
+ * daemon slots (K = 120) at order 2 (tools/perf_osd.py; profiles/perf_osd.json).
+ * The process_* calls, ft8b200_decode and the whole-recording calls honour it; off, every output and launch is as without it. */
+#define FT8B200_OSD_DEFAULT_MAX_HARD 174
+int ft8b200_set_osd(ft8b200_ctx_t *ctx, int order, int max_hard_errors);
+/* Stage-wise OSD with the context's order, cap and protocol: upgrades the n_slots x max_candidates outputs of ft8b200_decode in
+ * place (d_llr = its normalised LLRs).  An accepted codeword makes the entry ok = 1, stage = 4, status.ldpc_errors = 0 with the
+ * codeword's CRC fields, msg as a BP decode would, d_plain (optional) = the codeword; a rejected one changes none of them.
+ * d_osd: 0 = not attempted (stage 3/4, beyond d_ncand, a non-finite LLR or order 0), 1 = attempted and rejected, 2 = decoded by OSD.
+ * d_osd_hard: the winner's hard-decision distance, -1 when not attempted.  d_osd_cw (optional, uint8[...][174]): the winner whether
+ * or not it was accepted (zeros when not attempted). */
+int ft8b200_osd(ft8b200_ctx_t *ctx, const float *d_llr, int n_slots, const int *d_ncand, uint8_t *d_ok, uint8_t *d_stage,
+                decode_status_t *d_status, message_t *d_msg, uint8_t *d_plain, uint8_t *d_osd, int32_t *d_osd_hard, uint8_t *d_osd_cw,
+                void *stream);
+/* d_osd / d_osd_hard (as above) of the last process_* or decode batch run with OSD on (n_slots x max_candidates); NULL before that */
+int ft8b200_osd_workspace(ft8b200_ctx_t *ctx, uint8_t **d_osd, int32_t **d_osd_hard);
+
 /* a15: the daemon's duplicate table + CQ filter, one slot per thread.  d_results: n_slots x max_messages
  * (zeroed here first), d_nresults: n_slots; optional first-seen unique message log: d_umsg (n_slots x
  * max_messages message_t), d_ufreq (float), d_uscore (int32), d_ucand (int32, optional: index of the candidate
@@ -393,6 +414,9 @@ int ft8b200_pipe_partition_smids(ft8b200_pipe_t *p, int which, uint32_t *mask8);
  * shows within a dozen batches whether ONE batch's back end fits under the next batch's block sums) and restores afterwards.
  * Results are identical either way.  Not while batches are in flight. */
 int ft8b200_pipe_set_back_chain(ft8b200_pipe_t *p, int on);
+/* ft8b200_set_osd on every lane (a cluster's pipes through ft8b200_cluster_pipe).  FT8B200_EBUSY while batches are in flight;
+ * ft8b200_osd_workspace of a lane is not exposed: the pipe returns spot records only. */
+int ft8b200_pipe_set_osd(ft8b200_pipe_t *p, int order, int max_hard_errors);
 int ft8b200_pipe_autotune(ft8b200_pipe_t *p, const uint8_t *d_iq, size_t bytes_per_stream, size_t stream_stride_bytes, int n_slots,
                           const int *candidates, int n_candidates, int batches, int *best_back_sms, int *best_comb_front, float *ms_out);
 void ft8b200_pipe_destroy(ft8b200_pipe_t *p);

@@ -267,6 +267,28 @@ class Context:
                                         _p(cand), _p(ncand), _p(ok), _p(stage), _p(status), _p(msg), _p(plain), _p(llr), _st(stream)))
         return ok, stage, status, msg, plain, llr
 
+    def set_osd(self, order: int, max_hard_errors: int = -1):
+        """Ordered-statistics decoding after BP: order 0 (off), 1 or 2; max_hard_errors < 0 = FT8B200_OSD_DEFAULT_MAX_HARD."""
+        self._chk(self.L.ft8b200_set_osd(C.c_void_p(self.h), int(order), int(max_hard_errors)))
+
+    def osd(self, llr, ncand, ok, stage, status, msg, plain=None, want_cw=False, stream: int | None = None):
+        """Stage-wise OSD over ft8b200_decode's outputs (updated in place) -> (osd uint8[n, K], osd_hard int32[n, K], cw uint8[n, K, 174] or None)."""
+        import torch
+        n = llr.shape[0]
+        dev = llr.device
+        osd = torch.zeros((n, self.K), dtype=torch.uint8, device=dev)
+        hard = torch.zeros((n, self.K), dtype=torch.int32, device=dev)
+        cw = torch.zeros((n, self.K, 174), dtype=torch.uint8, device=dev) if want_cw else None
+        self._chk(self.L.ft8b200_osd(C.c_void_p(self.h), _p(llr), n, _p(ncand), _p(ok), _p(stage), _p(status), _p(msg), _p(plain), _p(osd), _p(hard),
+                                     _p(cw), _st(stream)))
+        return osd, hard, cw
+
+    def osd_workspace_ptrs(self):
+        """Device pointers (osd, osd_hard) of the last batch decoded with OSD on (0 before that)."""
+        a, b = C.c_void_p(0), C.c_void_p(0)
+        self._chk(self.L.ft8b200_osd_workspace(C.c_void_p(self.h), C.byref(a), C.byref(b)))
+        return a.value or 0, b.value or 0
+
     def spots(self, cand, ncand, ok, msg, freq_osr=2, want_log=True, stream: int | None = None):
         import torch
         n = cand.shape[0]
@@ -503,6 +525,10 @@ class Pipe:
         f, b = C.c_int(0), C.c_int(0)
         self._chk(self.L.ft8b200_pipe_set_partition(C.c_void_p(self.h), int(back_sms), C.byref(f), C.byref(b)))
         return f.value, b.value
+
+    def set_osd(self, order: int, max_hard_errors: int = -1):
+        """Context.set_osd on every lane; not while batches are in flight."""
+        self._chk(self.L.ft8b200_pipe_set_osd(C.c_void_p(self.h), int(order), int(max_hard_errors)))
 
     def set_back_chain(self, on: bool):
         """Back ends of consecutive batches serialised on the back partition (what the autotune probes with)."""

@@ -76,6 +76,10 @@ struct ft8b200_ctx {
     int sm_count = 0;
     // workspaces (grown on demand)
     DevBuf raw, sums, si, sq, peak, count, mag, cand, ncand, ok, stage, status, msg, results, nresults, table, lists, scores, work, work_total;
+    // ordered-statistics decoding after BP (ft8b200_set_osd): 0 = off; the LLRs it reads and its per-candidate outputs
+    int osd_order = 0;
+    int osd_max_hard = FT8B200_OSD_DEFAULT_MAX_HARD;
+    DevBuf llr, osd, osd_hard;
     // optional per-stage timing of the last process_* call (CUDA events on the launching stream)
     bool profiling = false;
     int overlap = 0;                       // number of slot groups ft8b200_process_raw pipelines (0/1 = off)
@@ -112,6 +116,14 @@ void tally(ft8b200_ctx_t *ctx) {
     ctx->launches = 0;
 }
 
+int ensure_osd_buffers(ft8b200_ctx_t *ctx, int n_slots) {
+    const size_t E = (size_t)n_slots * ctx->cfg.max_candidates;
+    int rc;
+    if ((rc = ctx->llr.ensure(E * kLdpcN * sizeof(float)))) return rc;
+    if ((rc = ctx->osd.ensure(E))) return rc;
+    return ctx->osd_hard.ensure(E * sizeof(int32_t));
+}
+
 int ensure_slot_buffers(ft8b200_ctx_t *ctx, int n_slots) {
     const size_t K = (size_t)ctx->cfg.max_candidates, M = (size_t)ctx->cfg.max_messages, S = (size_t)n_slots;
     int rc;
@@ -125,6 +137,7 @@ int ensure_slot_buffers(ft8b200_ctx_t *ctx, int n_slots) {
     if ((rc = ctx->results.ensure(S * M * sizeof(struct decoder_results)))) return rc;
     if ((rc = ctx->nresults.ensure(S * sizeof(int32_t)))) return rc;
     if ((rc = ctx->table.ensure(S * M * sizeof(int16_t)))) return rc;
+    if (ctx->osd_order && (rc = ensure_osd_buffers(ctx, n_slots))) return rc;
     return 0;
 }
 
@@ -234,7 +247,8 @@ void ft8b200_destroy(ft8b200_ctx_t *ctx) {
     cudaFree(ctx->tb.window1024); cudaFree(ctx->tb.twiddle1024); cudaFree(ctx->tb.db_thresholds); cudaFree(ctx->tb.wf_blob);
     cudaFree(ctx->tb.mon_window); cudaFree(ctx->tb.mon_twiddle); cudaFree(ctx->tb.mon_super);
     DevBuf *bufs[] = {&ctx->raw, &ctx->sums, &ctx->si, &ctx->sq, &ctx->peak, &ctx->count, &ctx->mag, &ctx->cand, &ctx->ncand, &ctx->ok,
-                      &ctx->stage, &ctx->status, &ctx->msg, &ctx->results, &ctx->nresults, &ctx->table, &ctx->lists, &ctx->scores, &ctx->work, &ctx->work_total};
+                      &ctx->stage, &ctx->status, &ctx->msg, &ctx->results, &ctx->nresults, &ctx->table, &ctx->lists, &ctx->scores, &ctx->work, &ctx->work_total,
+                      &ctx->llr, &ctx->osd, &ctx->osd_hard};
     for (DevBuf *b : bufs) b->release();
     delete ctx;
 }
@@ -355,8 +369,19 @@ int decode_proto(ft8b200_ctx_t *ctx, int protocol, const uint8_t *d_mag, size_t 
         pull = ctx->work_total.as<unsigned int>();
         CU(cudaMemsetAsync(pull, 0, 4 * sizeof(unsigned int), pick(ctx, stream)));
     }
+    if (ctx->osd_order) {
+        if ((rc = ensure_osd_buffers(ctx, n_slots))) return rc;
+        if (!d_llr) d_llr = ctx->llr.as<float>();
+    }
     CU(launch_decode(d_mag, slot_stride_bytes, n_slots, num_blocks, num_bins, time_osr, freq_osr, protocol, ctx->cfg.max_candidates, ctx->cfg.ldpc_iterations,
                      d_cand, d_ncand, d_ok, d_stage, d_status, d_msg, d_plain, d_llr, nullptr, pull, ctx->sm_count, pick(ctx, stream), &ctx->launches));
+    if (ctx->osd_order) {
+        unsigned int *next = ctx->work_total.as<unsigned int>() + 2;
+        CU(cudaMemsetAsync(next, 0, sizeof(unsigned int), pick(ctx, stream)));
+        CU(launch_osd(n_slots, ctx->cfg.max_candidates, protocol, ctx->osd_order, ctx->osd_max_hard, d_llr, d_ncand, d_ok, d_stage, d_status, d_msg,
+                      d_plain, ctx->osd.as<uint8_t>(), ctx->osd_hard.as<int32_t>(), nullptr, nullptr, nullptr, next, ctx->sm_count, pick(ctx, stream),
+                      &ctx->launches));
+    }
     tally(ctx);
     return 0;
 }
@@ -393,6 +418,38 @@ int ft8b200_spots(ft8b200_ctx_t *ctx, int n_slots, int freq_osr, const candidate
     return 0;
 }
 
+int ft8b200_set_osd(ft8b200_ctx_t *ctx, int order, int max_hard_errors) {
+    if (!ctx || order < 0 || order > 2) return fail(FT8B200_EINVAL, "ft8b200_set_osd: order 0 (off), 1 or 2");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    ctx->osd_order = order;
+    ctx->osd_max_hard = max_hard_errors < 0 ? FT8B200_OSD_DEFAULT_MAX_HARD : max_hard_errors;
+    return 0;
+}
+
+int ft8b200_osd(ft8b200_ctx_t *ctx, const float *d_llr, int n_slots, const int *d_ncand, uint8_t *d_ok, uint8_t *d_stage, decode_status_t *d_status,
+                message_t *d_msg, uint8_t *d_plain, uint8_t *d_osd, int32_t *d_osd_hard, uint8_t *d_osd_cw, void *stream) {
+    int rc = ctx_enter(ctx);
+    if (rc) return rc;
+    if (!d_llr || !d_ncand || !d_ok || !d_stage || !d_status || !d_msg || !d_osd || !d_osd_hard || n_slots < 1)
+        return fail(FT8B200_EINVAL, "ft8b200_osd: bad argument");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    if ((rc = ctx->work_total.ensure(4 * sizeof(unsigned int)))) return rc;
+    cudaStream_t st = pick(ctx, stream);
+    unsigned int *next = ctx->work_total.as<unsigned int>() + 2;
+    CU(cudaMemsetAsync(next, 0, sizeof(unsigned int), st));
+    CU(launch_osd(n_slots, ctx->cfg.max_candidates, ctx->protocol, ctx->osd_order, ctx->osd_max_hard, d_llr, d_ncand, d_ok, d_stage, d_status, d_msg,
+                  d_plain, d_osd, d_osd_hard, d_osd_cw, nullptr, nullptr, next, ctx->sm_count, st, &ctx->launches));
+    tally(ctx);
+    return 0;
+}
+
+int ft8b200_osd_workspace(ft8b200_ctx_t *ctx, uint8_t **d_osd, int32_t **d_osd_hard) {
+    if (!ctx) return fail(FT8B200_EINVAL, "null context");
+    if (d_osd) *d_osd = ctx->osd.as<uint8_t>();
+    if (d_osd_hard) *d_osd_hard = ctx->osd_hard.as<int32_t>();
+    return 0;
+}
+
 // ---- per-stage timing: one event pair per (stage, group); stage times are summed over the groups -------------
 static void mark(ft8b200_ctx_t *ctx, int stage, int group, bool end, cudaStream_t st) {
     if (!ctx->profiling || group >= kMaxGroups) return;
@@ -424,9 +481,15 @@ static int run_back_end(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, 
                         st, &ctx->launches));
     mark(ctx, 3, group, true, st);
     mark(ctx, 4, group, false, st);
+    float *llr = ctx->osd_order ? ctx->llr.as<float>() + (size_t)s0 * K * kLdpcN : nullptr;
     CU(launch_decode(mag, kWfBytes, n, 92, 256, 2, 2, PROTO_FT8, ctx->cfg.max_candidates, ctx->cfg.ldpc_iterations, cand, ncand, ok, stage,
-                     ctx->status.as<decode_status_t>() + (size_t)s0 * K, ctx->msg.as<message_t>() + (size_t)s0 * K, nullptr, nullptr,
+                     ctx->status.as<decode_status_t>() + (size_t)s0 * K, ctx->msg.as<message_t>() + (size_t)s0 * K, nullptr, llr,
                      ctx->work.as<uint32_t>(), ctx->work_total.as<unsigned int>(), sms, st, &ctx->launches));
+    if (ctx->osd_order)  // the work list's entries BP left at stage 1 or 2; word [2] of work_total (zeroed by launch_find_sync) is its pull counter
+        CU(launch_osd(n, ctx->cfg.max_candidates, PROTO_FT8, ctx->osd_order, ctx->osd_max_hard, llr, ncand, ok, stage,
+                      ctx->status.as<decode_status_t>() + (size_t)s0 * K, ctx->msg.as<message_t>() + (size_t)s0 * K, nullptr,
+                      ctx->osd.as<uint8_t>() + (size_t)s0 * K, ctx->osd_hard.as<int32_t>() + (size_t)s0 * K, nullptr, ctx->work.as<uint32_t>(),
+                      ctx->work_total.as<unsigned int>(), ctx->work_total.as<unsigned int>() + 2, sms, st, &ctx->launches));
     mark(ctx, 4, group, true, st);
     mark(ctx, 5, group, false, st);
     CU(launch_spots(n, ctx->cfg.max_candidates, ctx->cfg.max_messages, ctx->cfg.min_score, 2, cand, ncand, ok, ctx->msg.as<message_t>() + (size_t)s0 * K,

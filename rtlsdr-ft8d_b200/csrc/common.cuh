@@ -64,6 +64,12 @@ cudaError_t launch_decode(const uint8_t *d_mag, size_t slot_stride, int n_slots,
 cudaError_t launch_spots(int n_slots, int max_cand, int max_msgs, int min_score, int freq_osr, const candidate_t *d_cand, const int *d_ncand,
                          const uint8_t *d_ok, const message_t *d_msg, struct decoder_results *d_results, int32_t *d_nresults,
                          message_t *d_umsg, float *d_ufreq, int32_t *d_uscore, int32_t *d_ucand, int16_t *d_table, cudaStream_t st, int *launches);
+// ordered-statistics decoding of the entries BP left at stage 1 or 2 (order 0: nothing attempted); with d_work the entries of the
+// find_sync work list, otherwise all n_slots * max_cand.  *d_next: the pull counter, zeroed by the caller.
+cudaError_t launch_osd(int n_slots, int max_cand, int protocol, int order, int max_hard, const float *d_llr, const int *d_ncand, uint8_t *d_ok,
+                       uint8_t *d_stage, decode_status_t *d_status, message_t *d_msg, uint8_t *d_plain, uint8_t *d_osd, int32_t *d_osd_hard,
+                       uint8_t *d_osd_cw, const uint32_t *d_work, const unsigned int *d_work_total, unsigned int *d_next, int sm_count,
+                       cudaStream_t st, int *launches);
 cudaError_t launch_unpack77_batch(const uint8_t *d_payloads, int n, char *d_text32, int32_t *d_status, cudaStream_t st, int *launches);
 cudaError_t upload_ldpc_tables();
 void set_decode_variant(int v);  // 0 = node-centred belief propagation (default), 1 = edge-centred

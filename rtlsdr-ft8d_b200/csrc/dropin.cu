@@ -117,6 +117,9 @@ ft8b200_ctx_t *default_ctx() {
         if (dev) cfg.device = atoi(dev);
         g_ctx = ft8b200_create(&cfg);
         if (!g_ctx) die("ft8b200_create (default context)");
+        // deeper decoding for a relinked program without code changes: FT8B200_OSD=<order>, FT8B200_OSD_MAX_HARD=<cap> (INTEGRATION.md)
+        const char *osd = getenv("FT8B200_OSD"), *cap = getenv("FT8B200_OSD_MAX_HARD");
+        if (osd && ft8b200_set_osd(g_ctx, atoi(osd), cap ? atoi(cap) : -1) != 0) die("FT8B200_OSD (0, 1 or 2)");
     }
     return g_ctx;
 }
