@@ -187,6 +187,13 @@ int ft8b200_monitor_flush(monitor_t *me);
 #define FT8B200_DECIM 751           /* input samples per output sample (rtlsdr_ft8d.c:156-160) */
 #define FT8B200_WF_BYTES 94208      /* daemon waterfall bytes per slot (rtlsdr_ft8d.h:54) */
 #define FT8B200_RAW_SLOT_BYTES 72000000
+/* Batch sizes: the entry points that take slots of 3200 sps samples, waterfalls, candidates or audio (process_slots /
+ * _conditioned, condition, waterfall, find_sync, decode, osd, spots, monitor_waterfall, synth_*, the pipe's submit_slots,
+ * the stream and file calls) accept any n_slots >= 1 the device memory holds; beyond 65 535 slots their per-slot kernels
+ * run as several launches.  The raw-IQ entry points (decimate, decimate_streams, process_raw, process_raw_streams and the
+ * pipe and cluster submits built on them) refuse more than FT8B200_MAX_RAW_ROWS streams or output rows per call with
+ * FT8B200_EINVAL: that many raw slots are 4.7 TB. */
+#define FT8B200_MAX_RAW_ROWS 65535
 
 typedef struct ft8b200_ctx ft8b200_ctx_t;
 typedef struct ft8b200_stream ft8b200_stream_t;
@@ -286,6 +293,8 @@ int ft8b200_process_raw(ft8b200_ctx_t *ctx, const uint8_t *d_iq, size_t bytes_pe
 /* whole path over continuous streams (see ft8b200_decimate_streams): n_streams*slots_per_stream result rows */
 int ft8b200_process_raw_streams(ft8b200_ctx_t *ctx, const uint8_t *d_iq, size_t bytes_per_stream, size_t stream_stride_bytes, int n_streams,
                                 int slots_per_stream, size_t bytes_per_slot, void *stream);
+/* n_slots x 48000 conditioned samples per rail; d_i and d_q must be 16-byte aligned (as for ft8b200_waterfall), otherwise
+ * FT8B200_EINVAL before anything is queued.  The same holds for ft8b200_process_conditioned and ft8b200_pipe_submit_slots. */
 int ft8b200_process_slots(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, int n_slots, void *stream);
 /* same, but the samples are NOT yet conditioned: d_peak[slot] = max(|I|,|Q|) and decoder()'s 0.5/peak scale is applied on load */
 int ft8b200_process_conditioned(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, const float *d_peak, int n_slots, void *stream);
@@ -432,7 +441,8 @@ int ft8b200_pipe_submit_streams(ft8b200_pipe_t *p, const uint8_t *d_iq, size_t b
 /* The same executor fed at the OTHER boundary of the path, the input of ft8_subsystem() (rtlsdr_ft8d.h:164): n_slots x 48000 float
  * samples per rail at 3200 sps.  _host: conditioned samples in (pinned) host memory, copied H2D on the lane's stream; device form:
  * d_peak == NULL for conditioned samples, else decoder()'s 0.5/peak scale is applied on load.  384 KB per slot instead of 72 MB:
- * this is the call for hosts that decimate elsewhere (or replay .iq/.c2 recordings).  Use a pipe without an SM partition. */
+ * this is the call for hosts that decimate elsewhere (or replay .iq/.c2 recordings).  Use a pipe without an SM partition.
+ * d_i and d_q must be 16-byte aligned; a refused batch is not in flight. */
 int ft8b200_pipe_submit_slots(ft8b200_pipe_t *p, const float *d_i, const float *d_q, const float *d_peak, int n_slots);
 int ft8b200_pipe_submit_slots_host(ft8b200_pipe_t *p, const float *h_i, const float *h_q, int n_slots);
 int ft8b200_pipe_collect(ft8b200_pipe_t *p, struct decoder_results *h_results, int32_t *h_nresults, int capacity_slots);

@@ -277,6 +277,8 @@ static int decimate_impl(ft8b200_ctx_t *ctx, const uint8_t *d_iq, size_t bytes_p
         return fail(FT8B200_EINVAL, "ft8b200_decimate: byte counts must be multiples of 8, stream stride and base 16-byte aligned");
     if (segs < 1 || (segs > 1 && (seg_bytes < 8 || (seg_bytes & 7) || seg_bytes * (size_t)segs > bytes_per_stream || seg_bytes / 2 / kDecim + 1 > (size_t)kSlot)))
         return fail(FT8B200_EINVAL, "ft8b200_decimate_streams: slots_per_stream * bytes_per_slot must fit the stream, bytes_per_slot a multiple of 8 and <= one 48000-sample slot");
+    if ((long long)n_streams * segs > FT8B200_MAX_RAW_ROWS)
+        return fail(FT8B200_EINVAL, "ft8b200_decimate: more than FT8B200_MAX_RAW_ROWS (65535) streams or output rows in one call; split the batch");
     const int blocks = (int)((bytes_per_stream / 2) / kDecim);
     // the 128-bit loads of the last super-block may read up to 14 bytes past the last complete block
     if ((size_t)(blocks / 8) * 12016 > bytes_per_stream) return fail(FT8B200_EINVAL, "internal: super-block overrun");
@@ -524,6 +526,8 @@ static int process_raw_impl(ft8b200_ctx_t *ctx, const uint8_t *d_iq, size_t byte
         return fail(FT8B200_EINVAL, "ft8b200_process_raw: byte counts must be multiples of 8, stream stride and base 16-byte aligned");
     if (segs < 1 || (segs > 1 && (seg_bytes < 8 || (seg_bytes & 7) || seg_bytes * (size_t)segs > bytes_per_stream || seg_bytes / 2 / kDecim + 1 > (size_t)kSlot)))
         return fail(FT8B200_EINVAL, "ft8b200_process_raw_streams: slots_per_stream * bytes_per_slot must fit the stream, bytes_per_slot a multiple of 8 and <= one 48000-sample slot");
+    if ((long long)n_slots * segs > FT8B200_MAX_RAW_ROWS)
+        return fail(FT8B200_EINVAL, "ft8b200_process_raw: more than FT8B200_MAX_RAW_ROWS (65535) streams or result rows in one call; split the batch");
     std::lock_guard<std::mutex> lk(ctx->mu);
     cudaStream_t st = pick(ctx, stream);
     const int blocks = (int)((bytes_per_stream / 2) / kDecim);
@@ -624,6 +628,8 @@ int ft8b200_process_conditioned(ft8b200_ctx_t *ctx, const float *d_i, const floa
     int rc = ctx_enter(ctx);
     if (rc) return rc;
     if (!d_i || !d_q || n_slots < 1) return fail(FT8B200_EINVAL, "ft8b200_process_slots: bad argument");
+    // the waterfall kernel reads the samples with 16-byte cp.async (as ft8b200_waterfall requires): refused before anything is queued
+    if ((((size_t)d_i) | ((size_t)d_q)) & 15) return fail(FT8B200_EINVAL, "ft8b200_process_slots: d_i and d_q must be 16-byte aligned");
     std::lock_guard<std::mutex> lk(ctx->mu);
     cudaStream_t st = pick(ctx, stream);
     if ((rc = ensure_slot_buffers(ctx, n_slots))) return rc;

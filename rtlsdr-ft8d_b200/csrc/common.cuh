@@ -34,7 +34,10 @@ struct DeviceTables {
 };
 
 // ---- launchers (each returns cudaGetLastError()) ----
-constexpr int kHistBlocks = 59;  // block sums a flush needs from before its first block: 56 FIR taps + 3 comb delays
+// gridDim.y limit: launches that put the slot (or stream) in blockIdx.y cover at most this many rows each; the slot-wise
+// launchers run larger batches as consecutive launches, the raw-IQ entry points refuse more rows (FT8B200_MAX_RAW_ROWS)
+constexpr int kMaxGridRows = 65535;
+constexpr int kHistBlocks = 59; // block sums a flush needs from before its first block: 56 FIR taps + 3 comb delays
 constexpr int kK1StreamingDense = -1;   // `variant` of launch_cic_block_sums: the streaming kernel at 5 CTAs per SM (for a launch that owns only part of the SMs)
 cudaError_t launch_cic_block_sums(const uint8_t *d_iq, size_t stream_stride_bytes, int n_streams, int blocks_per_stream, BlockSums *d_sums,
                                   size_t sums_stride, int variant, int sm_count, cudaStream_t st, int *launches);

@@ -753,10 +753,15 @@ cudaError_t launch_shift_history(BlockSums *d_sums_with_prefix, int n_blocks, cu
 }
 
 cudaError_t launch_condition(float *d_i, float *d_q, const float *d_peak, int n_slots, cudaStream_t st, int *launches) {
-    dim3 grid((kSlot + 255) / 256, n_slots);
-    condition_kernel<<<grid, 256, 0, st>>>(d_i, d_q, d_peak);
-    ++*launches;
-    return cudaGetLastError();
+    for (int s0 = 0; s0 < n_slots; s0 += kMaxGridRows) {   // the slot is blockIdx.y
+        const int rows = n_slots - s0 < kMaxGridRows ? n_slots - s0 : kMaxGridRows;
+        const size_t o = (size_t)s0 * kSlot;
+        condition_kernel<<<dim3((kSlot + 255) / 256, rows), 256, 0, st>>>(d_i + o, d_q + o, d_peak + s0);
+        ++*launches;
+        const cudaError_t e = cudaGetLastError();
+        if (e != cudaSuccess) return e;
+    }
+    return cudaSuccess;
 }
 
 }  // namespace ft8b200

@@ -150,6 +150,8 @@ int submit(ft8b200_pipe_t *p, const uint8_t *h_iq, const uint8_t *d_iq, size_t b
            size_t seg_bytes = 0) {
     if (!p) return FT8B200_BAD_ARG();
     if ((!h_iq && !d_iq) || n_slots < 1 || (bytes_per_stream & 7) || segs < 1) return pfail(p, FT8B200_EINVAL, "ft8b200_pipe_submit: bad argument");
+    if ((long long)n_slots * segs > FT8B200_MAX_RAW_ROWS)   // before the host copy and the pinned record buffers are sized for it
+        return pfail(p, FT8B200_EINVAL, "ft8b200_pipe_submit: more than FT8B200_MAX_RAW_ROWS (65535) streams or result rows in one batch; split it");
     const int n_rows = n_slots * segs;
     if (p->count == (int)p->lanes.size()) return pfail(p, FT8B200_EBUSY, "ft8b200_pipe_submit: every lane is in flight, collect first");
     PCU(cudaSetDevice(p->cfg.device));

@@ -609,30 +609,40 @@ cudaError_t launch_find_sync(const uint8_t *d_mag, size_t slot_stride, int n_slo
     if (splits < 1) splits = 1;
     const int to_per_cta = (36 + splits - 1) / splits;
     splits = (36 + to_per_cta - 1) / to_per_cta;
-    dim3 grid(planes * splits, n_slots);
     const size_t staged = ((size_t)g.nb * g.nbins + 15) & ~(size_t)15;
     const bool ft4 = protocol == PROTO_FT4;
     const size_t fast_smem = (((size_t)g.nb * kRawPitch + 15) & ~(size_t)15) + (size_t)4 * fast_rows(g.nb) * kTilePitch * sizeof(int16_t);
-    if (!ft4 && fast_smem <= 96 * 1024 && (((size_t)d_mag | slot_stride | (size_t)g.stride | (size_t)g.nbins) & 3) == 0) {
-        // FT8 fast path: derived int16 planes per (plane, tile of 64 frequency offsets)
-        const int tiles = (g.nfo + kTileF - 1) / kTileF;
-        e = cudaFuncSetAttribute(sync_score_ft8_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
-        if (e != cudaSuccess) return e;
-        sync_score_ft8_kernel<<<dim3(planes * tiles, n_slots), kScoreThreads, fast_smem, st>>>(d_mag, slot_stride, g, tiles, d_scores, sa, term_magic(g.nb));
-    } else if (staged <= 200 * 1024) {
-        if (g.nbins == 256 && !ft4) {
-            sync_score_kernel<256, true, false><<<grid, kScoreThreads, staged, st>>>(d_mag, slot_stride, g, splits, to_per_cta, d_scores, sa);
+    // the slot is blockIdx.y: a batch of more than kMaxGridRows slots is scored by consecutive launches, each over slots
+    // [s0, s0 + rows) with its pointers moved to slot s0 (one launch, exactly as before, for every smaller batch)
+    for (int s0 = 0; s0 < n_slots; s0 += kMaxGridRows) {
+        const int rows = n_slots - s0 < kMaxGridRows ? n_slots - s0 : kMaxGridRows;
+        const uint8_t *mag = d_mag + (size_t)s0 * slot_stride;
+        int16_t *scores = d_scores + (size_t)s0 * g.npos;
+        SelArgs sc = sa;
+        sc.count += s0;
+        sc.lists += (size_t)s0 * kListCap;
+        const dim3 grid(planes * splits, rows);
+        if (!ft4 && fast_smem <= 96 * 1024 && (((size_t)d_mag | slot_stride | (size_t)g.stride | (size_t)g.nbins) & 3) == 0) {
+            // FT8 fast path: derived int16 planes per (plane, tile of 64 frequency offsets)
+            const int tiles = (g.nfo + kTileF - 1) / kTileF;
+            e = cudaFuncSetAttribute(sync_score_ft8_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
+            if (e != cudaSuccess) return e;
+            sync_score_ft8_kernel<<<dim3(planes * tiles, rows), kScoreThreads, fast_smem, st>>>(mag, slot_stride, g, tiles, scores, sc, term_magic(g.nb));
+        } else if (staged <= 200 * 1024) {
+            if (g.nbins == 256 && !ft4) {
+                sync_score_kernel<256, true, false><<<grid, kScoreThreads, staged, st>>>(mag, slot_stride, g, splits, to_per_cta, scores, sc);
+            } else {
+                auto kern = ft4 ? sync_score_kernel<0, true, true> : sync_score_kernel<0, true, false>;
+                if (staged > 48 * 1024 && (e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)staged)) != cudaSuccess) return e;
+                kern<<<grid, kScoreThreads, staged, st>>>(mag, slot_stride, g, splits, to_per_cta, scores, sc);
+            }
         } else {
-            auto kern = ft4 ? sync_score_kernel<0, true, true> : sync_score_kernel<0, true, false>;
-            if (staged > 48 * 1024 && (e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)staged)) != cudaSuccess) return e;
-            kern<<<grid, kScoreThreads, staged, st>>>(d_mag, slot_stride, g, splits, to_per_cta, d_scores, sa);
+            auto kern = ft4 ? sync_score_kernel<0, false, true> : sync_score_kernel<0, false, false>;
+            kern<<<grid, kScoreThreads, 0, st>>>(mag, slot_stride, g, splits, to_per_cta, scores, sc);
         }
-    } else {
-        auto kern = ft4 ? sync_score_kernel<0, false, true> : sync_score_kernel<0, false, false>;
-        kern<<<grid, kScoreThreads, 0, st>>>(d_mag, slot_stride, g, splits, to_per_cta, d_scores, sa);
+        ++*launches;
+        if ((e = cudaGetLastError()) != cudaSuccess) return e;
     }
-    ++*launches;
-    if ((e = cudaGetLastError()) != cudaSuccess) return e;
     if (d_work_total) {
         e = cudaMemsetAsync(d_work_total, 0, 4 * sizeof(unsigned int), st);  // [0] items, [1] next item (decode_kernel)
         if (e != cudaSuccess) return e;

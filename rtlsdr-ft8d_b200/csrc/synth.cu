@@ -563,9 +563,15 @@ int ft8b200_synth_raw(ft8b200_ctx_t *ctx, const ft8b200_signal_t *h_signals, con
     if (rc) return rc;
     const long long n_samples = (long long)(bytes_per_slot / 2);
     const int noise_q8 = (int)lround((double)noise_lsb * 65536.0 / 147.79715829474123);  // sigma of a sum of 4 uniform bytes
-    dim3 grid((unsigned)((n_samples + 8 * 256 - 1) / (8 * 256)), (unsigned)n_slots);
-    synth_raw_kernel<<<grid, 256, 0, st>>>(d_sigs, d_first, gf, noise_q8, seed, first_slot_index, d_iq, slot_stride_bytes, n_samples);
-    const bool ok = cudaGetLastError() == cudaSuccess && cudaStreamSynchronize(st) == cudaSuccess;
+    bool ok = true;
+    for (int s0 = 0; ok && s0 < n_slots; s0 += kMaxGridRows) {   // the slot is blockIdx.y
+        const int rows = n_slots - s0 < kMaxGridRows ? n_slots - s0 : kMaxGridRows;
+        dim3 grid((unsigned)((n_samples + 8 * 256 - 1) / (8 * 256)), (unsigned)rows);
+        synth_raw_kernel<<<grid, 256, 0, st>>>(d_sigs, d_first + s0, gf, noise_q8, seed, first_slot_index + s0, d_iq + (size_t)s0 * slot_stride_bytes,
+                                               slot_stride_bytes, n_samples);
+        ok = cudaGetLastError() == cudaSuccess;
+    }
+    ok = ok && cudaStreamSynchronize(st) == cudaSuccess;
     cudaFree(d_sigs); cudaFree(d_first);
     return ok ? 0 : FT8B200_CUDA_FAIL();
 }
@@ -582,11 +588,18 @@ static int synth_float(ft8b200_ctx_t *ctx, int kind, int protocol, const ft8b200
     int rc = upload_signals(h_signals, h_first, n_slots, kind, protocol, &d_sigs, &d_first, &gf, st);
     if (rc) return rc;
     const float scale = (float)((double)noise_sigma / 209.02153956946134);  // sigma of a sum of 8 uniform bytes
-    dim3 grid((unsigned)((n_samples + 255) / 256), (unsigned)n_slots);
-    if (kind == 1) synth_float_kernel<512, true><<<grid, 256, 0, st>>>(d_sigs, d_first, gf, scale, seed, first_slot_index, d_i, d_q, slot_stride, n_samples);
-    else if (protocol == PROTO_FT4) synth_float_kernel<576, false><<<grid, 256, 0, st>>>(d_sigs, d_first, gf, scale, seed, first_slot_index, d_i, nullptr, slot_stride, n_samples);
-    else synth_float_kernel<1920, false><<<grid, 256, 0, st>>>(d_sigs, d_first, gf, scale, seed, first_slot_index, d_i, nullptr, slot_stride, n_samples);
-    const bool ok = cudaGetLastError() == cudaSuccess && cudaStreamSynchronize(st) == cudaSuccess;
+    bool ok = true;
+    for (int s0 = 0; ok && s0 < n_slots; s0 += kMaxGridRows) {   // the slot is blockIdx.y
+        const int rows = n_slots - s0 < kMaxGridRows ? n_slots - s0 : kMaxGridRows;
+        dim3 grid((unsigned)((n_samples + 255) / 256), (unsigned)rows);
+        const int *first = d_first + s0;
+        float *oi = d_i + (size_t)s0 * slot_stride, *oq = d_q ? d_q + (size_t)s0 * slot_stride : nullptr;
+        if (kind == 1) synth_float_kernel<512, true><<<grid, 256, 0, st>>>(d_sigs, first, gf, scale, seed, first_slot_index + s0, oi, oq, slot_stride, n_samples);
+        else if (protocol == PROTO_FT4) synth_float_kernel<576, false><<<grid, 256, 0, st>>>(d_sigs, first, gf, scale, seed, first_slot_index + s0, oi, nullptr, slot_stride, n_samples);
+        else synth_float_kernel<1920, false><<<grid, 256, 0, st>>>(d_sigs, first, gf, scale, seed, first_slot_index + s0, oi, nullptr, slot_stride, n_samples);
+        ok = cudaGetLastError() == cudaSuccess;
+    }
+    ok = ok && cudaStreamSynchronize(st) == cudaSuccess;
     cudaFree(d_sigs); cudaFree(d_first);
     return ok ? 0 : FT8B200_CUDA_FAIL();
 }
