@@ -88,8 +88,11 @@ __device__ __forceinline__ void bfly4(cpx &f0, cpx &f1, cpx &f2, cpx &f3, const 
     f1.r = __fadd_rn(d5.r, s4.i); f1.i = __fsub_rn(d5.i, s4.r);
     f3.r = __fsub_rn(d5.r, s4.i); f3.i = __fadd_rn(d5.i, s4.r);
 }
-// kiss_fft multiplies by twiddle 0 = (1, -0) like by any other; the product equals the input except possibly for the
-// sign of a zero, which cannot reach |X|^2 -- so index-0 twiddles are skipped WHERE THAT IS KNOWN AT COMPILE TIME (pass A).
+// kiss_fft multiplies by twiddle 0 = (1, -0) like by any other.  For a finite input the product equals the input except
+// possibly for the sign of a zero, which cannot reach |X|^2.  For a non-finite one it does not: inf * -0 is NaN, so kiss_fft
+// turns (inf, y) into (inf, NaN) where skipping keeps (inf, y).  That cannot change a byte either: every bin such a frame
+// reaches is then inf or NaN (no other twiddle has an exact zero component), and the quantiser maps both to 0
+// (test_non_finite_and_extreme_float_slots).  So index-0 twiddles are skipped WHERE THAT IS KNOWN AT COMPILE TIME (pass A).
 // Where it depends on the lane (i0 == 0 in pass B, i == 0 in pass C) the multiplication is simply performed, as kiss_fft
 // does: a per-lane special case made every warp execute both the twiddled and the untwiddled butterfly (2 of its 32 lanes
 // took the short path), which cost pass B half as much again as the arithmetic it saved.
