@@ -201,6 +201,8 @@ void orc_bp_decode(const float *llr, int max_iters, uint8_t *plain, int *errors_
     float c_in[FT8T_M][7];   /* "toc": tanh of variable -> check messages */
     int best = FT8T_M;
     memset(v2c_in, 0, sizeof(v2c_in));
+    /* ldpc.c leaves plain[] unwritten when no round runs (max_iters = 0); the kernels report the all-zero word */
+    memset(plain, 0, FT8T_N);
     for (int it = 0; it < max_iters; ++it) {
         int ones = 0;
         for (int n = 0; n < FT8T_N; ++n) {

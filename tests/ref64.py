@@ -12,6 +12,8 @@ Independence rules (what keeps these references from sharing a mistake with the 
 - The CRC-14 is implemented here as plain polynomial division; it is checked against tests/golden/kat.npz["crc_test3"],
   which the unmodified reference computed.
 - The daemon's FFT window is kat.npz["window"], which the reference recorded.
+- Belief propagation's tanh and atanh are the Pade approximants derived from their Taylor series (pade_coefficients());
+  only the tanh clamp (TANH_CLAMP) is taken from the reference's text.
 - The FFTs are numpy's float64 ones, not kiss_fft's float arithmetic, so results may differ from the kernels' by the
   north-star allowances (waterfall cells +-1 LSB on <= 0.01 % of cells, decimator floats 1e-5 relative), never by more.
 """
@@ -264,6 +266,155 @@ def llrs(mag, cand, num_blocks, num_bins, time_osr, freq_osr, protocol=1):
     var = (np.sum(x * x) - np.sum(x) ** 2 / 174.0) / 174.0
     with np.errstate(divide="ignore", invalid="ignore"):
         return x * np.sqrt(24.0 / var), var
+
+
+# ---- belief propagation (ft8_lib ldpc.c:130-251) ----------------------------------------------------------------------
+# ft8_lib's tanh clamp, the one BP constant taken from the reference's text: fast_tanh returns -+1 beyond it.  The [5/4]
+# approximant reaches 1.007 at 4.97, so the clamp is a small step, not a smooth joint.
+TANH_CLAMP = 4.97
+
+
+def pade_coefficients(f, m=5, n=4):
+    """The [m/n] Pade approximant of tanh or atanh (f = "tanh" / "atanh") from its Taylor series at 0, scaled so that the
+    denominator's constant term is 945 and rounded to the integers the scaling gives -> (numerator, denominator)
+    ascending in powers of x.  The rounding is checked, so a series that does not give integers raises."""
+    import mpmath
+    with mpmath.workdps(40):
+        p, q = mpmath.pade(mpmath.taylor(getattr(mpmath, f), 0, m + n), m, n)
+        scale = 945 / q[0]
+        out = []
+        for c in (p, q):
+            v = [c_ * scale for c_ in c]
+            r = [int(mpmath.nint(x)) for x in v]
+            assert all(abs(x - k) < mpmath.mpf(10) ** -30 for x, k in zip(v, r)), (f, v)
+            out.append(tuple(r))
+    return tuple(out)
+
+
+def _pade(x, coefs):
+    num, den = coefs
+    return np.polynomial.polynomial.polyval(x, num) / np.polynomial.polynomial.polyval(x, den)
+
+
+_BP_GRAPH = None
+
+
+def _bp_graph():
+    """Edges of the check rows as (row m, position j, variable n), in row order, and the 0/1 edge -> variable matrix."""
+    global _BP_GRAPH
+    if _BP_GRAPH is None:
+        nm = ldpc_checks()
+        m_idx, j_idx = np.nonzero(nm >= 0)
+        n_idx = nm[m_idx, j_idx]
+        A = np.zeros((m_idx.size, 174))
+        A[np.arange(m_idx.size), n_idx] = 1.0
+        _BP_GRAPH = (m_idx, j_idx, n_idx, A, nm.shape)
+    return _BP_GRAPH
+
+
+def bp_decode64(llr, max_rounds):
+    """Flooding sum-product decoding in float64 on ft8_lib's schedule, for C candidates at once (llr: [C, 174]).
+
+    Check -> variable messages (tov) start at 0.  Each round first takes the hard decision bit = (llr + sum of tov) > 0;
+    an all-zero word stops the run (not a message); otherwise the parity errors are counted, the minimum is kept, and 0
+    errors stops the run.  Then every variable sends its check t = tanh(-(llr + the other two tov) / 2), and every check
+    sends its variables tov = -2 atanh(product of the row's other t).  tanh and atanh are the [5/4] Pade approximants of
+    pade_coefficients(), tanh clamped to -+1 beyond TANH_CLAMP.
+
+    Returns the trajectory over the rounds each candidate executes (round r = 1 .. max_rounds):
+      bits   uint8 [R, C, 174]  the hard decision of round r
+      errors int   [R, C]       its parity errors (83 - like the minimum's start - in an all-zero round, which counts none)
+      margin float [R, C]       the smallest |llr + sum of tov| over the 174 posteriors of round r (NaN posteriors ignored)
+      ran    bool  [R, C]       whether the candidate executed round r
+      stop   int   [C]          the round that stopped the run (0: none did within max_rounds)
+      zero   bool  [C]          the stopping round's word was all zero (else it satisfied every check)
+    bp_at() turns this into what a decoder limited to n rounds outputs."""
+    x = np.asarray(llr, np.float64)
+    C = x.shape[0]
+    m_idx, j_idx, n_idx, A, shape = _bp_graph()
+    th, ath = pade_coefficients("tanh"), pade_coefficients("atanh")
+    R = max_rounds
+    bits = np.zeros((R, C, 174), np.uint8)
+    errors = np.full((R, C), 83, np.int64)
+    margin = np.full((R, C), np.inf)
+    ran = np.zeros((R, C), bool)
+    stop = np.zeros(C, np.int64)
+    zero = np.zeros(C, bool)
+    H = parity_matrix().T.astype(np.int64)
+    tov = np.zeros((C, m_idx.size))
+    live = np.arange(C)
+    for r in range(R):
+        if live.size == 0:
+            break
+        xl, tl = x[live], tov[live]
+        post = xl + tl @ A
+        b = post > 0
+        ran[r, live] = True
+        bits[r, live] = b
+        with np.errstate(invalid="ignore"):
+            margin[r, live] = np.where(np.isnan(post), np.inf, np.abs(post)).min(axis=1)
+        ones = b.any(axis=1)
+        err = (b.astype(np.int64) @ H % 2).sum(axis=1)
+        errors[r, live] = np.where(ones, err, 83)
+        done = ~ones | (err == 0)
+        stop[live[done]] = r + 1
+        zero[live[done]] = ~ones[done]
+        keep = ~done
+        live, post, tl = live[keep], post[keep], tl[keep]
+        if live.size == 0 or r + 1 == R:
+            break
+        t = -(post[:, n_idx] - tl) / 2                                  # llr + the variable's other two tov, halved, negated
+        with np.errstate(invalid="ignore"):
+            v = np.where(t < -TANH_CLAMP, -1.0, np.where(t > TANH_CLAMP, 1.0, _pade(t, th)))
+        toc = np.ones((live.size,) + shape)
+        toc[:, m_idx, j_idx] = v
+        one = np.ones((live.size, shape[0], 1))
+        pre = np.cumprod(np.concatenate([one, toc[:, :, :-1]], axis=2), axis=2)               # positions before j
+        suf = np.cumprod(np.concatenate([one, toc[:, :, :0:-1]], axis=2), axis=2)[:, :, ::-1]  # positions after j
+        others = (pre * suf)[:, m_idx, j_idx]                           # product of the row's other positions
+        tov[live] = -2.0 * _pade(others, ath)
+    return dict(bits=bits, errors=errors, margin=margin, ran=ran, stop=stop, zero=zero)
+
+
+def bp_at(traj, n):
+    """What a decoder limited to n rounds outputs, from bp_decode64's trajectory (n <= its max_rounds):
+    -> (plain uint8 [C, 174]: the last executed round's hard decision, zeros for n = 0;
+        ldpc_errors [C]: the minimum parity errors over the executed rounds, 83 when none counted;
+        rounds [C]: how many rounds ran)."""
+    C = traj["stop"].size
+    rounds = np.where(traj["stop"] > 0, np.minimum(traj["stop"], n), n)
+    plain = np.zeros((C, 174), np.uint8)
+    errors = np.full(C, 83, np.int64)
+    for c in range(C):
+        k = int(rounds[c])
+        if k:
+            plain[c] = traj["bits"][k - 1, c]
+            errors[c] = min(83, int(traj["errors"][:k, c].min()))
+    return plain, errors, rounds
+
+
+# The agreement rule between a float32 decoder and bp_decode64: a (candidate, n) pair is resolved when every posterior of
+# every round the float64 run executes up to n, after the first, is at least TAU x max|llr| in magnitude, and at least
+# TAU_LONG x max|llr| from round LONG_ROUNDS + 1 on.  Round 1's posteriors are the LLRs themselves, the same numbers in both;
+# NaN posteriors compare false in both.  Runs that go on past LONG_ROUNDS without converging wander, and float32 rounding
+# then grows until a posterior flips: seen between rounds 50 and 100 at margins up to 6e-4 x max|llr|.
+TAU, TAU_LONG, LONG_ROUNDS = 1e-5, 1e-2, 50
+
+
+def bp_resolved(traj, llr, n):
+    """(plain, ldpc_errors, margin) of the float64 run at n; margin is the smallest posterior magnitude over the rounds the
+    rule covers, in units of that round's bar, so that the pair is resolved when margin >= 1."""
+    plain, errors, rounds = bp_at(traj, n)
+    x = np.abs(np.asarray(llr, np.float64))
+    with np.errstate(all="ignore"):
+        scale = np.max(np.where(np.isnan(x), -np.inf, x), axis=1)
+        bar = np.where(np.arange(traj["margin"].shape[0]) < LONG_ROUNDS, TAU, TAU_LONG)[:, None] * scale[None, :]
+        rel = traj["margin"] / bar
+    rel = np.where(np.isnan(rel), np.inf, rel)
+    rel[0] = np.inf
+    cm = np.minimum.accumulate(rel, axis=0)
+    idx = np.maximum(rounds - 1, 0)
+    return plain, errors, np.where(rounds > 0, cm[idx, np.arange(idx.size)], np.inf)
 
 
 # ---- channel symbols --------------------------------------------------------------------------------------------------
