@@ -277,6 +277,31 @@ int ft8b200_osd(ft8b200_ctx_t *ctx, const float *d_llr, int n_slots, const int *
                 void *stream);
 /* d_osd / d_osd_hard (as above) of the last process_* or decode batch run with OSD on (n_slots x max_candidates); NULL before that */
 int ft8b200_osd_workspace(ft8b200_ctx_t *ctx, uint8_t **d_osd, int32_t **d_osd_hard);
+/* Multi-pass decoding (DESIGN.md section 2.4.2) on the daemon path -- every process_raw*, process_slots / process_conditioned call,
+ * and through them the pipe, the cluster, the drop-in ft8_subsystem, the stream and .iq file paths.  passes = 1 (default) decodes
+ * a slot once, exactly as without this call.  With 2 or 3, after each pass the messages the spot table accepted as new in that
+ * pass (in acceptance order; duplicates and messages dropped by a full table are not) are subtracted from the pass's input as
+ * unit-amplitude GFSK waveforms (ft8b200_subtract), and the residual is searched again: waterfall with the slot's original peak
+ * scale, find_sync (same max_candidates and min_score), decode (+ OSD when on), and the spot table in append mode -- it keeps the
+ * slot's earlier records, de-duplicates against every earlier pass by hash and text, and appends new records behind them (freq and
+ * snr from the new candidate).  A slot with nothing new in a pass is not searched again.  Pass 1's outputs (records, workspace
+ * rows) are those of passes = 1; the later passes only append.  The later passes use their own context workspaces, allocated only
+ * with passes > 1.  ft8b200_stage_times reports subtraction + later passes as a seventh stage.
+ * Out of scope: the 12 kHz audio entry points (ft8b200_decode_audio, decode_ft8 and the monitor), whose geometry differs.
+ * Any passes other than 1, 2 or 3 is FT8B200_EINVAL. */
+int ft8b200_set_passes(ft8b200_ctx_t *ctx, int passes);
+/* Stage-wise subtraction of decoded FT8 messages from daemon slots (3200 sps complex, FT8B200_SLOT_SAMPLES floats per slot row,
+ * dense).  Slot s has d_nmsg[s] (clamped to 0 ... max_messages) messages: d_cand[s][j] (candidate_t, max_messages per slot)
+ * and d_cw[s][j] (174 bytes, one codeword bit per byte, ft8b200_decode's d_plain order).  Each message's start sample and tone-0
+ * frequency follow from its candidate (s0 = 512 time_offset + 256 time_sub + 256, f0 = 3.125 (2 freq_offset + freq_sub) Hz);
+ * the GFSK reference is refined on the INPUT slot over dt = -128 ... +128 samples (step 16) x df = -8 ... +8 steps of 6.25/32 Hz,
+ * then dt +- 8 samples at the chosen df, and d_grid[s][j] = {dt in samples, df in steps} receives the result.  The messages are
+ * then subtracted in list order, each with the amplitude of the residual against it smoothed by a 1025-tap Hann window:
+ * d_ri / d_rq (same layout as d_i / d_q; may be d_i / d_q themselves, not otherwise overlapping) receive the residual.
+ * The subtraction is linear in the samples, so no peak scale is needed: conditioned or unconditioned slots give the residual of
+ * what was passed in.  tests/subtract_ref.py is the float64 definition. */
+int ft8b200_subtract(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, int n_slots, const candidate_t *d_cand, const uint8_t *d_cw,
+                     const int32_t *d_nmsg, float *d_ri, float *d_rq, int32_t *d_grid, void *stream);
 
 /* a15: the daemon's duplicate table + CQ filter, one slot per thread.  d_results: n_slots x max_messages
  * (zeroed here first), d_nresults: n_slots; optional first-seen unique message log: d_umsg (n_slots x
@@ -426,6 +451,8 @@ int ft8b200_pipe_set_back_chain(ft8b200_pipe_t *p, int on);
 /* ft8b200_set_osd on every lane (a cluster's pipes through ft8b200_cluster_pipe).  FT8B200_EBUSY while batches are in flight;
  * ft8b200_osd_workspace of a lane is not exposed: the pipe returns spot records only. */
 int ft8b200_pipe_set_osd(ft8b200_pipe_t *p, int order, int max_hard_errors);
+/* ft8b200_set_passes on every lane (a cluster's pipes through ft8b200_cluster_pipe).  FT8B200_EBUSY while batches are in flight. */
+int ft8b200_pipe_set_passes(ft8b200_pipe_t *p, int passes);
 int ft8b200_pipe_autotune(ft8b200_pipe_t *p, const uint8_t *d_iq, size_t bytes_per_stream, size_t stream_stride_bytes, int n_slots,
                           const int *candidates, int n_candidates, int batches, int *best_back_sms, int *best_comb_front, float *ms_out);
 void ft8b200_pipe_destroy(ft8b200_pipe_t *p);

@@ -283,6 +283,21 @@ class Context:
                                      _p(cw), _st(stream)))
         return osd, hard, cw
 
+    def set_passes(self, passes: int):
+        """Multi-pass decoding with signal subtraction on the daemon path: 1 (default, one pass), 2 or 3 (ft8b200_set_passes)."""
+        self._chk(self.L.ft8b200_set_passes(C.c_void_p(self.h), int(passes)))
+
+    def subtract(self, d_i, d_q, cand, cw, nmsg, out=None, stream: int | None = None):
+        """Stage-wise ft8b200_subtract: slots float32 [n, 48000] (I, Q), per slot up to M messages -- cand uint8 [n, M, 8]
+        (candidate_t), cw uint8 [n, M, 174] (codeword bits), nmsg int32 [n] -> (residual I, residual Q, grid int32 [n, M, 2] of
+        (dt samples, df steps)).  out = (ri, rq) to write the residual into (may be d_i, d_q)."""
+        import torch
+        n = d_i.shape[0]
+        ri, rq = out if out is not None else (torch.empty_like(d_i), torch.empty_like(d_q))
+        grid = torch.zeros((n, self.M, 2), dtype=torch.int32, device=d_i.device)
+        self._chk(self.L.ft8b200_subtract(C.c_void_p(self.h), _p(d_i), _p(d_q), n, _p(cand), _p(cw), _p(nmsg), _p(ri), _p(rq), _p(grid), _st(stream)))
+        return ri, rq, grid
+
     def osd_workspace_ptrs(self):
         """Device pointers (osd, osd_hard) of the last batch decoded with OSD on (0 before that)."""
         a, b = C.c_void_p(0), C.c_void_p(0)
@@ -418,10 +433,12 @@ class Context:
         self._chk(self.L.ft8b200_set_overlap(C.c_void_p(self.h), int(groups)))
 
     def stage_times(self):
-        """ms per stage of the last process_* call: dict(block_sums, comb_fir, waterfall, sync, decode, spots)."""
-        ms = (C.c_float * 6)()
-        self._chk(self.L.ft8b200_stage_times(C.c_void_p(self.h), ms, 6))
-        return dict(zip(("block_sums", "comb_fir", "waterfall", "sync", "decode", "spots"), [float(x) for x in ms]))
+        """ms per stage of the last process_* call: dict(block_sums, comb_fir, waterfall, sync, decode, spots), and later_passes
+        (subtraction + passes 2 and 3) when the context decodes in more than one pass."""
+        ms = (C.c_float * 7)(*([-2.0] * 7))
+        self._chk(self.L.ft8b200_stage_times(C.c_void_p(self.h), ms, 7))
+        names = ("block_sums", "comb_fir", "waterfall", "sync", "decode", "spots", "later_passes")
+        return {k: float(x) for k, x in zip(names, ms) if x != -2.0}
 
     def results_device_ptrs(self):
         a, b = C.c_void_p(0), C.c_void_p(0)
@@ -529,6 +546,10 @@ class Pipe:
     def set_osd(self, order: int, max_hard_errors: int = -1):
         """Context.set_osd on every lane; not while batches are in flight."""
         self._chk(self.L.ft8b200_pipe_set_osd(C.c_void_p(self.h), int(order), int(max_hard_errors)))
+
+    def set_passes(self, passes: int):
+        """Context.set_passes on every lane; not while batches are in flight."""
+        self._chk(self.L.ft8b200_pipe_set_passes(C.c_void_p(self.h), int(passes)))
 
     def set_back_chain(self, on: bool):
         """Back ends of consecutive batches serialised on the back partition (what the autotune probes with)."""

@@ -80,6 +80,12 @@ struct ft8b200_ctx {
     int osd_order = 0;
     int osd_max_hard = FT8B200_OSD_DEFAULT_MAX_HARD;
     DevBuf llr, osd, osd_hard;
+    // multi-pass decoding (ft8b200_set_passes): 1 = off.  With passes > 1: the codewords of pass 1 (plain), the slot's log of accepted
+    // messages across passes (ulog/ufreq/uscore/ucand, first = record count before the last pass), the refined grid points, the
+    // residual slots (ri/rq), and the rows of the later passes (pass 1 keeps the rows above)
+    int passes = 1;
+    DevBuf plain, ulog, ufreq, uscore, ucand, first, grid, ri, rq, sub_scratch;
+    DevBuf mag2, cand2, ncand2, ok2, stage2, status2, msg2, plain2, llr2, osd2, osd_hard2;
     // optional per-stage timing of the last process_* call (CUDA events on the launching stream)
     bool profiling = false;
     int overlap = 0;                       // number of slot groups ft8b200_process_raw pipelines (0/1 = off)
@@ -92,8 +98,8 @@ struct ft8b200_ctx {
     cudaEvent_t ev_k1 = nullptr;
     cudaEvent_t ev_back = nullptr;         // recorded on the back-end stream behind the last process_raw's spot table (ft8b200_back_event)
     cudaEvent_t back_wait = nullptr;       // one-shot: the next process_raw's back end waits for it (ft8b200_set_back_wait)
-    cudaEvent_t ev[6][kMaxGroups][2] = {};
-    bool ev_valid[6][kMaxGroups] = {};
+    cudaEvent_t ev[7][kMaxGroups][2] = {};   // stage 6: subtraction and the later passes (passes > 1)
+    bool ev_valid[7][kMaxGroups] = {};
     cudaStream_t aux = nullptr;            // high-priority side stream for the back end of a slot group
     cudaStream_t own_aux = nullptr;
     int sm_back = 0;                       // SMs the back-end kernels size their persistent grids for (0 = sm_count)
@@ -124,6 +130,27 @@ int ensure_osd_buffers(ft8b200_ctx_t *ctx, int n_slots) {
     return ctx->osd_hard.ensure(E * sizeof(int32_t));
 }
 
+int ensure_pass_buffers(ft8b200_ctx_t *ctx, int n_slots) {
+    const size_t K = (size_t)ctx->cfg.max_candidates, M = (size_t)ctx->cfg.max_messages, S = (size_t)n_slots;
+    int rc;
+    DevBuf *rows[] = {&ctx->ok2, &ctx->stage2};
+    for (DevBuf *b : rows) if ((rc = b->ensure(S * K))) return rc;
+    if ((rc = ctx->plain.ensure(S * K * kLdpcN)) || (rc = ctx->plain2.ensure(S * K * kLdpcN))) return rc;
+    if ((rc = ctx->ulog.ensure(S * M * sizeof(message_t))) || (rc = ctx->ufreq.ensure(S * M * sizeof(float)))) return rc;
+    if ((rc = ctx->uscore.ensure(S * M * sizeof(int32_t))) || (rc = ctx->ucand.ensure(S * M * sizeof(int32_t)))) return rc;
+    if ((rc = ctx->first.ensure(S * sizeof(int32_t))) || (rc = ctx->grid.ensure(S * M * 2 * sizeof(int32_t)))) return rc;
+    if ((rc = ctx->ri.ensure(S * kSlot * sizeof(float))) || (rc = ctx->rq.ensure(S * kSlot * sizeof(float)))) return rc;
+    if ((rc = ctx->sub_scratch.ensure(subtract_scratch_bytes(n_slots, ctx->sm_count)))) return rc;
+    if ((rc = ctx->mag2.ensure(S * kWfBytes)) || (rc = ctx->cand2.ensure(S * K * sizeof(candidate_t)))) return rc;
+    if ((rc = ctx->ncand2.ensure(S * sizeof(int))) || (rc = ctx->status2.ensure(S * K * sizeof(decode_status_t)))) return rc;
+    if ((rc = ctx->msg2.ensure(S * K * sizeof(message_t)))) return rc;
+    if (ctx->osd_order) {
+        if ((rc = ctx->llr2.ensure(S * K * kLdpcN * sizeof(float))) || (rc = ctx->osd2.ensure(S * K))) return rc;
+        if ((rc = ctx->osd_hard2.ensure(S * K * sizeof(int32_t)))) return rc;
+    }
+    return 0;
+}
+
 int ensure_slot_buffers(ft8b200_ctx_t *ctx, int n_slots) {
     const size_t K = (size_t)ctx->cfg.max_candidates, M = (size_t)ctx->cfg.max_messages, S = (size_t)n_slots;
     int rc;
@@ -138,6 +165,7 @@ int ensure_slot_buffers(ft8b200_ctx_t *ctx, int n_slots) {
     if ((rc = ctx->nresults.ensure(S * sizeof(int32_t)))) return rc;
     if ((rc = ctx->table.ensure(S * M * sizeof(int16_t)))) return rc;
     if (ctx->osd_order && (rc = ensure_osd_buffers(ctx, n_slots))) return rc;
+    if (ctx->passes > 1 && (rc = ensure_pass_buffers(ctx, n_slots))) return rc;
     return 0;
 }
 
@@ -217,6 +245,7 @@ ft8b200_ctx_t *ft8b200_create(const ft8b200_config_t *cfg_in) {
     okc = okc && cudaMemcpy(ctx->tb.db_thresholds, thr.data(), 257 * sizeof(float), cudaMemcpyHostToDevice) == cudaSuccess;
     okc = okc && upload_fir_constants() == cudaSuccess;
     okc = okc && upload_ldpc_tables() == cudaSuccess;
+    okc = okc && upload_subtract_tables() == cudaSuccess;
     {
         std::vector<float> blob(waterfall_blob_floats());
         build_waterfall_tables(win.data(), tw.data(), thr.data(), blob.data());
@@ -248,7 +277,9 @@ void ft8b200_destroy(ft8b200_ctx_t *ctx) {
     cudaFree(ctx->tb.mon_window); cudaFree(ctx->tb.mon_twiddle); cudaFree(ctx->tb.mon_super);
     DevBuf *bufs[] = {&ctx->raw, &ctx->sums, &ctx->si, &ctx->sq, &ctx->peak, &ctx->count, &ctx->mag, &ctx->cand, &ctx->ncand, &ctx->ok,
                       &ctx->stage, &ctx->status, &ctx->msg, &ctx->results, &ctx->nresults, &ctx->table, &ctx->lists, &ctx->scores, &ctx->work, &ctx->work_total,
-                      &ctx->llr, &ctx->osd, &ctx->osd_hard};
+                      &ctx->llr, &ctx->osd, &ctx->osd_hard, &ctx->plain, &ctx->ulog, &ctx->ufreq, &ctx->uscore, &ctx->ucand, &ctx->first,
+                      &ctx->grid, &ctx->ri, &ctx->rq, &ctx->sub_scratch, &ctx->mag2, &ctx->cand2, &ctx->ncand2, &ctx->ok2, &ctx->stage2,
+                      &ctx->status2, &ctx->msg2, &ctx->plain2, &ctx->llr2, &ctx->osd2, &ctx->osd_hard2};
     for (DevBuf *b : bufs) b->release();
     delete ctx;
 }
@@ -428,6 +459,30 @@ int ft8b200_set_osd(ft8b200_ctx_t *ctx, int order, int max_hard_errors) {
     return 0;
 }
 
+int ft8b200_set_passes(ft8b200_ctx_t *ctx, int passes) {
+    if (!ctx) return fail(FT8B200_EINVAL, "null context");
+    if (passes < 1 || passes > 3) return fail(FT8B200_EINVAL, "ft8b200_set_passes: passes must be 1 (one pass, the default), 2 or 3");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    ctx->passes = passes;
+    return 0;
+}
+
+int ft8b200_subtract(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, int n_slots, const candidate_t *d_cand, const uint8_t *d_cw,
+                     const int32_t *d_nmsg, float *d_ri, float *d_rq, int32_t *d_grid, void *stream) {
+    int rc = ctx_enter(ctx);
+    if (rc) return rc;
+    if (!d_i || !d_q || !d_cand || !d_cw || !d_nmsg || !d_ri || !d_rq || !d_grid || n_slots < 1 || n_slots > FT8B200_MAX_RAW_ROWS)
+        return fail(FT8B200_EINVAL, "ft8b200_subtract: null buffer or n_slots outside 1 ... 65535");
+    if ((((size_t)d_i) | ((size_t)d_q) | ((size_t)d_ri) | ((size_t)d_rq)) & 3) return fail(FT8B200_EINVAL, "ft8b200_subtract: float buffers must be 4-byte aligned");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    if ((rc = ctx->sub_scratch.ensure(subtract_scratch_bytes(n_slots, ctx->sm_count)))) return rc;
+    const int M = ctx->cfg.max_messages;
+    CU(launch_subtract(d_i, d_q, d_ri, d_rq, n_slots, d_cand, d_cw, M, nullptr, nullptr, d_nmsg, M, d_grid, ctx->sub_scratch.as<float2>(), false,
+                       ctx->sm_count, pick(ctx, stream), &ctx->launches));
+    tally(ctx);
+    return 0;
+}
+
 int ft8b200_osd(ft8b200_ctx_t *ctx, const float *d_llr, int n_slots, const int *d_ncand, uint8_t *d_ok, uint8_t *d_stage, decode_status_t *d_status,
                 message_t *d_msg, uint8_t *d_plain, uint8_t *d_osd, int32_t *d_osd_hard, uint8_t *d_osd_cw, void *stream) {
     int rc = ctx_enter(ctx);
@@ -465,7 +520,9 @@ static void clear_marks(ft8b200_ctx_t *ctx) {
     for (auto &s : ctx->ev_valid) for (bool &v : s) v = false;
 }
 
-// waterfall -> sync -> decode -> spots for slots [s0, s0+n) of the context buffers, all on `st`
+// waterfall -> sync -> decode -> spots for slots [s0, s0+n) of the context buffers, all on `st`; with passes > 1 the decoded
+// messages are then subtracted and the residual searched again (later_passes)
+static int later_passes(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, const float *d_peak, int s0, int n, int sms, cudaStream_t st);
 static int run_back_end(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, const float *d_peak, int s0, int n, int group, cudaStream_t st) {
     const size_t K = (size_t)ctx->cfg.max_candidates, M = (size_t)ctx->cfg.max_messages;
     uint8_t *mag = ctx->mag.as<uint8_t>() + (size_t)s0 * kWfBytes;
@@ -484,20 +541,77 @@ static int run_back_end(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, 
     mark(ctx, 3, group, true, st);
     mark(ctx, 4, group, false, st);
     float *llr = ctx->osd_order ? ctx->llr.as<float>() + (size_t)s0 * K * kLdpcN : nullptr;
+    const bool multi = ctx->passes > 1;
+    uint8_t *plain = multi ? ctx->plain.as<uint8_t>() + (size_t)s0 * K * kLdpcN : nullptr;   // the codewords subtraction needs
     CU(launch_decode(mag, kWfBytes, n, 92, 256, 2, 2, PROTO_FT8, ctx->cfg.max_candidates, ctx->cfg.ldpc_iterations, cand, ncand, ok, stage,
-                     ctx->status.as<decode_status_t>() + (size_t)s0 * K, ctx->msg.as<message_t>() + (size_t)s0 * K, nullptr, llr,
+                     ctx->status.as<decode_status_t>() + (size_t)s0 * K, ctx->msg.as<message_t>() + (size_t)s0 * K, plain, llr,
                      ctx->work.as<uint32_t>(), ctx->work_total.as<unsigned int>(), sms, st, &ctx->launches));
     if (ctx->osd_order)  // the work list's entries BP left at stage 1 or 2; word [2] of work_total (zeroed by launch_find_sync) is its pull counter
         CU(launch_osd(n, ctx->cfg.max_candidates, PROTO_FT8, ctx->osd_order, ctx->osd_max_hard, llr, ncand, ok, stage,
-                      ctx->status.as<decode_status_t>() + (size_t)s0 * K, ctx->msg.as<message_t>() + (size_t)s0 * K, nullptr,
+                      ctx->status.as<decode_status_t>() + (size_t)s0 * K, ctx->msg.as<message_t>() + (size_t)s0 * K, plain,
                       ctx->osd.as<uint8_t>() + (size_t)s0 * K, ctx->osd_hard.as<int32_t>() + (size_t)s0 * K, nullptr, ctx->work.as<uint32_t>(),
                       ctx->work_total.as<unsigned int>(), ctx->work_total.as<unsigned int>() + 2, sms, st, &ctx->launches));
     mark(ctx, 4, group, true, st);
     mark(ctx, 5, group, false, st);
-    CU(launch_spots(n, ctx->cfg.max_candidates, ctx->cfg.max_messages, ctx->cfg.min_score, 2, cand, ncand, ok, ctx->msg.as<message_t>() + (size_t)s0 * K,
-                    ctx->results.as<struct decoder_results>() + (size_t)s0 * M, ctx->nresults.as<int32_t>() + s0, nullptr, nullptr, nullptr, nullptr,
-                    ctx->table.as<int16_t>() + (size_t)s0 * M, st, &ctx->launches));
+    if (!multi) {
+        CU(launch_spots(n, ctx->cfg.max_candidates, ctx->cfg.max_messages, ctx->cfg.min_score, 2, cand, ncand, ok, ctx->msg.as<message_t>() + (size_t)s0 * K,
+                        ctx->results.as<struct decoder_results>() + (size_t)s0 * M, ctx->nresults.as<int32_t>() + s0, nullptr, nullptr, nullptr, nullptr,
+                        ctx->table.as<int16_t>() + (size_t)s0 * M, st, &ctx->launches));
+    } else {   // the same table, which also logs what it accepts, in order, for the subtraction and the later passes' de-duplication
+        CU(launch_spots(n, ctx->cfg.max_candidates, ctx->cfg.max_messages, ctx->cfg.min_score, 2, cand, ncand, ok, ctx->msg.as<message_t>() + (size_t)s0 * K,
+                        ctx->results.as<struct decoder_results>() + (size_t)s0 * M, ctx->nresults.as<int32_t>() + s0, ctx->ulog.as<message_t>() + (size_t)s0 * M,
+                        ctx->ufreq.as<float>() + (size_t)s0 * M, ctx->uscore.as<int32_t>() + (size_t)s0 * M, ctx->ucand.as<int32_t>() + (size_t)s0 * M,
+                        ctx->table.as<int16_t>() + (size_t)s0 * M, st, &ctx->launches, false, ctx->first.as<int32_t>() + s0));
+    }
     mark(ctx, 5, group, true, st);
+    if (multi) {
+        mark(ctx, 6, group, false, st);
+        if (int rc = later_passes(ctx, d_i, d_q, d_peak, s0, n, sms, st)) return rc;
+        mark(ctx, 6, group, true, st);
+    }
+    return 0;
+}
+
+// Pass p >= 2 (DESIGN.md section 2.4.2): the messages pass p - 1 accepted as new (log entries [first, nresults) of each slot) are
+// refined on that pass's input x and subtracted from it into the residual slots (in place from pass 3 on); a slot with none gets a
+// zero residual and so no candidates.  The residual goes through waterfall (with the slot's original peak scale: the quantiser is
+// absolute), sync, decode (+ OSD) into the later-pass rows, and the spot table appends what is new.
+static int later_passes(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, const float *d_peak, int s0, int n, int sms, cudaStream_t st) {
+    const size_t K = (size_t)ctx->cfg.max_candidates, M = (size_t)ctx->cfg.max_messages;
+    const float *xi = d_i + (size_t)s0 * kSlot, *xq = d_q + (size_t)s0 * kSlot;
+    float *ri = ctx->ri.as<float>() + (size_t)s0 * kSlot, *rq = ctx->rq.as<float>() + (size_t)s0 * kSlot;
+    const candidate_t *prev_cand = ctx->cand.as<candidate_t>() + (size_t)s0 * K;
+    const uint8_t *prev_plain = ctx->plain.as<uint8_t>() + (size_t)s0 * K * kLdpcN;
+    uint8_t *mag = ctx->mag2.as<uint8_t>() + (size_t)s0 * kWfBytes;
+    candidate_t *cand = ctx->cand2.as<candidate_t>() + (size_t)s0 * K;
+    int *ncand = ctx->ncand2.as<int>() + s0;
+    uint8_t *ok = ctx->ok2.as<uint8_t>() + (size_t)s0 * K, *stage = ctx->stage2.as<uint8_t>() + (size_t)s0 * K;
+    decode_status_t *status = ctx->status2.as<decode_status_t>() + (size_t)s0 * K;
+    message_t *msg = ctx->msg2.as<message_t>() + (size_t)s0 * K;
+    uint8_t *plain = ctx->plain2.as<uint8_t>() + (size_t)s0 * K * kLdpcN;
+    float *llr = ctx->osd_order ? ctx->llr2.as<float>() + (size_t)s0 * K * kLdpcN : nullptr;
+    int32_t *first = ctx->first.as<int32_t>() + s0, *nres = ctx->nresults.as<int32_t>() + s0, *ucand = ctx->ucand.as<int32_t>() + (size_t)s0 * M;
+    for (int p = 2; p <= ctx->passes; ++p) {
+        CU(launch_subtract(xi, xq, ri, rq, n, prev_cand, prev_plain, (int)K, ucand, first, nres, (int)M, ctx->grid.as<int32_t>() + (size_t)s0 * M * 2,
+                           ctx->sub_scratch.as<float2>(), true, sms, st, &ctx->launches));
+        xi = ri;
+        xq = rq;
+        CU(launch_waterfall(ctx->tb, ri, rq, d_peak ? d_peak + s0 : nullptr, n, mag, sms, st, &ctx->launches));
+        CU(launch_find_sync(mag, kWfBytes, n, 92, 256, 2, 2, PROTO_FT8, ctx->cfg.max_candidates, ctx->cfg.min_score, cand, ncand, ctx->scores.as<int16_t>(),
+                            ctx->lists.as<uint32_t>(), ctx->work.as<uint32_t>(), ctx->work_total.as<unsigned int>(), sms, st, &ctx->launches));
+        CU(launch_decode(mag, kWfBytes, n, 92, 256, 2, 2, PROTO_FT8, ctx->cfg.max_candidates, ctx->cfg.ldpc_iterations, cand, ncand, ok, stage, status, msg,
+                         plain, llr, ctx->work.as<uint32_t>(), ctx->work_total.as<unsigned int>(), sms, st, &ctx->launches));
+        if (ctx->osd_order)
+            CU(launch_osd(n, ctx->cfg.max_candidates, PROTO_FT8, ctx->osd_order, ctx->osd_max_hard, llr, ncand, ok, stage, status, msg, plain,
+                          ctx->osd2.as<uint8_t>() + (size_t)s0 * K, ctx->osd_hard2.as<int32_t>() + (size_t)s0 * K, nullptr, ctx->work.as<uint32_t>(),
+                          ctx->work_total.as<unsigned int>(), ctx->work_total.as<unsigned int>() + 2, sms, st, &ctx->launches));
+        CU(launch_spots(n, ctx->cfg.max_candidates, ctx->cfg.max_messages, ctx->cfg.min_score, 2, cand, ncand, ok, msg,
+                        ctx->results.as<struct decoder_results>() + (size_t)s0 * M, nres, ctx->ulog.as<message_t>() + (size_t)s0 * M,
+                        ctx->ufreq.as<float>() + (size_t)s0 * M, ctx->uscore.as<int32_t>() + (size_t)s0 * M, ucand, ctx->table.as<int16_t>() + (size_t)s0 * M,
+                        st, &ctx->launches, true, first));
+        prev_cand = cand;
+        prev_plain = plain;
+    }
     return 0;
 }
 
@@ -757,12 +871,13 @@ void *ft8b200_front_event(ft8b200_ctx_t *ctx) { return ctx ? ctx->ev_front : nul
 
 // ms[0..5] = block sums, comb+FIR, waterfall, sync, decode, spots of the last process_* call, summed over its slot
 // groups (-1 = stage not run).  With overlap on, front-end and back-end stages run concurrently: the sum of the stage
-// times then exceeds the wall time of the call.
+// times then exceeds the wall time of the call.  ms[6] (written only when n >= 7 and passes > 1): subtraction and the later passes.
 int ft8b200_stage_times(ft8b200_ctx_t *ctx, float *ms, int n) {
     int rc = ctx_enter(ctx);
     if (rc) return rc;
     if (!ms || n < 6) return fail(FT8B200_EINVAL, "ft8b200_stage_times: need room for 6 floats");
-    for (int k = 0; k < 6; ++k) {
+    const int stages = (n >= 7 && ctx->passes > 1) ? 7 : 6;
+    for (int k = 0; k < stages; ++k) {
         float total = 0.0f;
         bool any = false;
         for (int g = 0; g < kMaxGroups; ++g) {

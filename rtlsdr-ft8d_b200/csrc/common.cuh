@@ -66,13 +66,25 @@ cudaError_t launch_decode(const uint8_t *d_mag, size_t slot_stride, int n_slots,
                           unsigned int *d_work_total, int sm_count, cudaStream_t st, int *launches);
 cudaError_t launch_spots(int n_slots, int max_cand, int max_msgs, int min_score, int freq_osr, const candidate_t *d_cand, const int *d_ncand,
                          const uint8_t *d_ok, const message_t *d_msg, struct decoder_results *d_results, int32_t *d_nresults,
-                         message_t *d_umsg, float *d_ufreq, int32_t *d_uscore, int32_t *d_ucand, int16_t *d_table, cudaStream_t st, int *launches);
+                         message_t *d_umsg, float *d_ufreq, int32_t *d_uscore, int32_t *d_ucand, int16_t *d_table, cudaStream_t st, int *launches,
+                         bool append = false, int32_t *d_first = nullptr);
+// append (a later pass of multi-pass decoding): keep the slot's records and the log d_umsg/d_ufreq/d_uscore/d_ucand (required) of the
+// earlier passes, de-duplicate against the log and append behind it.  d_first (optional): the slot's record count before this call.
 // ordered-statistics decoding of the entries BP left at stage 1 or 2 (order 0: nothing attempted); with d_work the entries of the
 // find_sync work list, otherwise all n_slots * max_cand.  *d_next: the pull counter, zeroed by the caller.
 cudaError_t launch_osd(int n_slots, int max_cand, int protocol, int order, int max_hard, const float *d_llr, const int *d_ncand, uint8_t *d_ok,
                        uint8_t *d_stage, decode_status_t *d_status, message_t *d_msg, uint8_t *d_plain, uint8_t *d_osd, int32_t *d_osd_hard,
                        uint8_t *d_osd_cw, const uint32_t *d_work, const unsigned int *d_work_total, unsigned int *d_next, int sm_count,
                        cudaStream_t st, int *launches);
+// subtract.cu: refinement + subtraction of decoded messages (multi-pass decoding).  Entry j in [lo, hi) of slot s is row
+// (d_row ? d_row[s * list_stride + j] : j) of d_cand / d_cw (cand_stride rows per slot); d_grid (int32 [n_slots][list_stride][2])
+// receives its refined (dt samples, df steps); y = x minus every listed message (y may be x).  zero_idle: a slot with no entry
+// gets y = 0.  d_scratch: subtract_scratch_bytes.
+cudaError_t upload_subtract_tables();
+size_t subtract_scratch_bytes(int n_slots, int sm_count);
+cudaError_t launch_subtract(const float *d_xi, const float *d_xq, float *d_yi, float *d_yq, int n_slots, const candidate_t *d_cand,
+                            const uint8_t *d_cw, int cand_stride, const int32_t *d_row, const int32_t *d_lo, const int32_t *d_hi, int list_stride,
+                            int32_t *d_grid, float2 *d_scratch, bool zero_idle, int sm_count, cudaStream_t st, int *launches);
 cudaError_t launch_unpack77_batch(const uint8_t *d_payloads, int n, char *d_text32, int32_t *d_status, cudaStream_t st, int *launches);
 cudaError_t upload_ldpc_tables();
 void set_decode_variant(int v);  // 0 = node-centred belief propagation (default), 1 = edge-centred

@@ -120,6 +120,9 @@ ft8b200_ctx_t *default_ctx() {
         // deeper decoding for a relinked program without code changes: FT8B200_OSD=<order>, FT8B200_OSD_MAX_HARD=<cap> (INTEGRATION.md)
         const char *osd = getenv("FT8B200_OSD"), *cap = getenv("FT8B200_OSD_MAX_HARD");
         if (osd && ft8b200_set_osd(g_ctx, atoi(osd), cap ? atoi(cap) : -1) != 0) die("FT8B200_OSD (0, 1 or 2)");
+        // multi-pass decoding with signal subtraction: FT8B200_PASSES=<1, 2 or 3>
+        const char *passes = getenv("FT8B200_PASSES");
+        if (passes && ft8b200_set_passes(g_ctx, atoi(passes)) != 0) die("FT8B200_PASSES (1, 2 or 3)");
     }
     return g_ctx;
 }

@@ -458,6 +458,15 @@ int ft8b200_pipe_set_osd(ft8b200_pipe_t *p, int order, int max_hard_errors) {
     return 0;
 }
 
+int ft8b200_pipe_set_passes(ft8b200_pipe_t *p, int passes) {
+    if (!p) return FT8B200_BAD_ARG();
+    if (passes < 1 || passes > 3) return pfail(p, FT8B200_EINVAL, "ft8b200_pipe_set_passes: passes must be 1, 2 or 3");
+    if (p->count) return pfail(p, FT8B200_EBUSY, "ft8b200_pipe_set_passes: batches in flight");
+    for (Lane &l : p->lanes)
+        if (int rc = ft8b200_set_passes(l.ctx, passes)) return rc;
+    return 0;
+}
+
 int ft8b200_pipe_autotune(ft8b200_pipe_t *p, const uint8_t *d_iq, size_t bytes_per_stream, size_t stream_stride_bytes, int n_slots,
                           const int *candidates, int n_candidates, int batches, int *best_back_sms, int *best_comb_front, float *ms_out) {
     if (!p || !d_iq || !candidates || n_candidates < 1 || n_slots < 1) return FT8B200_BAD_ARG();
