@@ -11,6 +11,7 @@ For one daemon slot x (3200 sps complex, 48 000 samples) and a list of decoded m
   index, then the lower df index;
 - subtraction, in list order on the running residual y (from y = x): over the message's span (its 79 symbols within the slot)
   c = y conj(r), a = c smoothed by h[k] = cos^2(pi k / 1026), |k| <= 512, normalised by the taps inside the span, y -= a r.
+Which messages a pass subtracts is step 1 of the multi-pass definition (accept): the ones the spot table accepted as new.
 This module imports ref64 (gfsk_phase and the protocol constants) and nothing of the library or the oracle."""
 import numpy as np
 from scipy.signal import fftconvolve
@@ -92,6 +93,31 @@ def smooth(c):
     num = fftconvolve(c, WINDOW, mode="same")
     den = fftconvolve(np.ones(c.size), WINDOW, mode="same")
     return num / den
+
+
+def message_key(msg):
+    """(hash, text up to its first NUL) of a msg_dtype record: what the spot table tells messages apart by."""
+    return int(msg["hash"]), bytes(msg["text"]).split(b"\0")[0]
+
+
+def accept(rows, log, max_msgs, min_score):
+    """Step 1 of a pass: the rows (cand, ok, msg: one slot's candidates of one pass, cand_dtype / uint8 / msg_dtype) the spot table
+    accepts as new, in candidate order.  A row is live when ok is set and its score is >= min_score; it is accepted when its key is
+    not in log (the keys accepted by earlier passes and earlier rows) and log holds fewer than max_msgs keys.  With linear probing
+    and no deletions that is exactly the table's behaviour, a full table included.  Extends log; returns the accepted row indices."""
+    cand, ok, msg = rows
+    seen = set(log)
+    out = []
+    for k in range(len(cand)):
+        if not ok[k] or int(cand[k]["score"]) < min_score:
+            continue
+        key = message_key(msg[k])
+        if key in seen or len(log) >= max_msgs:
+            continue
+        seen.add(key)
+        log.append(key)
+        out.append(k)
+    return out
 
 
 def subtract(x, msgs, grids=None):
