@@ -277,6 +277,28 @@ int ft8b200_osd(ft8b200_ctx_t *ctx, const float *d_llr, int n_slots, const int *
                 void *stream);
 /* d_osd / d_osd_hard (as above) of the last process_* or decode batch run with OSD on (n_slots x max_candidates); NULL before that */
 int ft8b200_osd_workspace(ft8b200_ctx_t *ctx, uint8_t **d_osd, int32_t **d_osd_hard);
+/* A-priori (AP) decoding (DESIGN.md section 2.4.3) of the candidates BP and OSD leave undecoded (stage 1 or 2) under the hypothesis
+ * "CQ ??? ???": a plain CQ (c28 = 2, r1 = 0) of type i3 = 1 fixes message bits 0-28 and 74-76, the 32 bits every record of the spot
+ * table shares.  Their LLRs are set to +-1.01 max |llr| (FT4: the scrambled values) and belief propagation runs again with the same
+ * iteration limit.  The word is accepted when its syndrome is zero, its CRC holds, it keeps the 32 forced bits, it differs in at most
+ * max_hard_errors of 174 positions from the hard decision of the unforced LLRs, its call_2 is a standard callsign with no R and a
+ * locator or none, and it unpacks.  on: 0 = off (default; nothing launched or allocated), 1 = on; anything else is FT8B200_EINVAL.
+ * max_hard_errors < 0 selects FT8B200_AP_DEFAULT_MAX_HARD: the largest cap at which AP decoded no message at all on 4096 noise-only
+ * daemon slots (K = 120), with OSD off and at order 2 (tools/perf_ap.py; profiles/perf_ap.json).  A false CQ record would be
+ * published with an invented callsign, so the bar is zero.  Measured on a B200, AP decoded nothing there at any cap, so the rule
+ * gives 174, i.e. no cap; the plausibility and forced-bit gates carry the rejection.  The process_* calls and ft8b200_decode
+ * honour it (after OSD). */
+#define FT8B200_AP_DEFAULT_MAX_HARD 174
+int ft8b200_set_ap(ft8b200_ctx_t *ctx, int on, int max_hard_errors);
+/* Stage-wise AP with the context's switch, cap, protocol and ldpc_iterations: upgrades the n_slots x max_candidates outputs of
+ * ft8b200_decode (and ft8b200_osd) in place, d_llr = the normalised LLRs.  An accepted word makes the entry ok = 1, stage = 4,
+ * status.ldpc_errors = 0 with its CRC fields, msg as a BP decode would, d_plain (optional) = the word; a rejected one changes none of
+ * them.  d_ap: 0 = not attempted (stage 3/4, beyond d_ncand, a non-finite LLR or AP off), 1 = attempted and rejected, 2 = decoded by
+ * AP.  d_ap_hard: the hard-decision distance of AP's final word, -1 when not attempted. */
+int ft8b200_ap(ft8b200_ctx_t *ctx, const float *d_llr, int n_slots, const int *d_ncand, uint8_t *d_ok, uint8_t *d_stage, decode_status_t *d_status,
+               message_t *d_msg, uint8_t *d_plain, uint8_t *d_ap, int32_t *d_ap_hard, void *stream);
+/* d_ap / d_ap_hard (as above) of the last process_* or decode batch run with AP on (n_slots x max_candidates); NULL before that */
+int ft8b200_ap_workspace(ft8b200_ctx_t *ctx, uint8_t **d_ap, int32_t **d_ap_hard);
 /* Multi-pass decoding (DESIGN.md section 2.4.2) on the daemon path -- every process_raw*, process_slots / process_conditioned call,
  * and through them the pipe, the cluster, the drop-in ft8_subsystem, the stream and .iq file paths.  passes = 1 (default) decodes
  * a slot once, exactly as without this call.  With 2 or 3, after each pass the messages the spot table accepted as new in that
@@ -451,6 +473,8 @@ int ft8b200_pipe_set_back_chain(ft8b200_pipe_t *p, int on);
 /* ft8b200_set_osd on every lane (a cluster's pipes through ft8b200_cluster_pipe).  FT8B200_EBUSY while batches are in flight;
  * ft8b200_osd_workspace of a lane is not exposed: the pipe returns spot records only. */
 int ft8b200_pipe_set_osd(ft8b200_pipe_t *p, int order, int max_hard_errors);
+/* ft8b200_set_ap on every lane (a cluster's pipes through ft8b200_cluster_pipe).  FT8B200_EBUSY while batches are in flight. */
+int ft8b200_pipe_set_ap(ft8b200_pipe_t *p, int on, int max_hard_errors);
 /* ft8b200_set_passes on every lane (a cluster's pipes through ft8b200_cluster_pipe).  FT8B200_EBUSY while batches are in flight. */
 int ft8b200_pipe_set_passes(ft8b200_pipe_t *p, int passes);
 int ft8b200_pipe_autotune(ft8b200_pipe_t *p, const uint8_t *d_iq, size_t bytes_per_stream, size_t stream_stride_bytes, int n_slots,

@@ -283,6 +283,27 @@ class Context:
                                      _p(cw), _st(stream)))
         return osd, hard, cw
 
+    def set_ap(self, on: int, max_hard_errors: int = -1):
+        """A-priori decoding of "CQ ??? ???" after BP and OSD: 0 (off) or 1; max_hard_errors < 0 = FT8B200_AP_DEFAULT_MAX_HARD."""
+        self._chk(self.L.ft8b200_set_ap(C.c_void_p(self.h), int(on), int(max_hard_errors)))
+
+    def ap(self, llr, ncand, ok, stage, status, msg, plain=None, stream: int | None = None):
+        """Stage-wise AP over ft8b200_decode's (and ft8b200_osd's) outputs, updated in place -> (ap uint8[n, K], ap_hard int32[n, K])."""
+        import torch
+        n = llr.shape[0]
+        dev = llr.device
+        ap = torch.zeros((n, self.K), dtype=torch.uint8, device=dev)
+        hard = torch.zeros((n, self.K), dtype=torch.int32, device=dev)
+        self._chk(self.L.ft8b200_ap(C.c_void_p(self.h), _p(llr), n, _p(ncand), _p(ok), _p(stage), _p(status), _p(msg), _p(plain), _p(ap), _p(hard),
+                                    _st(stream)))
+        return ap, hard
+
+    def ap_workspace_ptrs(self):
+        """Device pointers (ap, ap_hard) of the last batch decoded with AP on (0 before that)."""
+        a, b = C.c_void_p(0), C.c_void_p(0)
+        self._chk(self.L.ft8b200_ap_workspace(C.c_void_p(self.h), C.byref(a), C.byref(b)))
+        return a.value or 0, b.value or 0
+
     def set_passes(self, passes: int):
         """Multi-pass decoding with signal subtraction on the daemon path: 1 (default, one pass), 2 or 3 (ft8b200_set_passes)."""
         self._chk(self.L.ft8b200_set_passes(C.c_void_p(self.h), int(passes)))
@@ -546,6 +567,10 @@ class Pipe:
     def set_osd(self, order: int, max_hard_errors: int = -1):
         """Context.set_osd on every lane; not while batches are in flight."""
         self._chk(self.L.ft8b200_pipe_set_osd(C.c_void_p(self.h), int(order), int(max_hard_errors)))
+
+    def set_ap(self, on: int, max_hard_errors: int = -1):
+        """Context.set_ap on every lane; not while batches are in flight."""
+        self._chk(self.L.ft8b200_pipe_set_ap(C.c_void_p(self.h), int(on), int(max_hard_errors)))
 
     def set_passes(self, passes: int):
         """Context.set_passes on every lane; not while batches are in flight."""

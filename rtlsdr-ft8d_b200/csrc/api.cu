@@ -80,12 +80,16 @@ struct ft8b200_ctx {
     int osd_order = 0;
     int osd_max_hard = FT8B200_OSD_DEFAULT_MAX_HARD;
     DevBuf llr, osd, osd_hard;
+    // a-priori decoding of "CQ ??? ???" after BP and OSD (ft8b200_set_ap): 0 = off; its per-candidate outputs (it reads llr too)
+    int ap_on = 0;
+    int ap_max_hard = FT8B200_AP_DEFAULT_MAX_HARD;
+    DevBuf ap, ap_hard;
     // multi-pass decoding (ft8b200_set_passes): 1 = off.  With passes > 1: the codewords of pass 1 (plain), the slot's log of accepted
     // messages across passes (ulog/ufreq/uscore/ucand, first = record count before the last pass), the refined grid points, the
     // residual slots (ri/rq), and the rows of the later passes (pass 1 keeps the rows above)
     int passes = 1;
     DevBuf plain, ulog, ufreq, uscore, ucand, first, grid, ri, rq, sub_scratch;
-    DevBuf mag2, cand2, ncand2, ok2, stage2, status2, msg2, plain2, llr2, osd2, osd_hard2;
+    DevBuf mag2, cand2, ncand2, ok2, stage2, status2, msg2, plain2, llr2, osd2, osd_hard2, ap2, ap_hard2;
     // optional per-stage timing of the last process_* call (CUDA events on the launching stream)
     bool profiling = false;
     int overlap = 0;                       // number of slot groups ft8b200_process_raw pipelines (0/1 = off)
@@ -130,6 +134,14 @@ int ensure_osd_buffers(ft8b200_ctx_t *ctx, int n_slots) {
     return ctx->osd_hard.ensure(E * sizeof(int32_t));
 }
 
+int ensure_ap_buffers(ft8b200_ctx_t *ctx, int n_slots) {
+    const size_t E = (size_t)n_slots * ctx->cfg.max_candidates;
+    int rc;
+    if ((rc = ctx->llr.ensure(E * kLdpcN * sizeof(float)))) return rc;
+    if ((rc = ctx->ap.ensure(E))) return rc;
+    return ctx->ap_hard.ensure(E * sizeof(int32_t));
+}
+
 int ensure_pass_buffers(ft8b200_ctx_t *ctx, int n_slots) {
     const size_t K = (size_t)ctx->cfg.max_candidates, M = (size_t)ctx->cfg.max_messages, S = (size_t)n_slots;
     int rc;
@@ -148,6 +160,10 @@ int ensure_pass_buffers(ft8b200_ctx_t *ctx, int n_slots) {
         if ((rc = ctx->llr2.ensure(S * K * kLdpcN * sizeof(float))) || (rc = ctx->osd2.ensure(S * K))) return rc;
         if ((rc = ctx->osd_hard2.ensure(S * K * sizeof(int32_t)))) return rc;
     }
+    if (ctx->ap_on) {
+        if ((rc = ctx->llr2.ensure(S * K * kLdpcN * sizeof(float))) || (rc = ctx->ap2.ensure(S * K))) return rc;
+        if ((rc = ctx->ap_hard2.ensure(S * K * sizeof(int32_t)))) return rc;
+    }
     return 0;
 }
 
@@ -165,6 +181,7 @@ int ensure_slot_buffers(ft8b200_ctx_t *ctx, int n_slots) {
     if ((rc = ctx->nresults.ensure(S * sizeof(int32_t)))) return rc;
     if ((rc = ctx->table.ensure(S * M * sizeof(int16_t)))) return rc;
     if (ctx->osd_order && (rc = ensure_osd_buffers(ctx, n_slots))) return rc;
+    if (ctx->ap_on && (rc = ensure_ap_buffers(ctx, n_slots))) return rc;
     if (ctx->passes > 1 && (rc = ensure_pass_buffers(ctx, n_slots))) return rc;
     return 0;
 }
@@ -279,7 +296,8 @@ void ft8b200_destroy(ft8b200_ctx_t *ctx) {
                       &ctx->stage, &ctx->status, &ctx->msg, &ctx->results, &ctx->nresults, &ctx->table, &ctx->lists, &ctx->scores, &ctx->work, &ctx->work_total,
                       &ctx->llr, &ctx->osd, &ctx->osd_hard, &ctx->plain, &ctx->ulog, &ctx->ufreq, &ctx->uscore, &ctx->ucand, &ctx->first,
                       &ctx->grid, &ctx->ri, &ctx->rq, &ctx->sub_scratch, &ctx->mag2, &ctx->cand2, &ctx->ncand2, &ctx->ok2, &ctx->stage2,
-                      &ctx->status2, &ctx->msg2, &ctx->plain2, &ctx->llr2, &ctx->osd2, &ctx->osd_hard2};
+                      &ctx->status2, &ctx->msg2, &ctx->plain2, &ctx->llr2, &ctx->osd2, &ctx->osd_hard2, &ctx->ap, &ctx->ap_hard,
+                      &ctx->ap2, &ctx->ap_hard2};
     for (DevBuf *b : bufs) b->release();
     delete ctx;
 }
@@ -406,6 +424,10 @@ int decode_proto(ft8b200_ctx_t *ctx, int protocol, const uint8_t *d_mag, size_t 
         if ((rc = ensure_osd_buffers(ctx, n_slots))) return rc;
         if (!d_llr) d_llr = ctx->llr.as<float>();
     }
+    if (ctx->ap_on) {
+        if ((rc = ensure_ap_buffers(ctx, n_slots))) return rc;
+        if (!d_llr) d_llr = ctx->llr.as<float>();
+    }
     CU(launch_decode(d_mag, slot_stride_bytes, n_slots, num_blocks, num_bins, time_osr, freq_osr, protocol, ctx->cfg.max_candidates, ctx->cfg.ldpc_iterations,
                      d_cand, d_ncand, d_ok, d_stage, d_status, d_msg, d_plain, d_llr, nullptr, pull, ctx->sm_count, pick(ctx, stream), &ctx->launches));
     if (ctx->osd_order) {
@@ -414,6 +436,13 @@ int decode_proto(ft8b200_ctx_t *ctx, int protocol, const uint8_t *d_mag, size_t 
         CU(launch_osd(n_slots, ctx->cfg.max_candidates, protocol, ctx->osd_order, ctx->osd_max_hard, d_llr, d_ncand, d_ok, d_stage, d_status, d_msg,
                       d_plain, ctx->osd.as<uint8_t>(), ctx->osd_hard.as<int32_t>(), nullptr, nullptr, nullptr, next, ctx->sm_count, pick(ctx, stream),
                       &ctx->launches));
+    }
+    if (ctx->ap_on) {
+        unsigned int *next = ctx->work_total.as<unsigned int>() + 3;
+        CU(cudaMemsetAsync(next, 0, sizeof(unsigned int), pick(ctx, stream)));
+        CU(launch_ap(n_slots, ctx->cfg.max_candidates, protocol, 1, ctx->ap_max_hard, ctx->cfg.ldpc_iterations, d_llr, d_ncand, d_ok, d_stage, d_status,
+                     d_msg, d_plain, ctx->ap.as<uint8_t>(), ctx->ap_hard.as<int32_t>(), nullptr, nullptr, next, ctx->sm_count, pick(ctx, stream),
+                     &ctx->launches));
     }
     tally(ctx);
     return 0;
@@ -456,6 +485,15 @@ int ft8b200_set_osd(ft8b200_ctx_t *ctx, int order, int max_hard_errors) {
     std::lock_guard<std::mutex> lk(ctx->mu);
     ctx->osd_order = order;
     ctx->osd_max_hard = max_hard_errors < 0 ? FT8B200_OSD_DEFAULT_MAX_HARD : max_hard_errors;
+    return 0;
+}
+
+int ft8b200_set_ap(ft8b200_ctx_t *ctx, int on, int max_hard_errors) {
+    if (!ctx) return fail(FT8B200_EINVAL, "null context");
+    if (on != 0 && on != 1) return fail(FT8B200_EINVAL, "ft8b200_set_ap: on must be 0 (off, the default) or 1");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    ctx->ap_on = on;
+    ctx->ap_max_hard = max_hard_errors < 0 ? FT8B200_AP_DEFAULT_MAX_HARD : max_hard_errors;
     return 0;
 }
 
@@ -507,6 +545,30 @@ int ft8b200_osd_workspace(ft8b200_ctx_t *ctx, uint8_t **d_osd, int32_t **d_osd_h
     return 0;
 }
 
+int ft8b200_ap(ft8b200_ctx_t *ctx, const float *d_llr, int n_slots, const int *d_ncand, uint8_t *d_ok, uint8_t *d_stage, decode_status_t *d_status,
+               message_t *d_msg, uint8_t *d_plain, uint8_t *d_ap, int32_t *d_ap_hard, void *stream) {
+    int rc = ctx_enter(ctx);
+    if (rc) return rc;
+    if (!d_llr || !d_ncand || !d_ok || !d_stage || !d_status || !d_msg || !d_ap || !d_ap_hard || n_slots < 1)
+        return fail(FT8B200_EINVAL, "ft8b200_ap: bad argument");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    if ((rc = ctx->work_total.ensure(4 * sizeof(unsigned int)))) return rc;
+    cudaStream_t st = pick(ctx, stream);
+    unsigned int *next = ctx->work_total.as<unsigned int>() + 3;
+    CU(cudaMemsetAsync(next, 0, sizeof(unsigned int), st));
+    CU(launch_ap(n_slots, ctx->cfg.max_candidates, ctx->protocol, ctx->ap_on, ctx->ap_max_hard, ctx->cfg.ldpc_iterations, d_llr, d_ncand, d_ok, d_stage,
+                 d_status, d_msg, d_plain, d_ap, d_ap_hard, nullptr, nullptr, next, ctx->sm_count, st, &ctx->launches));
+    tally(ctx);
+    return 0;
+}
+
+int ft8b200_ap_workspace(ft8b200_ctx_t *ctx, uint8_t **d_ap, int32_t **d_ap_hard) {
+    if (!ctx) return fail(FT8B200_EINVAL, "null context");
+    if (d_ap) *d_ap = ctx->ap.as<uint8_t>();
+    if (d_ap_hard) *d_ap_hard = ctx->ap_hard.as<int32_t>();
+    return 0;
+}
+
 // ---- per-stage timing: one event pair per (stage, group); stage times are summed over the groups -------------
 static void mark(ft8b200_ctx_t *ctx, int stage, int group, bool end, cudaStream_t st) {
     if (!ctx->profiling || group >= kMaxGroups) return;
@@ -540,7 +602,7 @@ static int run_back_end(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, 
                         st, &ctx->launches));
     mark(ctx, 3, group, true, st);
     mark(ctx, 4, group, false, st);
-    float *llr = ctx->osd_order ? ctx->llr.as<float>() + (size_t)s0 * K * kLdpcN : nullptr;
+    float *llr = (ctx->osd_order || ctx->ap_on) ? ctx->llr.as<float>() + (size_t)s0 * K * kLdpcN : nullptr;
     const bool multi = ctx->passes > 1;
     uint8_t *plain = multi ? ctx->plain.as<uint8_t>() + (size_t)s0 * K * kLdpcN : nullptr;   // the codewords subtraction needs
     CU(launch_decode(mag, kWfBytes, n, 92, 256, 2, 2, PROTO_FT8, ctx->cfg.max_candidates, ctx->cfg.ldpc_iterations, cand, ncand, ok, stage,
@@ -551,6 +613,11 @@ static int run_back_end(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, 
                       ctx->status.as<decode_status_t>() + (size_t)s0 * K, ctx->msg.as<message_t>() + (size_t)s0 * K, plain,
                       ctx->osd.as<uint8_t>() + (size_t)s0 * K, ctx->osd_hard.as<int32_t>() + (size_t)s0 * K, nullptr, ctx->work.as<uint32_t>(),
                       ctx->work_total.as<unsigned int>(), ctx->work_total.as<unsigned int>() + 2, sms, st, &ctx->launches));
+    if (ctx->ap_on)  // what BP and OSD left at stage 1 or 2; word [3] of work_total (zeroed by launch_find_sync) is its pull counter
+        CU(launch_ap(n, ctx->cfg.max_candidates, PROTO_FT8, 1, ctx->ap_max_hard, ctx->cfg.ldpc_iterations, llr, ncand, ok, stage,
+                     ctx->status.as<decode_status_t>() + (size_t)s0 * K, ctx->msg.as<message_t>() + (size_t)s0 * K, plain,
+                     ctx->ap.as<uint8_t>() + (size_t)s0 * K, ctx->ap_hard.as<int32_t>() + (size_t)s0 * K, ctx->work.as<uint32_t>(),
+                     ctx->work_total.as<unsigned int>(), ctx->work_total.as<unsigned int>() + 3, sms, st, &ctx->launches));
     mark(ctx, 4, group, true, st);
     mark(ctx, 5, group, false, st);
     if (!multi) {
@@ -575,7 +642,7 @@ static int run_back_end(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, 
 // Pass p >= 2 (DESIGN.md section 2.4.2): the messages pass p - 1 accepted as new (log entries [first, nresults) of each slot) are
 // refined on that pass's input x and subtracted from it into the residual slots (in place from pass 3 on); a slot with none gets a
 // zero residual and so no candidates.  The residual goes through waterfall (with the slot's original peak scale: the quantiser is
-// absolute), sync, decode (+ OSD) into the later-pass rows, and the spot table appends what is new.
+// absolute), sync, decode (+ OSD, + AP) into the later-pass rows, and the spot table appends what is new.
 static int later_passes(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, const float *d_peak, int s0, int n, int sms, cudaStream_t st) {
     const size_t K = (size_t)ctx->cfg.max_candidates, M = (size_t)ctx->cfg.max_messages;
     const float *xi = d_i + (size_t)s0 * kSlot, *xq = d_q + (size_t)s0 * kSlot;
@@ -589,7 +656,7 @@ static int later_passes(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, 
     decode_status_t *status = ctx->status2.as<decode_status_t>() + (size_t)s0 * K;
     message_t *msg = ctx->msg2.as<message_t>() + (size_t)s0 * K;
     uint8_t *plain = ctx->plain2.as<uint8_t>() + (size_t)s0 * K * kLdpcN;
-    float *llr = ctx->osd_order ? ctx->llr2.as<float>() + (size_t)s0 * K * kLdpcN : nullptr;
+    float *llr = (ctx->osd_order || ctx->ap_on) ? ctx->llr2.as<float>() + (size_t)s0 * K * kLdpcN : nullptr;
     int32_t *first = ctx->first.as<int32_t>() + s0, *nres = ctx->nresults.as<int32_t>() + s0, *ucand = ctx->ucand.as<int32_t>() + (size_t)s0 * M;
     for (int p = 2; p <= ctx->passes; ++p) {
         CU(launch_subtract(xi, xq, ri, rq, n, prev_cand, prev_plain, (int)K, ucand, first, nres, (int)M, ctx->grid.as<int32_t>() + (size_t)s0 * M * 2,
@@ -605,6 +672,10 @@ static int later_passes(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, 
             CU(launch_osd(n, ctx->cfg.max_candidates, PROTO_FT8, ctx->osd_order, ctx->osd_max_hard, llr, ncand, ok, stage, status, msg, plain,
                           ctx->osd2.as<uint8_t>() + (size_t)s0 * K, ctx->osd_hard2.as<int32_t>() + (size_t)s0 * K, nullptr, ctx->work.as<uint32_t>(),
                           ctx->work_total.as<unsigned int>(), ctx->work_total.as<unsigned int>() + 2, sms, st, &ctx->launches));
+        if (ctx->ap_on)
+            CU(launch_ap(n, ctx->cfg.max_candidates, PROTO_FT8, 1, ctx->ap_max_hard, ctx->cfg.ldpc_iterations, llr, ncand, ok, stage, status, msg, plain,
+                         ctx->ap2.as<uint8_t>() + (size_t)s0 * K, ctx->ap_hard2.as<int32_t>() + (size_t)s0 * K, ctx->work.as<uint32_t>(),
+                         ctx->work_total.as<unsigned int>(), ctx->work_total.as<unsigned int>() + 3, sms, st, &ctx->launches));
         CU(launch_spots(n, ctx->cfg.max_candidates, ctx->cfg.max_messages, ctx->cfg.min_score, 2, cand, ncand, ok, msg,
                         ctx->results.as<struct decoder_results>() + (size_t)s0 * M, nres, ctx->ulog.as<message_t>() + (size_t)s0 * M,
                         ctx->ufreq.as<float>() + (size_t)s0 * M, ctx->uscore.as<int32_t>() + (size_t)s0 * M, ucand, ctx->table.as<int16_t>() + (size_t)s0 * M,

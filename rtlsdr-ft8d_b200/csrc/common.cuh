@@ -85,6 +85,11 @@ size_t subtract_scratch_bytes(int n_slots, int sm_count);
 cudaError_t launch_subtract(const float *d_xi, const float *d_xq, float *d_yi, float *d_yq, int n_slots, const candidate_t *d_cand,
                             const uint8_t *d_cw, int cand_stride, const int32_t *d_row, const int32_t *d_lo, const int32_t *d_hi, int list_stride,
                             int32_t *d_grid, float2 *d_scratch, bool zero_idle, int sm_count, cudaStream_t st, int *launches);
+// a-priori decoding ("CQ ??? ???") of the entries BP and OSD left at stage 1 or 2 (on = 0: nothing attempted); work list and
+// *d_next as launch_osd
+cudaError_t launch_ap(int n_slots, int max_cand, int protocol, int on, int max_hard, int max_iters, const float *d_llr, const int *d_ncand, uint8_t *d_ok,
+                      uint8_t *d_stage, decode_status_t *d_status, message_t *d_msg, uint8_t *d_plain, uint8_t *d_ap, int32_t *d_ap_hard,
+                      const uint32_t *d_work, const unsigned int *d_work_total, unsigned int *d_next, int sm_count, cudaStream_t st, int *launches);
 cudaError_t launch_unpack77_batch(const uint8_t *d_payloads, int n, char *d_text32, int32_t *d_status, cudaStream_t st, int *launches);
 cudaError_t upload_ldpc_tables();
 void set_decode_variant(int v);  // 0 = node-centred belief propagation (default), 1 = edge-centred

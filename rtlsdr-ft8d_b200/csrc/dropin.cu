@@ -120,6 +120,14 @@ ft8b200_ctx_t *default_ctx() {
         // deeper decoding for a relinked program without code changes: FT8B200_OSD=<order>, FT8B200_OSD_MAX_HARD=<cap> (INTEGRATION.md)
         const char *osd = getenv("FT8B200_OSD"), *cap = getenv("FT8B200_OSD_MAX_HARD");
         if (osd && ft8b200_set_osd(g_ctx, atoi(osd), cap ? atoi(cap) : -1) != 0) die("FT8B200_OSD (0, 1 or 2)");
+        // a-priori decoding of CQ calls: FT8B200_AP=<0 or 1>, FT8B200_AP_MAX_HARD=<cap> (INTEGRATION.md)
+        const char *ap = getenv("FT8B200_AP"), *ap_cap = getenv("FT8B200_AP_MAX_HARD");
+        if (ap) {
+            char *end = nullptr, *cap_end = nullptr;
+            const long on = strtol(ap, &end, 10), c = ap_cap ? strtol(ap_cap, &cap_end, 10) : -1;
+            if (!*ap || *end || (ap_cap && (!*ap_cap || *cap_end)) || on < 0 || on > 1 || c > 174 || ft8b200_set_ap(g_ctx, (int)on, (int)c) != 0)
+                die("FT8B200_AP (0 or 1) / FT8B200_AP_MAX_HARD (an integer up to 174; negative = the default)");
+        }
         // multi-pass decoding with signal subtraction: FT8B200_PASSES=<1, 2 or 3>
         const char *passes = getenv("FT8B200_PASSES");
         if (passes && ft8b200_set_passes(g_ctx, atoi(passes)) != 0) die("FT8B200_PASSES (1, 2 or 3)");
