@@ -299,6 +299,33 @@ int ft8b200_ap(ft8b200_ctx_t *ctx, const float *d_llr, int n_slots, const int *d
                message_t *d_msg, uint8_t *d_plain, uint8_t *d_ap, int32_t *d_ap_hard, void *stream);
 /* d_ap / d_ap_hard (as above) of the last process_* or decode batch run with AP on (n_slots x max_candidates); NULL before that */
 int ft8b200_ap_workspace(ft8b200_ctx_t *ctx, uint8_t **d_ap, int32_t **d_ap_hard);
+/* Fine-sync decoding (DESIGN.md section 2.4.4) on the daemon path -- every process_raw*, process_slots / process_conditioned call, and
+ * through them the pipe, the cluster, the drop-in ft8_subsystem, the stream and .iq file paths; FT8 only.  Every candidate BP, OSD
+ * (when on) and AP (when on) leave at stage 1 or 2 is demodulated again from the slot's 3200 sps samples: its start and tone-0
+ * frequency are refined against the 21 Costas symbols over dt = -256 ... +256 samples (step 16) x df = -8 ... +8 steps of 6.25/32
+ * Hz, then dt +- 8 samples at that df; the 79 x 8 tone powers of a rectangular symbol-synchronous transform at the winner give the
+ * reference's max-log LLRs (dB metric, a10's normalisation), and belief propagation runs on them with the same iteration limit.  The
+ * word is accepted when its syndrome is zero, its CRC holds, it unpacks and it differs in at most max_hard_errors of 174 positions
+ * from the hard decision of those LLRs.  An accepted word is a stage-4 decode written as a BP decode would be (its word into plain,
+ * so multi-pass decoding subtracts it); the candidate record is not changed.  In a later pass it runs on the residual that pass
+ * searched.  on: 0 = off (default; nothing launched or allocated), 1 = on; anything else is FT8B200_EINVAL.  max_hard_errors < 0
+ * selects FT8B200_FINESYNC_DEFAULT_MAX_HARD: the largest cap at which fine sync decoded no message at all on 4096 noise-only daemon
+ * slots (K = 120) (tools/perf_finesync.py; profiles/perf_finesync.json).  Measured on a B200, fine sync decoded nothing there at
+ * any cap, so the rule gives 174, i.e. no cap.  Decode time in ft8b200_stage_times includes it. */
+#define FT8B200_FINESYNC_DEFAULT_MAX_HARD 174
+int ft8b200_set_finesync(ft8b200_ctx_t *ctx, int on, int max_hard_errors);
+/* Stage-wise fine sync with the context's switch, cap and ldpc_iterations on daemon slots d_i / d_q (FT8B200_SLOT_SAMPLES floats per
+ * slot row, dense, 4-byte aligned) and the n_slots x max_candidates outputs of ft8b200_decode (and ft8b200_osd / ft8b200_ap), which
+ * are upgraded in place as above.  d_fs: 0 = not attempted (stage 3/4, beyond d_ncand, no energy in the span, a non-finite LLR or
+ * fine sync off), 1 = attempted and rejected, 2 = decoded by fine sync.  d_fs_hard: the hard-decision distance of the final word, -1
+ * when not attempted.  d_fs_grid (int32 [n_slots][max_candidates][2]): the refined (dt samples, df steps) and d_fs_llr (optional,
+ * float [n_slots][max_candidates][174]): the refined LLRs, both written for the candidates at stage 1 or 2 only.  Any n_slots outside
+ * 1 ... 65535 is FT8B200_EINVAL.  tests/finesync_ref.py is the float64 definition. */
+int ft8b200_finesync(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, int n_slots, const candidate_t *d_cand, const int *d_ncand, uint8_t *d_ok,
+                     uint8_t *d_stage, decode_status_t *d_status, message_t *d_msg, uint8_t *d_plain, uint8_t *d_fs, int32_t *d_fs_hard,
+                     int32_t *d_fs_grid, float *d_fs_llr, void *stream);
+/* d_fs / d_fs_hard (as above) of pass 1 of the last process_* batch run with fine sync on (n_slots x max_candidates); NULL before that */
+int ft8b200_finesync_workspace(ft8b200_ctx_t *ctx, uint8_t **d_fs, int32_t **d_fs_hard);
 /* Multi-pass decoding (DESIGN.md section 2.4.2) on the daemon path -- every process_raw*, process_slots / process_conditioned call,
  * and through them the pipe, the cluster, the drop-in ft8_subsystem, the stream and .iq file paths.  passes = 1 (default) decodes
  * a slot once, exactly as without this call.  With 2 or 3, after each pass the messages the spot table accepted as new in that
@@ -477,6 +504,8 @@ int ft8b200_pipe_set_osd(ft8b200_pipe_t *p, int order, int max_hard_errors);
 int ft8b200_pipe_set_ap(ft8b200_pipe_t *p, int on, int max_hard_errors);
 /* ft8b200_set_passes on every lane (a cluster's pipes through ft8b200_cluster_pipe).  FT8B200_EBUSY while batches are in flight. */
 int ft8b200_pipe_set_passes(ft8b200_pipe_t *p, int passes);
+/* ft8b200_set_finesync on every lane (a cluster's pipes through ft8b200_cluster_pipe).  FT8B200_EBUSY while batches are in flight. */
+int ft8b200_pipe_set_finesync(ft8b200_pipe_t *p, int on, int max_hard_errors);
 int ft8b200_pipe_autotune(ft8b200_pipe_t *p, const uint8_t *d_iq, size_t bytes_per_stream, size_t stream_stride_bytes, int n_slots,
                           const int *candidates, int n_candidates, int batches, int *best_back_sms, int *best_comb_front, float *ms_out);
 void ft8b200_pipe_destroy(ft8b200_pipe_t *p);

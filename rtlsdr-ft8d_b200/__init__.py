@@ -304,6 +304,31 @@ class Context:
         self._chk(self.L.ft8b200_ap_workspace(C.c_void_p(self.h), C.byref(a), C.byref(b)))
         return a.value or 0, b.value or 0
 
+    def set_finesync(self, on: int, max_hard_errors: int = -1):
+        """Fine-sync decoding after BP, OSD and AP: 0 (off) or 1; max_hard_errors < 0 = FT8B200_FINESYNC_DEFAULT_MAX_HARD."""
+        self._chk(self.L.ft8b200_set_finesync(C.c_void_p(self.h), int(on), int(max_hard_errors)))
+
+    def finesync(self, d_i, d_q, cand, ncand, ok, stage, status, msg, plain=None, want_llr=False, stream: int | None = None):
+        """Stage-wise fine sync on slots d_i / d_q float32 [n, 48000] over ft8b200_decode's (and OSD's, AP's) outputs, updated in place
+        -> (fs uint8[n, K], fs_hard int32[n, K], grid int32[n, K, 2] of (dt samples, df steps), llr float32[n, K, 174] or None); grid
+        and llr are written for the candidates at stage 1 or 2 only (zeros elsewhere)."""
+        import torch
+        n = d_i.shape[0]
+        dev = d_i.device
+        fs = torch.zeros((n, self.K), dtype=torch.uint8, device=dev)
+        hard = torch.zeros((n, self.K), dtype=torch.int32, device=dev)
+        grid = torch.zeros((n, self.K, 2), dtype=torch.int32, device=dev)
+        llr = torch.zeros((n, self.K, 174), dtype=torch.float32, device=dev) if want_llr else None
+        self._chk(self.L.ft8b200_finesync(C.c_void_p(self.h), _p(d_i), _p(d_q), n, _p(cand), _p(ncand), _p(ok), _p(stage), _p(status), _p(msg),
+                                          _p(plain), _p(fs), _p(hard), _p(grid), _p(llr), _st(stream)))
+        return fs, hard, grid, llr
+
+    def finesync_workspace_ptrs(self):
+        """Device pointers (fs, fs_hard) of pass 1 of the last batch decoded with fine sync on (0 before that)."""
+        a, b = C.c_void_p(0), C.c_void_p(0)
+        self._chk(self.L.ft8b200_finesync_workspace(C.c_void_p(self.h), C.byref(a), C.byref(b)))
+        return a.value or 0, b.value or 0
+
     def set_passes(self, passes: int):
         """Multi-pass decoding with signal subtraction on the daemon path: 1 (default, one pass), 2 or 3 (ft8b200_set_passes)."""
         self._chk(self.L.ft8b200_set_passes(C.c_void_p(self.h), int(passes)))
@@ -571,6 +596,10 @@ class Pipe:
     def set_ap(self, on: int, max_hard_errors: int = -1):
         """Context.set_ap on every lane; not while batches are in flight."""
         self._chk(self.L.ft8b200_pipe_set_ap(C.c_void_p(self.h), int(on), int(max_hard_errors)))
+
+    def set_finesync(self, on: int, max_hard_errors: int = -1):
+        """Context.set_finesync on every lane; not while batches are in flight."""
+        self._chk(self.L.ft8b200_pipe_set_finesync(C.c_void_p(self.h), int(on), int(max_hard_errors)))
 
     def set_passes(self, passes: int):
         """Context.set_passes on every lane; not while batches are in flight."""

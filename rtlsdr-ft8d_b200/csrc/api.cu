@@ -84,12 +84,16 @@ struct ft8b200_ctx {
     int ap_on = 0;
     int ap_max_hard = FT8B200_AP_DEFAULT_MAX_HARD;
     DevBuf ap, ap_hard;
+    // fine-sync decoding after BP, OSD and AP (ft8b200_set_finesync): 0 = off; its per-candidate outputs, refined LLRs and grid points
+    int fs_on = 0;
+    int fs_max_hard = FT8B200_FINESYNC_DEFAULT_MAX_HARD;
+    DevBuf fs, fs_hard, fs_llr, fs_grid;
     // multi-pass decoding (ft8b200_set_passes): 1 = off.  With passes > 1: the codewords of pass 1 (plain), the slot's log of accepted
     // messages across passes (ulog/ufreq/uscore/ucand, first = record count before the last pass), the refined grid points, the
     // residual slots (ri/rq), and the rows of the later passes (pass 1 keeps the rows above)
     int passes = 1;
     DevBuf plain, ulog, ufreq, uscore, ucand, first, grid, ri, rq, sub_scratch;
-    DevBuf mag2, cand2, ncand2, ok2, stage2, status2, msg2, plain2, llr2, osd2, osd_hard2, ap2, ap_hard2;
+    DevBuf mag2, cand2, ncand2, ok2, stage2, status2, msg2, plain2, llr2, osd2, osd_hard2, ap2, ap_hard2, fs2, fs_hard2;
     // optional per-stage timing of the last process_* call (CUDA events on the launching stream)
     bool profiling = false;
     int overlap = 0;                       // number of slot groups ft8b200_process_raw pipelines (0/1 = off)
@@ -142,6 +146,15 @@ int ensure_ap_buffers(ft8b200_ctx_t *ctx, int n_slots) {
     return ctx->ap_hard.ensure(E * sizeof(int32_t));
 }
 
+// fs_llr / fs_grid are scratch between finesync_kernel and fs_bp_kernel, so the later passes reuse them
+int ensure_fs_buffers(ft8b200_ctx_t *ctx, int n_slots) {
+    const size_t E = (size_t)n_slots * ctx->cfg.max_candidates;
+    int rc;
+    if ((rc = ctx->fs_llr.ensure(E * kLdpcN * sizeof(float))) || (rc = ctx->fs_grid.ensure(E * 2 * sizeof(int32_t)))) return rc;
+    if ((rc = ctx->fs.ensure(E))) return rc;
+    return ctx->fs_hard.ensure(E * sizeof(int32_t));
+}
+
 int ensure_pass_buffers(ft8b200_ctx_t *ctx, int n_slots) {
     const size_t K = (size_t)ctx->cfg.max_candidates, M = (size_t)ctx->cfg.max_messages, S = (size_t)n_slots;
     int rc;
@@ -164,6 +177,7 @@ int ensure_pass_buffers(ft8b200_ctx_t *ctx, int n_slots) {
         if ((rc = ctx->llr2.ensure(S * K * kLdpcN * sizeof(float))) || (rc = ctx->ap2.ensure(S * K))) return rc;
         if ((rc = ctx->ap_hard2.ensure(S * K * sizeof(int32_t)))) return rc;
     }
+    if (ctx->fs_on && ((rc = ctx->fs2.ensure(S * K)) || (rc = ctx->fs_hard2.ensure(S * K * sizeof(int32_t))))) return rc;
     return 0;
 }
 
@@ -182,6 +196,7 @@ int ensure_slot_buffers(ft8b200_ctx_t *ctx, int n_slots) {
     if ((rc = ctx->table.ensure(S * M * sizeof(int16_t)))) return rc;
     if (ctx->osd_order && (rc = ensure_osd_buffers(ctx, n_slots))) return rc;
     if (ctx->ap_on && (rc = ensure_ap_buffers(ctx, n_slots))) return rc;
+    if (ctx->fs_on && (rc = ensure_fs_buffers(ctx, n_slots))) return rc;
     if (ctx->passes > 1 && (rc = ensure_pass_buffers(ctx, n_slots))) return rc;
     return 0;
 }
@@ -191,7 +206,7 @@ int ensure_scratch(ft8b200_ctx_t *ctx, int npos, int n_slots) {
     if (rc0) return rc0;
     if ((rc0 = ctx->lists.ensure_zeroed(find_sync_list_bytes(n_slots)))) return rc0;   // survivor lists, score kernel -> selection
     if ((rc0 = ctx->work.ensure((size_t)n_slots * ctx->cfg.max_candidates * sizeof(uint32_t)))) return rc0;
-    if ((rc0 = ctx->work_total.ensure(4 * sizeof(unsigned int)))) return rc0;
+    if ((rc0 = ctx->work_total.ensure(5 * sizeof(unsigned int)))) return rc0;
     return 0;
 }
 
@@ -263,6 +278,7 @@ ft8b200_ctx_t *ft8b200_create(const ft8b200_config_t *cfg_in) {
     okc = okc && upload_fir_constants() == cudaSuccess;
     okc = okc && upload_ldpc_tables() == cudaSuccess;
     okc = okc && upload_subtract_tables() == cudaSuccess;
+    okc = okc && upload_finesync_tables() == cudaSuccess;
     {
         std::vector<float> blob(waterfall_blob_floats());
         build_waterfall_tables(win.data(), tw.data(), thr.data(), blob.data());
@@ -297,7 +313,7 @@ void ft8b200_destroy(ft8b200_ctx_t *ctx) {
                       &ctx->llr, &ctx->osd, &ctx->osd_hard, &ctx->plain, &ctx->ulog, &ctx->ufreq, &ctx->uscore, &ctx->ucand, &ctx->first,
                       &ctx->grid, &ctx->ri, &ctx->rq, &ctx->sub_scratch, &ctx->mag2, &ctx->cand2, &ctx->ncand2, &ctx->ok2, &ctx->stage2,
                       &ctx->status2, &ctx->msg2, &ctx->plain2, &ctx->llr2, &ctx->osd2, &ctx->osd_hard2, &ctx->ap, &ctx->ap_hard,
-                      &ctx->ap2, &ctx->ap_hard2};
+                      &ctx->ap2, &ctx->ap_hard2, &ctx->fs, &ctx->fs_hard, &ctx->fs_llr, &ctx->fs_grid, &ctx->fs2, &ctx->fs_hard2};
     for (DevBuf *b : bufs) b->release();
     delete ctx;
 }
@@ -413,7 +429,7 @@ int decode_proto(ft8b200_ctx_t *ctx, int protocol, const uint8_t *d_mag, size_t 
     if (!d_mag || !d_cand || !d_ncand || !d_ok || !d_stage || !d_status || !d_msg || n_slots < 1)
         return fail(FT8B200_EINVAL, "ft8b200_decode: bad argument");
     std::lock_guard<std::mutex> lk(ctx->mu);
-    if ((rc = ctx->work_total.ensure(4 * sizeof(unsigned int)))) return rc;
+    if ((rc = ctx->work_total.ensure(5 * sizeof(unsigned int)))) return rc;
     unsigned int *pull = nullptr;
     if (decode_variant() == 0 && (size_t)n_slots * ctx->cfg.max_candidates > 8u * 4u * (size_t)ctx->sm_count) {
         // more candidates than resident warps: let the warps pull them (counter = word [1], see launch_decode)
@@ -497,6 +513,15 @@ int ft8b200_set_ap(ft8b200_ctx_t *ctx, int on, int max_hard_errors) {
     return 0;
 }
 
+int ft8b200_set_finesync(ft8b200_ctx_t *ctx, int on, int max_hard_errors) {
+    if (!ctx) return fail(FT8B200_EINVAL, "null context");
+    if (on != 0 && on != 1) return fail(FT8B200_EINVAL, "ft8b200_set_finesync: on must be 0 (off, the default) or 1");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    ctx->fs_on = on;
+    ctx->fs_max_hard = max_hard_errors < 0 ? FT8B200_FINESYNC_DEFAULT_MAX_HARD : max_hard_errors;
+    return 0;
+}
+
 int ft8b200_set_passes(ft8b200_ctx_t *ctx, int passes) {
     if (!ctx) return fail(FT8B200_EINVAL, "null context");
     if (passes < 1 || passes > 3) return fail(FT8B200_EINVAL, "ft8b200_set_passes: passes must be 1 (one pass, the default), 2 or 3");
@@ -528,7 +553,7 @@ int ft8b200_osd(ft8b200_ctx_t *ctx, const float *d_llr, int n_slots, const int *
     if (!d_llr || !d_ncand || !d_ok || !d_stage || !d_status || !d_msg || !d_osd || !d_osd_hard || n_slots < 1)
         return fail(FT8B200_EINVAL, "ft8b200_osd: bad argument");
     std::lock_guard<std::mutex> lk(ctx->mu);
-    if ((rc = ctx->work_total.ensure(4 * sizeof(unsigned int)))) return rc;
+    if ((rc = ctx->work_total.ensure(5 * sizeof(unsigned int)))) return rc;
     cudaStream_t st = pick(ctx, stream);
     unsigned int *next = ctx->work_total.as<unsigned int>() + 2;
     CU(cudaMemsetAsync(next, 0, sizeof(unsigned int), st));
@@ -552,7 +577,7 @@ int ft8b200_ap(ft8b200_ctx_t *ctx, const float *d_llr, int n_slots, const int *d
     if (!d_llr || !d_ncand || !d_ok || !d_stage || !d_status || !d_msg || !d_ap || !d_ap_hard || n_slots < 1)
         return fail(FT8B200_EINVAL, "ft8b200_ap: bad argument");
     std::lock_guard<std::mutex> lk(ctx->mu);
-    if ((rc = ctx->work_total.ensure(4 * sizeof(unsigned int)))) return rc;
+    if ((rc = ctx->work_total.ensure(5 * sizeof(unsigned int)))) return rc;
     cudaStream_t st = pick(ctx, stream);
     unsigned int *next = ctx->work_total.as<unsigned int>() + 3;
     CU(cudaMemsetAsync(next, 0, sizeof(unsigned int), st));
@@ -566,6 +591,40 @@ int ft8b200_ap_workspace(ft8b200_ctx_t *ctx, uint8_t **d_ap, int32_t **d_ap_hard
     if (!ctx) return fail(FT8B200_EINVAL, "null context");
     if (d_ap) *d_ap = ctx->ap.as<uint8_t>();
     if (d_ap_hard) *d_ap_hard = ctx->ap_hard.as<int32_t>();
+    return 0;
+}
+
+int ft8b200_finesync(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, int n_slots, const candidate_t *d_cand, const int *d_ncand, uint8_t *d_ok,
+                     uint8_t *d_stage, decode_status_t *d_status, message_t *d_msg, uint8_t *d_plain, uint8_t *d_fs, int32_t *d_fs_hard,
+                     int32_t *d_fs_grid, float *d_fs_llr, void *stream) {
+    int rc = ctx_enter(ctx);
+    if (rc) return rc;
+    if (!d_i || !d_q || !d_cand || !d_ncand || !d_ok || !d_stage || !d_status || !d_msg || !d_fs || !d_fs_hard || !d_fs_grid || n_slots < 1 ||
+        n_slots > FT8B200_MAX_RAW_ROWS)
+        return fail(FT8B200_EINVAL, "ft8b200_finesync: null buffer or n_slots outside 1 ... 65535");
+    if ((((size_t)d_i) | ((size_t)d_q) | ((size_t)d_fs_llr)) & 3) return fail(FT8B200_EINVAL, "ft8b200_finesync: float buffers must be 4-byte aligned");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    if ((rc = ctx->work_total.ensure(5 * sizeof(unsigned int)))) return rc;
+    if (!d_fs_llr) {
+        if ((rc = ctx->fs_llr.ensure((size_t)n_slots * ctx->cfg.max_candidates * kLdpcN * sizeof(float)))) return rc;
+        d_fs_llr = ctx->fs_llr.as<float>();
+    }
+    cudaStream_t st = pick(ctx, stream);
+    unsigned int *next = ctx->work_total.as<unsigned int>() + 4;
+    CU(cudaMemsetAsync(next, 0, sizeof(unsigned int), st));
+    const int K = ctx->cfg.max_candidates;
+    CU(launch_finesync(n_slots, K, ctx->fs_on, d_i, d_q, d_cand, d_ncand, d_stage, d_fs_llr, d_fs_grid, nullptr, nullptr, next, ctx->sm_count, st,
+                       &ctx->launches));
+    CU(launch_fs_bp(n_slots, K, ctx->fs_on, ctx->fs_max_hard, ctx->cfg.ldpc_iterations, d_fs_llr, d_ncand, d_ok, d_stage, d_status, d_msg, d_plain,
+                    d_fs, d_fs_hard, nullptr, nullptr, ctx->sm_count, st, &ctx->launches));
+    tally(ctx);
+    return 0;
+}
+
+int ft8b200_finesync_workspace(ft8b200_ctx_t *ctx, uint8_t **d_fs, int32_t **d_fs_hard) {
+    if (!ctx) return fail(FT8B200_EINVAL, "null context");
+    if (d_fs) *d_fs = ctx->fs.as<uint8_t>();
+    if (d_fs_hard) *d_fs_hard = ctx->fs_hard.as<int32_t>();
     return 0;
 }
 
@@ -618,6 +677,16 @@ static int run_back_end(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, 
                      ctx->status.as<decode_status_t>() + (size_t)s0 * K, ctx->msg.as<message_t>() + (size_t)s0 * K, plain,
                      ctx->ap.as<uint8_t>() + (size_t)s0 * K, ctx->ap_hard.as<int32_t>() + (size_t)s0 * K, ctx->work.as<uint32_t>(),
                      ctx->work_total.as<unsigned int>(), ctx->work_total.as<unsigned int>() + 3, sms, st, &ctx->launches));
+    if (ctx->fs_on) {  // what BP, OSD and AP left at stage 1 or 2, from the slot's samples; word [4] of work_total is finesync_kernel's pull counter
+        float *fs_llr = ctx->fs_llr.as<float>() + (size_t)s0 * K * kLdpcN;
+        CU(launch_finesync(n, ctx->cfg.max_candidates, 1, d_i + (size_t)s0 * kSlot, d_q + (size_t)s0 * kSlot, cand, ncand, stage, fs_llr,
+                           ctx->fs_grid.as<int32_t>() + (size_t)s0 * K * 2, ctx->work.as<uint32_t>(), ctx->work_total.as<unsigned int>(),
+                           ctx->work_total.as<unsigned int>() + 4, sms, st, &ctx->launches));
+        CU(launch_fs_bp(n, ctx->cfg.max_candidates, 1, ctx->fs_max_hard, ctx->cfg.ldpc_iterations, fs_llr, ncand, ok, stage,
+                        ctx->status.as<decode_status_t>() + (size_t)s0 * K, ctx->msg.as<message_t>() + (size_t)s0 * K, plain,
+                        ctx->fs.as<uint8_t>() + (size_t)s0 * K, ctx->fs_hard.as<int32_t>() + (size_t)s0 * K, ctx->work.as<uint32_t>(),
+                        ctx->work_total.as<unsigned int>(), sms, st, &ctx->launches));
+    }
     mark(ctx, 4, group, true, st);
     mark(ctx, 5, group, false, st);
     if (!multi) {
@@ -676,6 +745,15 @@ static int later_passes(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, 
             CU(launch_ap(n, ctx->cfg.max_candidates, PROTO_FT8, 1, ctx->ap_max_hard, ctx->cfg.ldpc_iterations, llr, ncand, ok, stage, status, msg, plain,
                          ctx->ap2.as<uint8_t>() + (size_t)s0 * K, ctx->ap_hard2.as<int32_t>() + (size_t)s0 * K, ctx->work.as<uint32_t>(),
                          ctx->work_total.as<unsigned int>(), ctx->work_total.as<unsigned int>() + 3, sms, st, &ctx->launches));
+        if (ctx->fs_on) {  // on the residual this pass searched
+            float *fs_llr = ctx->fs_llr.as<float>() + (size_t)s0 * K * kLdpcN;
+            CU(launch_finesync(n, ctx->cfg.max_candidates, 1, ri, rq, cand, ncand, stage, fs_llr, ctx->fs_grid.as<int32_t>() + (size_t)s0 * K * 2,
+                               ctx->work.as<uint32_t>(), ctx->work_total.as<unsigned int>(), ctx->work_total.as<unsigned int>() + 4, sms, st,
+                               &ctx->launches));
+            CU(launch_fs_bp(n, ctx->cfg.max_candidates, 1, ctx->fs_max_hard, ctx->cfg.ldpc_iterations, fs_llr, ncand, ok, stage, status, msg, plain,
+                            ctx->fs2.as<uint8_t>() + (size_t)s0 * K, ctx->fs_hard2.as<int32_t>() + (size_t)s0 * K, ctx->work.as<uint32_t>(),
+                            ctx->work_total.as<unsigned int>(), sms, st, &ctx->launches));
+        }
         CU(launch_spots(n, ctx->cfg.max_candidates, ctx->cfg.max_messages, ctx->cfg.min_score, 2, cand, ncand, ok, msg,
                         ctx->results.as<struct decoder_results>() + (size_t)s0 * M, nres, ctx->ulog.as<message_t>() + (size_t)s0 * M,
                         ctx->ufreq.as<float>() + (size_t)s0 * M, ctx->uscore.as<int32_t>() + (size_t)s0 * M, ucand, ctx->table.as<int16_t>() + (size_t)s0 * M,

@@ -128,6 +128,14 @@ ft8b200_ctx_t *default_ctx() {
             if (!*ap || *end || (ap_cap && (!*ap_cap || *cap_end)) || on < 0 || on > 1 || c > 174 || ft8b200_set_ap(g_ctx, (int)on, (int)c) != 0)
                 die("FT8B200_AP (0 or 1) / FT8B200_AP_MAX_HARD (an integer up to 174; negative = the default)");
         }
+        // fine-sync decoding: FT8B200_FINESYNC=<0 or 1>, FT8B200_FINESYNC_MAX_HARD=<cap> (INTEGRATION.md)
+        const char *fs = getenv("FT8B200_FINESYNC"), *fs_cap = getenv("FT8B200_FINESYNC_MAX_HARD");
+        if (fs) {
+            char *end = nullptr, *cap_end = nullptr;
+            const long on = strtol(fs, &end, 10), c = fs_cap ? strtol(fs_cap, &cap_end, 10) : -1;
+            if (!*fs || *end || (fs_cap && (!*fs_cap || *cap_end)) || on < 0 || on > 1 || c > 174 || ft8b200_set_finesync(g_ctx, (int)on, (int)c) != 0)
+                die("FT8B200_FINESYNC (0 or 1) / FT8B200_FINESYNC_MAX_HARD (an integer up to 174; negative = the default)");
+        }
         // multi-pass decoding with signal subtraction: FT8B200_PASSES=<1, 2 or 3>
         const char *passes = getenv("FT8B200_PASSES");
         if (passes && ft8b200_set_passes(g_ctx, atoi(passes)) != 0) die("FT8B200_PASSES (1, 2 or 3)");

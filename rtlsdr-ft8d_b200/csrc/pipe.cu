@@ -466,6 +466,14 @@ int ft8b200_pipe_set_ap(ft8b200_pipe_t *p, int on, int max_hard_errors) {
     return 0;
 }
 
+int ft8b200_pipe_set_finesync(ft8b200_pipe_t *p, int on, int max_hard_errors) {
+    if (!p || (on != 0 && on != 1)) return FT8B200_BAD_ARG();
+    if (p->count) return pfail(p, FT8B200_EBUSY, "ft8b200_pipe_set_finesync: batches in flight");
+    for (Lane &l : p->lanes)
+        if (int rc = ft8b200_set_finesync(l.ctx, on, max_hard_errors)) return rc;
+    return 0;
+}
+
 int ft8b200_pipe_set_passes(ft8b200_pipe_t *p, int passes) {
     if (!p) return FT8B200_BAD_ARG();
     if (passes < 1 || passes > 3) return pfail(p, FT8B200_EINVAL, "ft8b200_pipe_set_passes: passes must be 1, 2 or 3");

@@ -14,6 +14,7 @@
 // fractional cycle goes through sincospif: the synthesiser's 4096-entry cosine table would leave 1.5e-3 of the signal behind.
 #include "common.cuh"
 #include "ft8_tables.h"
+#include "slot_search.cuh"
 
 #include <math.h>
 
@@ -21,13 +22,9 @@ using namespace ft8b200;
 
 namespace {
 
-constexpr int kSym = 512, kNsym = 79, kSpan = kSym * kNsym;   // 40448 samples
-constexpr double kFs = 3200.0, kToneHz = 6.25;
-constexpr int kGrid = 17;                  // points per axis of every search stage
+using namespace ft8b200::slot_search;
+constexpr int kGrid = kDfPoints;           // points per axis of every search stage
 constexpr int kCoarseStep = 16;            // coarse dt step (samples); the coarse dt grid is -128 ... +128
-constexpr double kDfStep = kToneHz / 32.0; // df step (Hz); the df grid is -8 ... +8 steps
-constexpr int kBlk = 8;                    // coarse stage: symbol sums are formed from sub-blocks of 8 samples (see refine_kernel)
-constexpr int kBlocks = kSym / kBlk;       // 64
 constexpr int kHalfWin = 512;              // smoothing window: 1025 taps, h[k] = cos^2(pi k / 1026), |k| <= 512
 constexpr double kWinW = 2.0 * 3.14159265358979323846 / 1026.0;
 constexpr int kChunk = 2048;               // smoothing: outputs per chunk; its halo of 2 x 512 samples is scanned with it
@@ -85,10 +82,6 @@ __device__ __forceinline__ float2 ref_sample(const MsgShared &ms, int m, double 
     return make_float2(env * cs, env * sn);
 }
 
-__device__ __forceinline__ float2 cmul_conj(float2 a, float2 b) {  // a * conj(b)
-    return make_float2(a.x * b.x + a.y * b.y, a.y * b.x - a.x * b.y);
-}
-
 struct MsgList {
     const candidate_t *cand;  // slot s, row r: cand[s * cand_stride + r]
     const uint8_t *cw;        // 174 bytes per row, indexed as cand
@@ -113,17 +106,9 @@ __device__ __forceinline__ bool list_entry(const MsgList &L, int s, int j, candi
     cw = L.cw + o * kLdpcN;
     return true;
 }
-__device__ __forceinline__ int nominal_start(const candidate_t &c) { return kSym * c.time_offset + (kSym / 2) * c.time_sub + kSym / 2; }
-__device__ __forceinline__ double nominal_f0(const candidate_t &c) { return 3.125 * (2 * c.freq_offset + c.freq_sub); }
-
-__device__ __forceinline__ float2 load_x(const float *xi, const float *xq, long long n) {
-    return (n >= 0 && n < kSlot) ? make_float2(xi[n], xq[n]) : make_float2(0.0f, 0.0f);
-}
-
-// Coarse stage: for each symbol the 17 dt candidates are downmixed by r at df = 0 and summed over sub-blocks of 8 samples; the
-// symbol sum at df is then sum_b B_b w_df[b] with w_df[b] = exp(-2 pi i df (8 b + 3.5) / fs).  Against the exact sum this drops
-// each sub-block's own rotation, a factor sinc(pi df 8 / fs) = 1 - 5e-6 at the largest df that is nearly common to all points.
-// The fine stage, at one df, is exact.
+// Coarse stage: for each symbol the 17 dt candidates are downmixed by r at df = 0 and summed over sub-blocks of 8 samples, then
+// rotated to each df (slot_search.cuh).  On a message's own waveform the dropped rotation within a sub-block is a factor
+// sinc(pi df 8 / fs) = 1 - 5e-6 at the largest df that is nearly common to all points.  The fine stage, at one df, is exact.
 __global__ void __launch_bounds__(kRefineThreads) refine_kernel(const float *__restrict__ x_i, const float *__restrict__ x_q, int n_slots, MsgList L,
                                                                 int32_t *__restrict__ grid_out) {
     __shared__ MsgShared ms;
@@ -135,12 +120,7 @@ __global__ void __launch_bounds__(kRefineThreads) refine_kernel(const float *__r
     __shared__ double metric[kGrid * kGrid];
     __shared__ int pick[2];
     const int tid = threadIdx.x;
-    for (int q = tid; q < kGrid * kBlocks; q += blockDim.x) {
-        const int f = q / kBlocks, b = q - f * kBlocks;
-        double sn, cs;
-        sincospi(-2.0 * (f - 8) * kDfStep * (kBlk * b + 0.5 * (kBlk - 1)) / kFs, &sn, &cs);
-        w[q] = make_float2((float)cs, (float)sn);
-    }
+    fill_rotations(w, kBlocks);
     const long long total = (long long)n_slots * L.list_stride;
     for (long long item = blockIdx.x; item < total; item += gridDim.x) {
         const int s = (int)(item % n_slots), j = (int)(item / n_slots);   // entry j of every slot before entry j + 1 of any
@@ -177,13 +157,7 @@ __global__ void __launch_bounds__(kRefineThreads) refine_kernel(const float *__r
                 const int p = tid + u * blockDim.x;
                 if (p >= kGrid * kGrid) break;
                 const int d = p / kGrid, f = p - d * kGrid;
-                float re = 0.0f, im = 0.0f;
-                for (int b = 0; b < kBlocks; ++b) {
-                    const float2 a = bs[d * kBlocks + b], c = w[f * kBlocks + b];
-                    re += a.x * c.x - a.y * c.y;
-                    im += a.x * c.y + a.y * c.x;
-                }
-                acc[u] += (double)re * re + (double)im * im;
+                acc[u] += rotated_power(bs + d * kBlocks, w + f * kBlocks);
             }
             __syncthreads();
         }
@@ -191,9 +165,7 @@ __global__ void __launch_bounds__(kRefineThreads) refine_kernel(const float *__r
             if (tid + u * blockDim.x < kGrid * kGrid) metric[tid + u * blockDim.x] = acc[u];
         __syncthreads();
         if (tid == 0) {
-            int best = 0;
-            for (int p = 1; p < kGrid * kGrid; ++p)
-                if (metric[p] > metric[best]) best = p;   // strict: ties keep the lower dt, then the lower df
+            const int best = pick_max(metric, kGrid * kGrid);
             pick[0] = -128 + kCoarseStep * (best / kGrid);
             pick[1] = best % kGrid - 8;
         }
@@ -228,9 +200,7 @@ __global__ void __launch_bounds__(kRefineThreads) refine_kernel(const float *__r
         if (tid < kGrid) metric[tid] = acc2;
         __syncthreads();
         if (tid == 0) {
-            int best = 0;
-            for (int p = 1; p < kGrid; ++p)
-                if (metric[p] > metric[best]) best = p;
+            const int best = pick_max(metric, kGrid);
             int32_t *g = grid_out + ((size_t)s * L.list_stride + j) * 2;
             g[0] = dt_c + best - 8;
             g[1] = df_i;

@@ -588,7 +588,7 @@ cudaError_t launch_find_sync(const uint8_t *d_mag, size_t slot_stride, int n_slo
     if (g.nfo < 1) {
         // fewer than 8 bins: the reference's `freq_offset + 7 < num_bins` loop (decode.c:189) never runs -> no candidates, no error
         cudaError_t e0 = cudaMemsetAsync(d_ncand, 0, (size_t)n_slots * sizeof(int), st);
-        if (e0 == cudaSuccess && d_work_total) e0 = cudaMemsetAsync(d_work_total, 0, 4 * sizeof(unsigned int), st);
+        if (e0 == cudaSuccess && d_work_total) e0 = cudaMemsetAsync(d_work_total, 0, 5 * sizeof(unsigned int), st);
         return e0;
     }
     if (g.nfo >= 4096 || freq_osr >= 4096 || g.npos >= (1 << 20)) return cudaErrorInvalidValue;
@@ -644,7 +644,8 @@ cudaError_t launch_find_sync(const uint8_t *d_mag, size_t slot_stride, int n_slo
         if ((e = cudaGetLastError()) != cudaSuccess) return e;
     }
     if (d_work_total) {
-        e = cudaMemsetAsync(d_work_total, 0, 4 * sizeof(unsigned int), st);  // [0] items, [1] next item (decode_kernel)
+        // [0] items, [1] next item (decode_kernel), [2] - [4] the pull counters of osd_kernel, ap_kernel and finesync_kernel
+        e = cudaMemsetAsync(d_work_total, 0, 5 * sizeof(unsigned int), st);
         if (e != cudaSuccess) return e;
     }
     // the selection's shared memory: heap + survivors
