@@ -61,6 +61,47 @@ struct DevBuf {
         bytes = 0;
     }
     template <class T> T *as() const { return reinterpret_cast<T *>(p); }
+    template <class T> T *at(size_t n) const { return p ? as<T>() + n : nullptr; }
+};
+
+// The per-candidate rows of one pass over S slots of K candidates: what find_sync and BP write, the codewords multi-pass decoding
+// subtracts (plain), the LLRs OSD and AP read, and the flag and hard-distance pair of each retry decoder (OSD, AP, fine sync).
+// A buffer whose option is off is not allocated.
+struct Rows {
+    DevBuf mag, cand, ncand, ok, stage, status, msg, plain, llr, osd, osd_hard, ap, ap_hard, fs, fs_hard;
+    // the rows of slots s0...: every pointer moved to slot s0, nullptr for a buffer that does not exist or (llr, plain) is not used
+    struct View {
+        uint8_t *mag; candidate_t *cand; int *ncand; uint8_t *ok, *stage; decode_status_t *status; message_t *msg; uint8_t *plain; float *llr;
+        uint8_t *osd; int32_t *osd_hard; uint8_t *ap; int32_t *ap_hard; uint8_t *fs; int32_t *fs_hard;
+    };
+    // the LLRs and the pair of each retry decoder that is on
+    int ensure_retry(size_t S, size_t K, bool osd_on, bool ap_on, bool fs_on) {
+        const size_t E = S * K;
+        int rc;
+        if ((osd_on || ap_on) && (rc = llr.ensure(E * kLdpcN * sizeof(float)))) return rc;
+        if (osd_on && ((rc = osd.ensure(E)) || (rc = osd_hard.ensure(E * sizeof(int32_t))))) return rc;
+        if (ap_on && ((rc = ap.ensure(E)) || (rc = ap_hard.ensure(E * sizeof(int32_t))))) return rc;
+        if (fs_on && ((rc = fs.ensure(E)) || (rc = fs_hard.ensure(E * sizeof(int32_t))))) return rc;
+        return 0;
+    }
+    int ensure(size_t S, size_t K, bool osd_on, bool ap_on, bool fs_on, bool need_plain) {
+        int rc;
+        if ((rc = mag.ensure(S * kWfBytes)) || (rc = cand.ensure(S * K * sizeof(candidate_t))) || (rc = ncand.ensure(S * sizeof(int)))) return rc;
+        if ((rc = ok.ensure(S * K)) || (rc = stage.ensure(S * K)) || (rc = status.ensure(S * K * sizeof(decode_status_t)))) return rc;
+        if ((rc = msg.ensure(S * K * sizeof(message_t)))) return rc;
+        if (need_plain && (rc = plain.ensure(S * K * kLdpcN))) return rc;
+        return ensure_retry(S, K, osd_on, ap_on, fs_on);
+    }
+    void release() {
+        for (DevBuf *b : {&mag, &cand, &ncand, &ok, &stage, &status, &msg, &plain, &llr, &osd, &osd_hard, &ap, &ap_hard, &fs, &fs_hard}) b->release();
+    }
+    View at(int s0, size_t K, bool llr_on, bool plain_on) const {
+        const size_t o = (size_t)s0 * K;
+        return {mag.at<uint8_t>((size_t)s0 * kWfBytes), cand.at<candidate_t>(o), ncand.at<int>(s0), ok.at<uint8_t>(o), stage.at<uint8_t>(o),
+                status.at<decode_status_t>(o), msg.at<message_t>(o), plain_on ? plain.at<uint8_t>(o * kLdpcN) : nullptr,
+                llr_on ? llr.at<float>(o * kLdpcN) : nullptr, osd.at<uint8_t>(o), osd_hard.at<int32_t>(o), ap.at<uint8_t>(o),
+                ap_hard.at<int32_t>(o), fs.at<uint8_t>(o), fs_hard.at<int32_t>(o)};
+    }
 };
 }  // namespace
 
@@ -74,26 +115,25 @@ struct ft8b200_ctx {
     int launches = 0;
     uint64_t launches_total = 0;
     int sm_count = 0;
-    // workspaces (grown on demand)
-    DevBuf raw, sums, si, sq, peak, count, mag, cand, ncand, ok, stage, status, msg, results, nresults, table, lists, scores, work, work_total;
-    // ordered-statistics decoding after BP (ft8b200_set_osd): 0 = off; the LLRs it reads and its per-candidate outputs
+    // workspaces (grown on demand); pass1: the per-candidate rows of the path's first pass, and of the stage-wise retry decoders
+    DevBuf raw, sums, si, sq, peak, count, results, nresults, table, lists, scores, work, work_total;
+    Rows pass1;
+    // the retry decoders after BP, each 0 = off: ordered-statistics decoding (ft8b200_set_osd), a-priori decoding of "CQ ??? ???"
+    // (ft8b200_set_ap) and fine-sync decoding (ft8b200_set_finesync), whose refined LLRs and grid points fs_llr / fs_grid are
+    // scratch between finesync_kernel and the BP after it, shared by all passes
     int osd_order = 0;
     int osd_max_hard = FT8B200_OSD_DEFAULT_MAX_HARD;
-    DevBuf llr, osd, osd_hard;
-    // a-priori decoding of "CQ ??? ???" after BP and OSD (ft8b200_set_ap): 0 = off; its per-candidate outputs (it reads llr too)
     int ap_on = 0;
     int ap_max_hard = FT8B200_AP_DEFAULT_MAX_HARD;
-    DevBuf ap, ap_hard;
-    // fine-sync decoding after BP, OSD and AP (ft8b200_set_finesync): 0 = off; its per-candidate outputs, refined LLRs and grid points
     int fs_on = 0;
     int fs_max_hard = FT8B200_FINESYNC_DEFAULT_MAX_HARD;
-    DevBuf fs, fs_hard, fs_llr, fs_grid;
-    // multi-pass decoding (ft8b200_set_passes): 1 = off.  With passes > 1: the codewords of pass 1 (plain), the slot's log of accepted
-    // messages across passes (ulog/ufreq/uscore/ucand, first = record count before the last pass), the refined grid points, the
-    // residual slots (ri/rq), and the rows of the later passes (pass 1 keeps the rows above)
+    DevBuf fs_llr, fs_grid;
+    // multi-pass decoding (ft8b200_set_passes): 1 = off.  With passes > 1: the slot's log of accepted messages across passes
+    // (ulog/ufreq/uscore/ucand, first = record count before the last pass), the refined grid points, the residual slots (ri/rq), and
+    // the rows of the later passes
     int passes = 1;
-    DevBuf plain, ulog, ufreq, uscore, ucand, first, grid, ri, rq, sub_scratch;
-    DevBuf mag2, cand2, ncand2, ok2, stage2, status2, msg2, plain2, llr2, osd2, osd_hard2, ap2, ap_hard2, fs2, fs_hard2;
+    DevBuf ulog, ufreq, uscore, ucand, first, grid, ri, rq, sub_scratch;
+    Rows later;
     // optional per-stage timing of the last process_* call (CUDA events on the launching stream)
     bool profiling = false;
     int overlap = 0;                       // number of slot groups ft8b200_process_raw pipelines (0/1 = off)
@@ -130,75 +170,22 @@ void tally(ft8b200_ctx_t *ctx) {
     ctx->launches = 0;
 }
 
-int ensure_osd_buffers(ft8b200_ctx_t *ctx, int n_slots) {
-    const size_t E = (size_t)n_slots * ctx->cfg.max_candidates;
-    int rc;
-    if ((rc = ctx->llr.ensure(E * kLdpcN * sizeof(float)))) return rc;
-    if ((rc = ctx->osd.ensure(E))) return rc;
-    return ctx->osd_hard.ensure(E * sizeof(int32_t));
-}
-
-int ensure_ap_buffers(ft8b200_ctx_t *ctx, int n_slots) {
-    const size_t E = (size_t)n_slots * ctx->cfg.max_candidates;
-    int rc;
-    if ((rc = ctx->llr.ensure(E * kLdpcN * sizeof(float)))) return rc;
-    if ((rc = ctx->ap.ensure(E))) return rc;
-    return ctx->ap_hard.ensure(E * sizeof(int32_t));
-}
-
-// fs_llr / fs_grid are scratch between finesync_kernel and fs_bp_kernel, so the later passes reuse them
-int ensure_fs_buffers(ft8b200_ctx_t *ctx, int n_slots) {
-    const size_t E = (size_t)n_slots * ctx->cfg.max_candidates;
-    int rc;
-    if ((rc = ctx->fs_llr.ensure(E * kLdpcN * sizeof(float))) || (rc = ctx->fs_grid.ensure(E * 2 * sizeof(int32_t)))) return rc;
-    if ((rc = ctx->fs.ensure(E))) return rc;
-    return ctx->fs_hard.ensure(E * sizeof(int32_t));
-}
-
-int ensure_pass_buffers(ft8b200_ctx_t *ctx, int n_slots) {
+int ensure_slot_buffers(ft8b200_ctx_t *ctx, int n_slots) {
     const size_t K = (size_t)ctx->cfg.max_candidates, M = (size_t)ctx->cfg.max_messages, S = (size_t)n_slots;
+    const bool multi = ctx->passes > 1;
     int rc;
-    DevBuf *rows[] = {&ctx->ok2, &ctx->stage2};
-    for (DevBuf *b : rows) if ((rc = b->ensure(S * K))) return rc;
-    if ((rc = ctx->plain.ensure(S * K * kLdpcN)) || (rc = ctx->plain2.ensure(S * K * kLdpcN))) return rc;
+    if ((rc = ctx->pass1.ensure(S, K, ctx->osd_order, ctx->ap_on, ctx->fs_on, multi))) return rc;
+    if ((rc = ctx->results.ensure(S * M * sizeof(struct decoder_results)))) return rc;
+    if ((rc = ctx->nresults.ensure(S * sizeof(int32_t)))) return rc;
+    if ((rc = ctx->table.ensure(S * M * sizeof(int16_t)))) return rc;
+    if (ctx->fs_on && ((rc = ctx->fs_llr.ensure(S * K * kLdpcN * sizeof(float))) || (rc = ctx->fs_grid.ensure(S * K * 2 * sizeof(int32_t))))) return rc;
+    if (!multi) return 0;
+    if ((rc = ctx->later.ensure(S, K, ctx->osd_order, ctx->ap_on, ctx->fs_on, true))) return rc;
     if ((rc = ctx->ulog.ensure(S * M * sizeof(message_t))) || (rc = ctx->ufreq.ensure(S * M * sizeof(float)))) return rc;
     if ((rc = ctx->uscore.ensure(S * M * sizeof(int32_t))) || (rc = ctx->ucand.ensure(S * M * sizeof(int32_t)))) return rc;
     if ((rc = ctx->first.ensure(S * sizeof(int32_t))) || (rc = ctx->grid.ensure(S * M * 2 * sizeof(int32_t)))) return rc;
     if ((rc = ctx->ri.ensure(S * kSlot * sizeof(float))) || (rc = ctx->rq.ensure(S * kSlot * sizeof(float)))) return rc;
-    if ((rc = ctx->sub_scratch.ensure(subtract_scratch_bytes(n_slots, ctx->sm_count)))) return rc;
-    if ((rc = ctx->mag2.ensure(S * kWfBytes)) || (rc = ctx->cand2.ensure(S * K * sizeof(candidate_t)))) return rc;
-    if ((rc = ctx->ncand2.ensure(S * sizeof(int))) || (rc = ctx->status2.ensure(S * K * sizeof(decode_status_t)))) return rc;
-    if ((rc = ctx->msg2.ensure(S * K * sizeof(message_t)))) return rc;
-    if (ctx->osd_order) {
-        if ((rc = ctx->llr2.ensure(S * K * kLdpcN * sizeof(float))) || (rc = ctx->osd2.ensure(S * K))) return rc;
-        if ((rc = ctx->osd_hard2.ensure(S * K * sizeof(int32_t)))) return rc;
-    }
-    if (ctx->ap_on) {
-        if ((rc = ctx->llr2.ensure(S * K * kLdpcN * sizeof(float))) || (rc = ctx->ap2.ensure(S * K))) return rc;
-        if ((rc = ctx->ap_hard2.ensure(S * K * sizeof(int32_t)))) return rc;
-    }
-    if (ctx->fs_on && ((rc = ctx->fs2.ensure(S * K)) || (rc = ctx->fs_hard2.ensure(S * K * sizeof(int32_t))))) return rc;
-    return 0;
-}
-
-int ensure_slot_buffers(ft8b200_ctx_t *ctx, int n_slots) {
-    const size_t K = (size_t)ctx->cfg.max_candidates, M = (size_t)ctx->cfg.max_messages, S = (size_t)n_slots;
-    int rc;
-    if ((rc = ctx->mag.ensure(S * kWfBytes))) return rc;
-    if ((rc = ctx->cand.ensure(S * K * sizeof(candidate_t)))) return rc;
-    if ((rc = ctx->ncand.ensure(S * sizeof(int)))) return rc;
-    if ((rc = ctx->ok.ensure(S * K))) return rc;
-    if ((rc = ctx->stage.ensure(S * K))) return rc;
-    if ((rc = ctx->status.ensure(S * K * sizeof(decode_status_t)))) return rc;
-    if ((rc = ctx->msg.ensure(S * K * sizeof(message_t)))) return rc;
-    if ((rc = ctx->results.ensure(S * M * sizeof(struct decoder_results)))) return rc;
-    if ((rc = ctx->nresults.ensure(S * sizeof(int32_t)))) return rc;
-    if ((rc = ctx->table.ensure(S * M * sizeof(int16_t)))) return rc;
-    if (ctx->osd_order && (rc = ensure_osd_buffers(ctx, n_slots))) return rc;
-    if (ctx->ap_on && (rc = ensure_ap_buffers(ctx, n_slots))) return rc;
-    if (ctx->fs_on && (rc = ensure_fs_buffers(ctx, n_slots))) return rc;
-    if (ctx->passes > 1 && (rc = ensure_pass_buffers(ctx, n_slots))) return rc;
-    return 0;
+    return ctx->sub_scratch.ensure(subtract_scratch_bytes(n_slots, ctx->sm_count));
 }
 
 int ensure_scratch(ft8b200_ctx_t *ctx, int npos, int n_slots) {
@@ -207,6 +194,36 @@ int ensure_scratch(ft8b200_ctx_t *ctx, int npos, int n_slots) {
     if ((rc0 = ctx->lists.ensure_zeroed(find_sync_list_bytes(n_slots)))) return rc0;   // survivor lists, score kernel -> selection
     if ((rc0 = ctx->work.ensure((size_t)n_slots * ctx->cfg.max_candidates * sizeof(uint32_t)))) return rc0;
     if ((rc0 = ctx->work_total.ensure(5 * sizeof(unsigned int)))) return rc0;
+    return 0;
+}
+
+// What runs after BP on the rows r of n slots starting at slot s0: OSD, AP and fine sync, each where it is on, each on what the ones
+// before it left at stage 1 or 2.  With the work list (the whole path) they visit its entries and find_sync has zeroed their pull
+// counters, words [2] - [4] of work_total; without it (ft8b200_decode) they visit every entry and the counters they use are zeroed
+// here.  Fine sync demodulates the slot samples xi / xq (kSlot floats per slot); without samples it does not run.
+int launch_retries(ft8b200_ctx_t *ctx, int protocol, const Rows::View &r, int s0, int n, const float *xi, const float *xq, const uint32_t *work,
+                   int sms, cudaStream_t st) {
+    const int K = ctx->cfg.max_candidates, iters = ctx->cfg.ldpc_iterations;
+    unsigned int *counters = ctx->work_total.as<unsigned int>();
+    const unsigned int *total = work ? counters : nullptr;
+    if (ctx->osd_order) {
+        if (!work) CU(cudaMemsetAsync(counters + 2, 0, sizeof(unsigned int), st));
+        CU(launch_osd(n, K, protocol, ctx->osd_order, ctx->osd_max_hard, r.llr, r.ncand, r.ok, r.stage, r.status, r.msg, r.plain, r.osd, r.osd_hard,
+                      nullptr, work, total, counters + 2, sms, st, &ctx->launches));
+    }
+    if (ctx->ap_on) {
+        if (!work) CU(cudaMemsetAsync(counters + 3, 0, sizeof(unsigned int), st));
+        CU(launch_rebp(n, K, protocol, cq_hypothesis(protocol), 1, ctx->ap_max_hard, iters, r.llr, r.ncand, r.ok, r.stage, r.status, r.msg, r.plain,
+                       r.ap, r.ap_hard, work, total, counters + 3, sms, st, &ctx->launches));
+    }
+    if (ctx->fs_on && xi) {  // (finesync_kernel demodulates FT8)
+        float *fs_llr = ctx->fs_llr.as<float>() + (size_t)s0 * K * kLdpcN;
+        if (!work) CU(cudaMemsetAsync(counters + 4, 0, sizeof(unsigned int), st));
+        CU(launch_finesync(n, K, 1, xi, xq, r.cand, r.ncand, r.stage, fs_llr, ctx->fs_grid.as<int32_t>() + (size_t)s0 * K * 2, work, total,
+                           counters + 4, sms, st, &ctx->launches));
+        CU(launch_rebp(n, K, PROTO_FT8, Hypothesis{}, 1, ctx->fs_max_hard, iters, fs_llr, r.ncand, r.ok, r.stage, r.status, r.msg, r.plain, r.fs,
+                       r.fs_hard, work, total, nullptr, sms, st, &ctx->launches));
+    }
     return 0;
 }
 
@@ -308,13 +325,12 @@ void ft8b200_destroy(ft8b200_ctx_t *ctx) {
     for (cudaEvent_t e : ctx->ev_group) if (e) cudaEventDestroy(e);
     cudaFree(ctx->tb.window1024); cudaFree(ctx->tb.twiddle1024); cudaFree(ctx->tb.db_thresholds); cudaFree(ctx->tb.wf_blob);
     cudaFree(ctx->tb.mon_window); cudaFree(ctx->tb.mon_twiddle); cudaFree(ctx->tb.mon_super);
-    DevBuf *bufs[] = {&ctx->raw, &ctx->sums, &ctx->si, &ctx->sq, &ctx->peak, &ctx->count, &ctx->mag, &ctx->cand, &ctx->ncand, &ctx->ok,
-                      &ctx->stage, &ctx->status, &ctx->msg, &ctx->results, &ctx->nresults, &ctx->table, &ctx->lists, &ctx->scores, &ctx->work, &ctx->work_total,
-                      &ctx->llr, &ctx->osd, &ctx->osd_hard, &ctx->plain, &ctx->ulog, &ctx->ufreq, &ctx->uscore, &ctx->ucand, &ctx->first,
-                      &ctx->grid, &ctx->ri, &ctx->rq, &ctx->sub_scratch, &ctx->mag2, &ctx->cand2, &ctx->ncand2, &ctx->ok2, &ctx->stage2,
-                      &ctx->status2, &ctx->msg2, &ctx->plain2, &ctx->llr2, &ctx->osd2, &ctx->osd_hard2, &ctx->ap, &ctx->ap_hard,
-                      &ctx->ap2, &ctx->ap_hard2, &ctx->fs, &ctx->fs_hard, &ctx->fs_llr, &ctx->fs_grid, &ctx->fs2, &ctx->fs_hard2};
+    DevBuf *bufs[] = {&ctx->raw, &ctx->sums, &ctx->si, &ctx->sq, &ctx->peak, &ctx->count, &ctx->results, &ctx->nresults, &ctx->table, &ctx->lists,
+                      &ctx->scores, &ctx->work, &ctx->work_total, &ctx->fs_llr, &ctx->fs_grid, &ctx->ulog, &ctx->ufreq, &ctx->uscore, &ctx->ucand,
+                      &ctx->first, &ctx->grid, &ctx->ri, &ctx->rq, &ctx->sub_scratch};
     for (DevBuf *b : bufs) b->release();
+    ctx->pass1.release();
+    ctx->later.release();
     delete ctx;
 }
 
@@ -430,36 +446,25 @@ int decode_proto(ft8b200_ctx_t *ctx, int protocol, const uint8_t *d_mag, size_t 
         return fail(FT8B200_EINVAL, "ft8b200_decode: bad argument");
     std::lock_guard<std::mutex> lk(ctx->mu);
     if ((rc = ctx->work_total.ensure(5 * sizeof(unsigned int)))) return rc;
+    cudaStream_t st = pick(ctx, stream);
     unsigned int *pull = nullptr;
     if (decode_variant() == 0 && (size_t)n_slots * ctx->cfg.max_candidates > 8u * 4u * (size_t)ctx->sm_count) {
         // more candidates than resident warps: let the warps pull them (counter = word [1], see launch_decode)
         pull = ctx->work_total.as<unsigned int>();
-        CU(cudaMemsetAsync(pull, 0, 4 * sizeof(unsigned int), pick(ctx, stream)));
+        CU(cudaMemsetAsync(pull, 0, 4 * sizeof(unsigned int), st));
     }
-    if (ctx->osd_order) {
-        if ((rc = ensure_osd_buffers(ctx, n_slots))) return rc;
-        if (!d_llr) d_llr = ctx->llr.as<float>();
-    }
-    if (ctx->ap_on) {
-        if ((rc = ensure_ap_buffers(ctx, n_slots))) return rc;
-        if (!d_llr) d_llr = ctx->llr.as<float>();
-    }
+    // OSD's and AP's outputs go to pass 1's rows (ft8b200_osd_workspace, ft8b200_ap_workspace), and so do the LLRs when the caller
+    // passes none; everything else is the caller's
+    if ((rc = ctx->pass1.ensure_retry((size_t)n_slots, (size_t)ctx->cfg.max_candidates, ctx->osd_order, ctx->ap_on, false))) return rc;
+    Rows::View r = ctx->pass1.at(0, ctx->cfg.max_candidates, ctx->osd_order || ctx->ap_on, false);
+    r.cand = const_cast<candidate_t *>(d_cand);  // the retry decoders only read the candidates
+    r.ncand = const_cast<int *>(d_ncand);
+    r.ok = d_ok; r.stage = d_stage; r.status = d_status; r.msg = d_msg; r.plain = d_plain;
+    if (d_llr) r.llr = d_llr;
     CU(launch_decode(d_mag, slot_stride_bytes, n_slots, num_blocks, num_bins, time_osr, freq_osr, protocol, ctx->cfg.max_candidates, ctx->cfg.ldpc_iterations,
-                     d_cand, d_ncand, d_ok, d_stage, d_status, d_msg, d_plain, d_llr, nullptr, pull, ctx->sm_count, pick(ctx, stream), &ctx->launches));
-    if (ctx->osd_order) {
-        unsigned int *next = ctx->work_total.as<unsigned int>() + 2;
-        CU(cudaMemsetAsync(next, 0, sizeof(unsigned int), pick(ctx, stream)));
-        CU(launch_osd(n_slots, ctx->cfg.max_candidates, protocol, ctx->osd_order, ctx->osd_max_hard, d_llr, d_ncand, d_ok, d_stage, d_status, d_msg,
-                      d_plain, ctx->osd.as<uint8_t>(), ctx->osd_hard.as<int32_t>(), nullptr, nullptr, nullptr, next, ctx->sm_count, pick(ctx, stream),
-                      &ctx->launches));
-    }
-    if (ctx->ap_on) {
-        unsigned int *next = ctx->work_total.as<unsigned int>() + 3;
-        CU(cudaMemsetAsync(next, 0, sizeof(unsigned int), pick(ctx, stream)));
-        CU(launch_ap(n_slots, ctx->cfg.max_candidates, protocol, 1, ctx->ap_max_hard, ctx->cfg.ldpc_iterations, d_llr, d_ncand, d_ok, d_stage, d_status,
-                     d_msg, d_plain, ctx->ap.as<uint8_t>(), ctx->ap_hard.as<int32_t>(), nullptr, nullptr, next, ctx->sm_count, pick(ctx, stream),
-                     &ctx->launches));
-    }
+                     d_cand, d_ncand, d_ok, d_stage, d_status, d_msg, d_plain, r.llr, nullptr, pull, ctx->sm_count, st, &ctx->launches));
+    // no slot samples: the stage-wise decode runs OSD and AP; fine sync is its own entry point (ft8b200_finesync)
+    if ((rc = launch_retries(ctx, protocol, r, 0, n_slots, nullptr, nullptr, nullptr, ctx->sm_count, st))) return rc;
     tally(ctx);
     return 0;
 }
@@ -565,8 +570,8 @@ int ft8b200_osd(ft8b200_ctx_t *ctx, const float *d_llr, int n_slots, const int *
 
 int ft8b200_osd_workspace(ft8b200_ctx_t *ctx, uint8_t **d_osd, int32_t **d_osd_hard) {
     if (!ctx) return fail(FT8B200_EINVAL, "null context");
-    if (d_osd) *d_osd = ctx->osd.as<uint8_t>();
-    if (d_osd_hard) *d_osd_hard = ctx->osd_hard.as<int32_t>();
+    if (d_osd) *d_osd = ctx->pass1.osd.as<uint8_t>();
+    if (d_osd_hard) *d_osd_hard = ctx->pass1.osd_hard.as<int32_t>();
     return 0;
 }
 
@@ -581,16 +586,16 @@ int ft8b200_ap(ft8b200_ctx_t *ctx, const float *d_llr, int n_slots, const int *d
     cudaStream_t st = pick(ctx, stream);
     unsigned int *next = ctx->work_total.as<unsigned int>() + 3;
     CU(cudaMemsetAsync(next, 0, sizeof(unsigned int), st));
-    CU(launch_ap(n_slots, ctx->cfg.max_candidates, ctx->protocol, ctx->ap_on, ctx->ap_max_hard, ctx->cfg.ldpc_iterations, d_llr, d_ncand, d_ok, d_stage,
-                 d_status, d_msg, d_plain, d_ap, d_ap_hard, nullptr, nullptr, next, ctx->sm_count, st, &ctx->launches));
+    CU(launch_rebp(n_slots, ctx->cfg.max_candidates, ctx->protocol, cq_hypothesis(ctx->protocol), ctx->ap_on, ctx->ap_max_hard, ctx->cfg.ldpc_iterations,
+                   d_llr, d_ncand, d_ok, d_stage, d_status, d_msg, d_plain, d_ap, d_ap_hard, nullptr, nullptr, next, ctx->sm_count, st, &ctx->launches));
     tally(ctx);
     return 0;
 }
 
 int ft8b200_ap_workspace(ft8b200_ctx_t *ctx, uint8_t **d_ap, int32_t **d_ap_hard) {
     if (!ctx) return fail(FT8B200_EINVAL, "null context");
-    if (d_ap) *d_ap = ctx->ap.as<uint8_t>();
-    if (d_ap_hard) *d_ap_hard = ctx->ap_hard.as<int32_t>();
+    if (d_ap) *d_ap = ctx->pass1.ap.as<uint8_t>();
+    if (d_ap_hard) *d_ap_hard = ctx->pass1.ap_hard.as<int32_t>();
     return 0;
 }
 
@@ -615,16 +620,16 @@ int ft8b200_finesync(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, int
     const int K = ctx->cfg.max_candidates;
     CU(launch_finesync(n_slots, K, ctx->fs_on, d_i, d_q, d_cand, d_ncand, d_stage, d_fs_llr, d_fs_grid, nullptr, nullptr, next, ctx->sm_count, st,
                        &ctx->launches));
-    CU(launch_fs_bp(n_slots, K, ctx->fs_on, ctx->fs_max_hard, ctx->cfg.ldpc_iterations, d_fs_llr, d_ncand, d_ok, d_stage, d_status, d_msg, d_plain,
-                    d_fs, d_fs_hard, nullptr, nullptr, ctx->sm_count, st, &ctx->launches));
+    CU(launch_rebp(n_slots, K, PROTO_FT8, Hypothesis{}, ctx->fs_on, ctx->fs_max_hard, ctx->cfg.ldpc_iterations, d_fs_llr, d_ncand, d_ok, d_stage, d_status,
+                   d_msg, d_plain, d_fs, d_fs_hard, nullptr, nullptr, nullptr, ctx->sm_count, st, &ctx->launches));
     tally(ctx);
     return 0;
 }
 
 int ft8b200_finesync_workspace(ft8b200_ctx_t *ctx, uint8_t **d_fs, int32_t **d_fs_hard) {
     if (!ctx) return fail(FT8B200_EINVAL, "null context");
-    if (d_fs) *d_fs = ctx->fs.as<uint8_t>();
-    if (d_fs_hard) *d_fs_hard = ctx->fs_hard.as<int32_t>();
+    if (d_fs) *d_fs = ctx->pass1.fs.as<uint8_t>();
+    if (d_fs_hard) *d_fs_hard = ctx->pass1.fs_hard.as<int32_t>();
     return 0;
 }
 
@@ -643,58 +648,36 @@ static void clear_marks(ft8b200_ctx_t *ctx) {
 
 // waterfall -> sync -> decode -> spots for slots [s0, s0+n) of the context buffers, all on `st`; with passes > 1 the decoded
 // messages are then subtracted and the residual searched again (later_passes)
-static int later_passes(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, const float *d_peak, int s0, int n, int sms, cudaStream_t st);
+static int later_passes(ft8b200_ctx_t *ctx, const Rows::View &p1, const float *d_i, const float *d_q, const float *d_peak, int s0, int n, int sms,
+                        cudaStream_t st);
 static int run_back_end(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, const float *d_peak, int s0, int n, int group, cudaStream_t st) {
     const size_t K = (size_t)ctx->cfg.max_candidates, M = (size_t)ctx->cfg.max_messages;
-    uint8_t *mag = ctx->mag.as<uint8_t>() + (size_t)s0 * kWfBytes;
-    candidate_t *cand = ctx->cand.as<candidate_t>() + (size_t)s0 * K;
-    int *ncand = ctx->ncand.as<int>() + s0;
-    uint8_t *ok = ctx->ok.as<uint8_t>() + (size_t)s0 * K, *stage = ctx->stage.as<uint8_t>() + (size_t)s0 * K;
+    const bool multi = ctx->passes > 1;
+    const Rows::View r = ctx->pass1.at(s0, K, ctx->osd_order || ctx->ap_on, multi);  // plain: the codewords subtraction needs
+    const float *xi = d_i + (size_t)s0 * kSlot, *xq = d_q + (size_t)s0 * kSlot;
+    uint32_t *work = ctx->work.as<uint32_t>();
+    unsigned int *work_total = ctx->work_total.as<unsigned int>();
     const int sms = (ctx->sm_back > 0 && st == ctx->aux) ? ctx->sm_back : ctx->sm_count;  // persistent grids fit the back-end partition
     mark(ctx, 2, group, false, st);
     // decoder()'s normalisation (when d_peak != NULL) is applied on load inside the waterfall kernel
-    CU(launch_waterfall(ctx->tb, d_i + (size_t)s0 * kSlot, d_q + (size_t)s0 * kSlot, d_peak ? d_peak + s0 : nullptr, n, mag, sms, st, &ctx->launches));
+    CU(launch_waterfall(ctx->tb, xi, xq, d_peak ? d_peak + s0 : nullptr, n, r.mag, sms, st, &ctx->launches));
     mark(ctx, 2, group, true, st);
     mark(ctx, 3, group, false, st);
-    CU(launch_find_sync(mag, kWfBytes, n, 92, 256, 2, 2, PROTO_FT8, ctx->cfg.max_candidates, ctx->cfg.min_score, cand, ncand, ctx->scores.as<int16_t>(),
-                        ctx->lists.as<uint32_t>(), ctx->work.as<uint32_t>(), ctx->work_total.as<unsigned int>(), sms,
-                        st, &ctx->launches));
+    CU(launch_find_sync(r.mag, kWfBytes, n, 92, 256, 2, 2, PROTO_FT8, ctx->cfg.max_candidates, ctx->cfg.min_score, r.cand, r.ncand,
+                        ctx->scores.as<int16_t>(), ctx->lists.as<uint32_t>(), work, work_total, sms, st, &ctx->launches));
     mark(ctx, 3, group, true, st);
     mark(ctx, 4, group, false, st);
-    float *llr = (ctx->osd_order || ctx->ap_on) ? ctx->llr.as<float>() + (size_t)s0 * K * kLdpcN : nullptr;
-    const bool multi = ctx->passes > 1;
-    uint8_t *plain = multi ? ctx->plain.as<uint8_t>() + (size_t)s0 * K * kLdpcN : nullptr;   // the codewords subtraction needs
-    CU(launch_decode(mag, kWfBytes, n, 92, 256, 2, 2, PROTO_FT8, ctx->cfg.max_candidates, ctx->cfg.ldpc_iterations, cand, ncand, ok, stage,
-                     ctx->status.as<decode_status_t>() + (size_t)s0 * K, ctx->msg.as<message_t>() + (size_t)s0 * K, plain, llr,
-                     ctx->work.as<uint32_t>(), ctx->work_total.as<unsigned int>(), sms, st, &ctx->launches));
-    if (ctx->osd_order)  // the work list's entries BP left at stage 1 or 2; word [2] of work_total (zeroed by launch_find_sync) is its pull counter
-        CU(launch_osd(n, ctx->cfg.max_candidates, PROTO_FT8, ctx->osd_order, ctx->osd_max_hard, llr, ncand, ok, stage,
-                      ctx->status.as<decode_status_t>() + (size_t)s0 * K, ctx->msg.as<message_t>() + (size_t)s0 * K, plain,
-                      ctx->osd.as<uint8_t>() + (size_t)s0 * K, ctx->osd_hard.as<int32_t>() + (size_t)s0 * K, nullptr, ctx->work.as<uint32_t>(),
-                      ctx->work_total.as<unsigned int>(), ctx->work_total.as<unsigned int>() + 2, sms, st, &ctx->launches));
-    if (ctx->ap_on)  // what BP and OSD left at stage 1 or 2; word [3] of work_total (zeroed by launch_find_sync) is its pull counter
-        CU(launch_ap(n, ctx->cfg.max_candidates, PROTO_FT8, 1, ctx->ap_max_hard, ctx->cfg.ldpc_iterations, llr, ncand, ok, stage,
-                     ctx->status.as<decode_status_t>() + (size_t)s0 * K, ctx->msg.as<message_t>() + (size_t)s0 * K, plain,
-                     ctx->ap.as<uint8_t>() + (size_t)s0 * K, ctx->ap_hard.as<int32_t>() + (size_t)s0 * K, ctx->work.as<uint32_t>(),
-                     ctx->work_total.as<unsigned int>(), ctx->work_total.as<unsigned int>() + 3, sms, st, &ctx->launches));
-    if (ctx->fs_on) {  // what BP, OSD and AP left at stage 1 or 2, from the slot's samples; word [4] of work_total is finesync_kernel's pull counter
-        float *fs_llr = ctx->fs_llr.as<float>() + (size_t)s0 * K * kLdpcN;
-        CU(launch_finesync(n, ctx->cfg.max_candidates, 1, d_i + (size_t)s0 * kSlot, d_q + (size_t)s0 * kSlot, cand, ncand, stage, fs_llr,
-                           ctx->fs_grid.as<int32_t>() + (size_t)s0 * K * 2, ctx->work.as<uint32_t>(), ctx->work_total.as<unsigned int>(),
-                           ctx->work_total.as<unsigned int>() + 4, sms, st, &ctx->launches));
-        CU(launch_fs_bp(n, ctx->cfg.max_candidates, 1, ctx->fs_max_hard, ctx->cfg.ldpc_iterations, fs_llr, ncand, ok, stage,
-                        ctx->status.as<decode_status_t>() + (size_t)s0 * K, ctx->msg.as<message_t>() + (size_t)s0 * K, plain,
-                        ctx->fs.as<uint8_t>() + (size_t)s0 * K, ctx->fs_hard.as<int32_t>() + (size_t)s0 * K, ctx->work.as<uint32_t>(),
-                        ctx->work_total.as<unsigned int>(), sms, st, &ctx->launches));
-    }
+    CU(launch_decode(r.mag, kWfBytes, n, 92, 256, 2, 2, PROTO_FT8, ctx->cfg.max_candidates, ctx->cfg.ldpc_iterations, r.cand, r.ncand, r.ok, r.stage,
+                     r.status, r.msg, r.plain, r.llr, work, work_total, sms, st, &ctx->launches));
+    if (int rc = launch_retries(ctx, PROTO_FT8, r, s0, n, xi, xq, work, sms, st)) return rc;
     mark(ctx, 4, group, true, st);
     mark(ctx, 5, group, false, st);
     if (!multi) {
-        CU(launch_spots(n, ctx->cfg.max_candidates, ctx->cfg.max_messages, ctx->cfg.min_score, 2, cand, ncand, ok, ctx->msg.as<message_t>() + (size_t)s0 * K,
+        CU(launch_spots(n, ctx->cfg.max_candidates, ctx->cfg.max_messages, ctx->cfg.min_score, 2, r.cand, r.ncand, r.ok, r.msg,
                         ctx->results.as<struct decoder_results>() + (size_t)s0 * M, ctx->nresults.as<int32_t>() + s0, nullptr, nullptr, nullptr, nullptr,
                         ctx->table.as<int16_t>() + (size_t)s0 * M, st, &ctx->launches));
     } else {   // the same table, which also logs what it accepts, in order, for the subtraction and the later passes' de-duplication
-        CU(launch_spots(n, ctx->cfg.max_candidates, ctx->cfg.max_messages, ctx->cfg.min_score, 2, cand, ncand, ok, ctx->msg.as<message_t>() + (size_t)s0 * K,
+        CU(launch_spots(n, ctx->cfg.max_candidates, ctx->cfg.max_messages, ctx->cfg.min_score, 2, r.cand, r.ncand, r.ok, r.msg,
                         ctx->results.as<struct decoder_results>() + (size_t)s0 * M, ctx->nresults.as<int32_t>() + s0, ctx->ulog.as<message_t>() + (size_t)s0 * M,
                         ctx->ufreq.as<float>() + (size_t)s0 * M, ctx->uscore.as<int32_t>() + (size_t)s0 * M, ctx->ucand.as<int32_t>() + (size_t)s0 * M,
                         ctx->table.as<int16_t>() + (size_t)s0 * M, st, &ctx->launches, false, ctx->first.as<int32_t>() + s0));
@@ -702,7 +685,7 @@ static int run_back_end(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, 
     mark(ctx, 5, group, true, st);
     if (multi) {
         mark(ctx, 6, group, false, st);
-        if (int rc = later_passes(ctx, d_i, d_q, d_peak, s0, n, sms, st)) return rc;
+        if (int rc = later_passes(ctx, r, d_i, d_q, d_peak, s0, n, sms, st)) return rc;
         mark(ctx, 6, group, true, st);
     }
     return 0;
@@ -711,55 +694,36 @@ static int run_back_end(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, 
 // Pass p >= 2 (DESIGN.md section 2.4.2): the messages pass p - 1 accepted as new (log entries [first, nresults) of each slot) are
 // refined on that pass's input x and subtracted from it into the residual slots (in place from pass 3 on); a slot with none gets a
 // zero residual and so no candidates.  The residual goes through waterfall (with the slot's original peak scale: the quantiser is
-// absolute), sync, decode (+ OSD, + AP) into the later-pass rows, and the spot table appends what is new.
-static int later_passes(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, const float *d_peak, int s0, int n, int sms, cudaStream_t st) {
+// absolute), sync, decode and the retry decoders (launch_retries: OSD, AP and fine sync on the residual, where on) into the later-pass
+// rows, and the spot table appends what is new.  p1: pass 1's rows of these slots.
+static int later_passes(ft8b200_ctx_t *ctx, const Rows::View &p1, const float *d_i, const float *d_q, const float *d_peak, int s0, int n, int sms,
+                        cudaStream_t st) {
     const size_t K = (size_t)ctx->cfg.max_candidates, M = (size_t)ctx->cfg.max_messages;
     const float *xi = d_i + (size_t)s0 * kSlot, *xq = d_q + (size_t)s0 * kSlot;
     float *ri = ctx->ri.as<float>() + (size_t)s0 * kSlot, *rq = ctx->rq.as<float>() + (size_t)s0 * kSlot;
-    const candidate_t *prev_cand = ctx->cand.as<candidate_t>() + (size_t)s0 * K;
-    const uint8_t *prev_plain = ctx->plain.as<uint8_t>() + (size_t)s0 * K * kLdpcN;
-    uint8_t *mag = ctx->mag2.as<uint8_t>() + (size_t)s0 * kWfBytes;
-    candidate_t *cand = ctx->cand2.as<candidate_t>() + (size_t)s0 * K;
-    int *ncand = ctx->ncand2.as<int>() + s0;
-    uint8_t *ok = ctx->ok2.as<uint8_t>() + (size_t)s0 * K, *stage = ctx->stage2.as<uint8_t>() + (size_t)s0 * K;
-    decode_status_t *status = ctx->status2.as<decode_status_t>() + (size_t)s0 * K;
-    message_t *msg = ctx->msg2.as<message_t>() + (size_t)s0 * K;
-    uint8_t *plain = ctx->plain2.as<uint8_t>() + (size_t)s0 * K * kLdpcN;
-    float *llr = (ctx->osd_order || ctx->ap_on) ? ctx->llr2.as<float>() + (size_t)s0 * K * kLdpcN : nullptr;
+    const Rows::View r = ctx->later.at(s0, K, ctx->osd_order || ctx->ap_on, true);
+    const candidate_t *prev_cand = p1.cand;
+    const uint8_t *prev_plain = p1.plain;
+    uint32_t *work = ctx->work.as<uint32_t>();
+    unsigned int *work_total = ctx->work_total.as<unsigned int>();
     int32_t *first = ctx->first.as<int32_t>() + s0, *nres = ctx->nresults.as<int32_t>() + s0, *ucand = ctx->ucand.as<int32_t>() + (size_t)s0 * M;
     for (int p = 2; p <= ctx->passes; ++p) {
         CU(launch_subtract(xi, xq, ri, rq, n, prev_cand, prev_plain, (int)K, ucand, first, nres, (int)M, ctx->grid.as<int32_t>() + (size_t)s0 * M * 2,
                            ctx->sub_scratch.as<float2>(), true, sms, st, &ctx->launches));
         xi = ri;
         xq = rq;
-        CU(launch_waterfall(ctx->tb, ri, rq, d_peak ? d_peak + s0 : nullptr, n, mag, sms, st, &ctx->launches));
-        CU(launch_find_sync(mag, kWfBytes, n, 92, 256, 2, 2, PROTO_FT8, ctx->cfg.max_candidates, ctx->cfg.min_score, cand, ncand, ctx->scores.as<int16_t>(),
-                            ctx->lists.as<uint32_t>(), ctx->work.as<uint32_t>(), ctx->work_total.as<unsigned int>(), sms, st, &ctx->launches));
-        CU(launch_decode(mag, kWfBytes, n, 92, 256, 2, 2, PROTO_FT8, ctx->cfg.max_candidates, ctx->cfg.ldpc_iterations, cand, ncand, ok, stage, status, msg,
-                         plain, llr, ctx->work.as<uint32_t>(), ctx->work_total.as<unsigned int>(), sms, st, &ctx->launches));
-        if (ctx->osd_order)
-            CU(launch_osd(n, ctx->cfg.max_candidates, PROTO_FT8, ctx->osd_order, ctx->osd_max_hard, llr, ncand, ok, stage, status, msg, plain,
-                          ctx->osd2.as<uint8_t>() + (size_t)s0 * K, ctx->osd_hard2.as<int32_t>() + (size_t)s0 * K, nullptr, ctx->work.as<uint32_t>(),
-                          ctx->work_total.as<unsigned int>(), ctx->work_total.as<unsigned int>() + 2, sms, st, &ctx->launches));
-        if (ctx->ap_on)
-            CU(launch_ap(n, ctx->cfg.max_candidates, PROTO_FT8, 1, ctx->ap_max_hard, ctx->cfg.ldpc_iterations, llr, ncand, ok, stage, status, msg, plain,
-                         ctx->ap2.as<uint8_t>() + (size_t)s0 * K, ctx->ap_hard2.as<int32_t>() + (size_t)s0 * K, ctx->work.as<uint32_t>(),
-                         ctx->work_total.as<unsigned int>(), ctx->work_total.as<unsigned int>() + 3, sms, st, &ctx->launches));
-        if (ctx->fs_on) {  // on the residual this pass searched
-            float *fs_llr = ctx->fs_llr.as<float>() + (size_t)s0 * K * kLdpcN;
-            CU(launch_finesync(n, ctx->cfg.max_candidates, 1, ri, rq, cand, ncand, stage, fs_llr, ctx->fs_grid.as<int32_t>() + (size_t)s0 * K * 2,
-                               ctx->work.as<uint32_t>(), ctx->work_total.as<unsigned int>(), ctx->work_total.as<unsigned int>() + 4, sms, st,
-                               &ctx->launches));
-            CU(launch_fs_bp(n, ctx->cfg.max_candidates, 1, ctx->fs_max_hard, ctx->cfg.ldpc_iterations, fs_llr, ncand, ok, stage, status, msg, plain,
-                            ctx->fs2.as<uint8_t>() + (size_t)s0 * K, ctx->fs_hard2.as<int32_t>() + (size_t)s0 * K, ctx->work.as<uint32_t>(),
-                            ctx->work_total.as<unsigned int>(), sms, st, &ctx->launches));
-        }
-        CU(launch_spots(n, ctx->cfg.max_candidates, ctx->cfg.max_messages, ctx->cfg.min_score, 2, cand, ncand, ok, msg,
+        CU(launch_waterfall(ctx->tb, ri, rq, d_peak ? d_peak + s0 : nullptr, n, r.mag, sms, st, &ctx->launches));
+        CU(launch_find_sync(r.mag, kWfBytes, n, 92, 256, 2, 2, PROTO_FT8, ctx->cfg.max_candidates, ctx->cfg.min_score, r.cand, r.ncand,
+                            ctx->scores.as<int16_t>(), ctx->lists.as<uint32_t>(), work, work_total, sms, st, &ctx->launches));
+        CU(launch_decode(r.mag, kWfBytes, n, 92, 256, 2, 2, PROTO_FT8, ctx->cfg.max_candidates, ctx->cfg.ldpc_iterations, r.cand, r.ncand, r.ok, r.stage,
+                         r.status, r.msg, r.plain, r.llr, work, work_total, sms, st, &ctx->launches));
+        if (int rc = launch_retries(ctx, PROTO_FT8, r, s0, n, ri, rq, work, sms, st)) return rc;
+        CU(launch_spots(n, ctx->cfg.max_candidates, ctx->cfg.max_messages, ctx->cfg.min_score, 2, r.cand, r.ncand, r.ok, r.msg,
                         ctx->results.as<struct decoder_results>() + (size_t)s0 * M, nres, ctx->ulog.as<message_t>() + (size_t)s0 * M,
                         ctx->ufreq.as<float>() + (size_t)s0 * M, ctx->uscore.as<int32_t>() + (size_t)s0 * M, ucand, ctx->table.as<int16_t>() + (size_t)s0 * M,
                         st, &ctx->launches, true, first));
-        prev_cand = cand;
-        prev_plain = plain;
+        prev_cand = r.cand;
+        prev_plain = r.plain;
     }
     return 0;
 }
@@ -1104,12 +1068,12 @@ int ft8b200_workspace(ft8b200_ctx_t *ctx, float **d_i, float **d_q, float **d_pe
     if (d_i) *d_i = ctx->si.as<float>();
     if (d_q) *d_q = ctx->sq.as<float>();
     if (d_peak) *d_peak = ctx->peak.as<float>();
-    if (d_mag) *d_mag = ctx->mag.as<uint8_t>();
-    if (d_cand) *d_cand = ctx->cand.as<candidate_t>();
-    if (d_ncand) *d_ncand = ctx->ncand.as<int>();
-    if (d_ok) *d_ok = ctx->ok.as<uint8_t>();
-    if (d_status) *d_status = ctx->status.as<decode_status_t>();
-    if (d_msg) *d_msg = ctx->msg.as<message_t>();
+    if (d_mag) *d_mag = ctx->pass1.mag.as<uint8_t>();
+    if (d_cand) *d_cand = ctx->pass1.cand.as<candidate_t>();
+    if (d_ncand) *d_ncand = ctx->pass1.ncand.as<int>();
+    if (d_ok) *d_ok = ctx->pass1.ok.as<uint8_t>();
+    if (d_status) *d_status = ctx->pass1.status.as<decode_status_t>();
+    if (d_msg) *d_msg = ctx->pass1.msg.as<message_t>();
     return 0;
 }
 

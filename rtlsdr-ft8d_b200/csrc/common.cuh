@@ -85,22 +85,28 @@ size_t subtract_scratch_bytes(int n_slots, int sm_count);
 cudaError_t launch_subtract(const float *d_xi, const float *d_xq, float *d_yi, float *d_yq, int n_slots, const candidate_t *d_cand,
                             const uint8_t *d_cw, int cand_stride, const int32_t *d_row, const int32_t *d_lo, const int32_t *d_hi, int list_stride,
                             int32_t *d_grid, float2 *d_scratch, bool zero_idle, int sm_count, cudaStream_t st, int *launches);
-// a-priori decoding ("CQ ??? ???") of the entries BP and OSD left at stage 1 or 2 (on = 0: nothing attempted); work list and
-// *d_next as launch_osd
-cudaError_t launch_ap(int n_slots, int max_cand, int protocol, int on, int max_hard, int max_iters, const float *d_llr, const int *d_ncand, uint8_t *d_ok,
-                      uint8_t *d_stage, decode_status_t *d_status, message_t *d_msg, uint8_t *d_plain, uint8_t *d_ap, int32_t *d_ap_hard,
-                      const uint32_t *d_work, const unsigned int *d_work_total, unsigned int *d_next, int sm_count, cudaStream_t st, int *launches);
-// fine-sync decoding of the entries BP, OSD and AP left at stage 1 or 2 (on = 0: nothing attempted); work list as launch_osd.
-// launch_finesync (finesync.cu): the Costas search on the slots d_xi / d_xq (kSlot floats per slot) and the refined LLRs into d_llr
-// ([n_slots][max_cand][174]) and d_grid ([n_slots][max_cand][2]), for the entries it attempts only; *d_next: its pull counter,
-// zeroed by the caller.  launch_fs_bp (decode.cu): BP on d_llr and the gates, d_fs / d_fs_hard for every entry.
+// BP again on d_llr, with the hypothesis' codeword positions forced, for the entries the decoders before left at stage 1 or 2
+// (on = 0: nothing attempted): a-priori decoding with cq_hypothesis(), fine-sync decoding with nothing forced (Hypothesis{}).
+// d_flag / d_hard get every entry's outcome.  Work list as launch_osd; with d_next the warps pull entries from that counter (zeroed by
+// the caller), without it they take a fixed stride.
+struct Hypothesis {
+    uint32_t mask[3], val[3];  // the forced codeword positions (bits 0-95) and their values
+    uint32_t scr[3];           // the FT4 scramble of message bits 0-76, which the CQ gate undoes
+    int cq_gate;               // accept only a plausible CQ: standard call_2, no R, a locator or none
+};
+Hypothesis cq_hypothesis(int protocol);  // "CQ ??? ???"
+cudaError_t launch_rebp(int n_slots, int max_cand, int protocol, const Hypothesis &hyp, int on, int max_hard, int max_iters, const float *d_llr,
+                        const int *d_ncand, uint8_t *d_ok, uint8_t *d_stage, decode_status_t *d_status, message_t *d_msg, uint8_t *d_plain,
+                        uint8_t *d_flag, int32_t *d_hard, const uint32_t *d_work, const unsigned int *d_work_total, unsigned int *d_next,
+                        int sm_count, cudaStream_t st, int *launches);
+// fine-sync decoding, front half (finesync.cu): for the entries BP, OSD and AP left at stage 1 or 2 (on = 0: nothing attempted), the
+// Costas search on the slots d_xi / d_xq (kSlot floats per slot) and the refined LLRs into d_llr ([n_slots][max_cand][174]) and d_grid
+// ([n_slots][max_cand][2]), for the entries it attempts only; work list as launch_osd, *d_next: its pull counter, zeroed by the
+// caller.  launch_rebp on d_llr is the back half.
 cudaError_t upload_finesync_tables();
 cudaError_t launch_finesync(int n_slots, int max_cand, int on, const float *d_xi, const float *d_xq, const candidate_t *d_cand, const int *d_ncand,
                             const uint8_t *d_stage, float *d_llr, int32_t *d_grid, const uint32_t *d_work, const unsigned int *d_work_total,
                             unsigned int *d_next, int sm_count, cudaStream_t st, int *launches);
-cudaError_t launch_fs_bp(int n_slots, int max_cand, int on, int max_hard, int max_iters, const float *d_llr, const int *d_ncand, uint8_t *d_ok,
-                         uint8_t *d_stage, decode_status_t *d_status, message_t *d_msg, uint8_t *d_plain, uint8_t *d_fs, int32_t *d_fs_hard,
-                         const uint32_t *d_work, const unsigned int *d_work_total, int sm_count, cudaStream_t st, int *launches);
 cudaError_t launch_unpack77_batch(const uint8_t *d_payloads, int n, char *d_text32, int32_t *d_status, cudaStream_t st, int *launches);
 cudaError_t upload_ldpc_tables();
 void set_decode_variant(int v);  // 0 = node-centred belief propagation (default), 1 = edge-centred

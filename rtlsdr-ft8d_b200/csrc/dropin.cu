@@ -12,6 +12,7 @@
 #include <string.h>
 
 #include <mutex>
+#include <string>
 #include <vector>
 
 using namespace ft8b200;
@@ -105,6 +106,18 @@ void die(const char *where) {
     fprintf(stderr, "libft8b200: %s failed: %s\n", where, ft8b200_last_error());
     abort();
 }
+
+// <name>=<0 or 1> and <name>_MAX_HARD=<cap> switch a decoder and cap its hard distance; anything but an integer, a switch other
+// than 0 or 1, or a cap above 174 stops the program
+void set_from_env(ft8b200_ctx_t *ctx, const char *name, int (*set)(ft8b200_ctx_t *, int, int)) {
+    const std::string cap_name = std::string(name) + "_MAX_HARD";
+    const char *v = getenv(name), *cap = getenv(cap_name.c_str());
+    if (!v) return;
+    char *end = nullptr, *cap_end = nullptr;
+    const long on = strtol(v, &end, 10), c = cap ? strtol(cap, &cap_end, 10) : -1;
+    if (!*v || *end || (cap && (!*cap || *cap_end)) || on < 0 || on > 1 || c > 174 || set(ctx, (int)on, (int)c) != 0)
+        die((std::string(name) + " (0 or 1) / " + cap_name + " (an integer up to 174; negative = the default)").c_str());
+}
 }  // namespace
 
 namespace ft8b200 {
@@ -120,22 +133,9 @@ ft8b200_ctx_t *default_ctx() {
         // deeper decoding for a relinked program without code changes: FT8B200_OSD=<order>, FT8B200_OSD_MAX_HARD=<cap> (INTEGRATION.md)
         const char *osd = getenv("FT8B200_OSD"), *cap = getenv("FT8B200_OSD_MAX_HARD");
         if (osd && ft8b200_set_osd(g_ctx, atoi(osd), cap ? atoi(cap) : -1) != 0) die("FT8B200_OSD (0, 1 or 2)");
-        // a-priori decoding of CQ calls: FT8B200_AP=<0 or 1>, FT8B200_AP_MAX_HARD=<cap> (INTEGRATION.md)
-        const char *ap = getenv("FT8B200_AP"), *ap_cap = getenv("FT8B200_AP_MAX_HARD");
-        if (ap) {
-            char *end = nullptr, *cap_end = nullptr;
-            const long on = strtol(ap, &end, 10), c = ap_cap ? strtol(ap_cap, &cap_end, 10) : -1;
-            if (!*ap || *end || (ap_cap && (!*ap_cap || *cap_end)) || on < 0 || on > 1 || c > 174 || ft8b200_set_ap(g_ctx, (int)on, (int)c) != 0)
-                die("FT8B200_AP (0 or 1) / FT8B200_AP_MAX_HARD (an integer up to 174; negative = the default)");
-        }
-        // fine-sync decoding: FT8B200_FINESYNC=<0 or 1>, FT8B200_FINESYNC_MAX_HARD=<cap> (INTEGRATION.md)
-        const char *fs = getenv("FT8B200_FINESYNC"), *fs_cap = getenv("FT8B200_FINESYNC_MAX_HARD");
-        if (fs) {
-            char *end = nullptr, *cap_end = nullptr;
-            const long on = strtol(fs, &end, 10), c = fs_cap ? strtol(fs_cap, &cap_end, 10) : -1;
-            if (!*fs || *end || (fs_cap && (!*fs_cap || *cap_end)) || on < 0 || on > 1 || c > 174 || ft8b200_set_finesync(g_ctx, (int)on, (int)c) != 0)
-                die("FT8B200_FINESYNC (0 or 1) / FT8B200_FINESYNC_MAX_HARD (an integer up to 174; negative = the default)");
-        }
+        // a-priori decoding of CQ calls and fine-sync decoding (INTEGRATION.md)
+        set_from_env(g_ctx, "FT8B200_AP", ft8b200_set_ap);
+        set_from_env(g_ctx, "FT8B200_FINESYNC", ft8b200_set_finesync);
         // multi-pass decoding with signal subtraction: FT8B200_PASSES=<1, 2 or 3>
         const char *passes = getenv("FT8B200_PASSES");
         if (passes && ft8b200_set_passes(g_ctx, atoi(passes)) != 0) die("FT8B200_PASSES (1, 2 or 3)");

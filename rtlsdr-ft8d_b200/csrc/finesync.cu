@@ -1,7 +1,7 @@
 // finesync.cu -- the front half of fine-sync decoding (DESIGN.md section 2.4.4, ft8b200_set_finesync, ft8b200_finesync): for every
 // candidate that BP, OSD and AP left at stage 1 or 2, a (dt, df) search against the Costas arrays on the slot's 3200 sps samples and
 // the symbol-synchronous spectra at the winner, turned into the reference's LLRs.  The back half (belief propagation and the gates)
-// is fs_bp_kernel in decode.cu.  tests/finesync_ref.py is the float64 definition this kernel is held to.
+// is rebp_kernel in decode.cu with nothing forced.  tests/finesync_ref.py is the float64 definition this kernel is held to.
 //
 // For a candidate with nominal start s0 and tone-0 frequency f0 (slot_search.cuh):
 //   S(s, f) = sum over the 21 Costas symbols k of |sum_{m < 512} x[s + 512 k + m] exp(-2 pi i (f + 6.25 costas[k]) m / 3200)|^2

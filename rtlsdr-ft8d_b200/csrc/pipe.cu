@@ -127,6 +127,16 @@ int pfail(ft8b200_pipe_t *p, int code, const std::string &msg) {
     p->err = msg;
     return code;
 }
+
+// a decoder setting for every lane's context; refused while batches are in flight.  `func`: the setter's name, for the message
+template <class Set>
+int set_lanes(ft8b200_pipe_t *p, const char *func, Set set) {
+    if (p->count) return pfail(p, FT8B200_EBUSY, std::string(func) + ": batches in flight");
+    for (Lane &l : p->lanes)
+        if (int rc = set(l.ctx)) return rc;
+    return 0;
+}
+
 #define PCU(call)                                                                                   \
     do {                                                                                            \
         cudaError_t e__ = (call);                                                                   \
@@ -452,35 +462,23 @@ int ft8b200_pipe_set_back_chain(ft8b200_pipe_t *p, int on) {
 
 int ft8b200_pipe_set_osd(ft8b200_pipe_t *p, int order, int max_hard_errors) {
     if (!p || order < 0 || order > 2) return FT8B200_BAD_ARG();
-    if (p->count) return pfail(p, FT8B200_EBUSY, "ft8b200_pipe_set_osd: batches in flight");
-    for (Lane &l : p->lanes)
-        if (int rc = ft8b200_set_osd(l.ctx, order, max_hard_errors)) return rc;
-    return 0;
+    return set_lanes(p, __func__, [&](ft8b200_ctx_t *c) { return ft8b200_set_osd(c, order, max_hard_errors); });
 }
 
 int ft8b200_pipe_set_ap(ft8b200_pipe_t *p, int on, int max_hard_errors) {
     if (!p || (on != 0 && on != 1)) return FT8B200_BAD_ARG();
-    if (p->count) return pfail(p, FT8B200_EBUSY, "ft8b200_pipe_set_ap: batches in flight");
-    for (Lane &l : p->lanes)
-        if (int rc = ft8b200_set_ap(l.ctx, on, max_hard_errors)) return rc;
-    return 0;
+    return set_lanes(p, __func__, [&](ft8b200_ctx_t *c) { return ft8b200_set_ap(c, on, max_hard_errors); });
 }
 
 int ft8b200_pipe_set_finesync(ft8b200_pipe_t *p, int on, int max_hard_errors) {
     if (!p || (on != 0 && on != 1)) return FT8B200_BAD_ARG();
-    if (p->count) return pfail(p, FT8B200_EBUSY, "ft8b200_pipe_set_finesync: batches in flight");
-    for (Lane &l : p->lanes)
-        if (int rc = ft8b200_set_finesync(l.ctx, on, max_hard_errors)) return rc;
-    return 0;
+    return set_lanes(p, __func__, [&](ft8b200_ctx_t *c) { return ft8b200_set_finesync(c, on, max_hard_errors); });
 }
 
 int ft8b200_pipe_set_passes(ft8b200_pipe_t *p, int passes) {
     if (!p) return FT8B200_BAD_ARG();
     if (passes < 1 || passes > 3) return pfail(p, FT8B200_EINVAL, "ft8b200_pipe_set_passes: passes must be 1, 2 or 3");
-    if (p->count) return pfail(p, FT8B200_EBUSY, "ft8b200_pipe_set_passes: batches in flight");
-    for (Lane &l : p->lanes)
-        if (int rc = ft8b200_set_passes(l.ctx, passes)) return rc;
-    return 0;
+    return set_lanes(p, __func__, [&](ft8b200_ctx_t *c) { return ft8b200_set_passes(c, passes); });
 }
 
 int ft8b200_pipe_autotune(ft8b200_pipe_t *p, const uint8_t *d_iq, size_t bytes_per_stream, size_t stream_stride_bytes, int n_slots,

@@ -644,7 +644,7 @@ cudaError_t launch_find_sync(const uint8_t *d_mag, size_t slot_stride, int n_slo
         if ((e = cudaGetLastError()) != cudaSuccess) return e;
     }
     if (d_work_total) {
-        // [0] items, [1] next item (decode_kernel), [2] - [4] the pull counters of osd_kernel, ap_kernel and finesync_kernel
+        // [0] items, [1] next item (decode_kernel), [2] - [4] the pull counters of OSD, AP (osd_kernel, rebp_kernel) and finesync_kernel
         e = cudaMemsetAsync(d_work_total, 0, 5 * sizeof(unsigned int), st);
         if (e != cudaSuccess) return e;
     }

@@ -175,7 +175,7 @@ def test_front_half_matches_the_definition(pkg, hand_slots, default_cap):
 
 
 def expected_back_half(oracle, llr, cap):
-    """-> (fs, hard, codeword or None) of fs_bp_kernel for one candidate at stage 1 or 2 with these LLRs."""
+    """-> (fs, hard, codeword or None) of rebp_kernel (fine sync: nothing forced) for one candidate at stage 1 or 2 with these LLRs."""
     if not np.all(np.isfinite(llr)):
         return 0, -1, None
     plain, err = oracle.bp_decode(llr, 20)
