@@ -326,6 +326,33 @@ int ft8b200_finesync(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, int
                      int32_t *d_fs_grid, float *d_fs_llr, void *stream);
 /* d_fs / d_fs_hard (as above) of pass 1 of the last process_* batch run with fine sync on (n_slots x max_candidates); NULL before that */
 int ft8b200_finesync_workspace(ft8b200_ctx_t *ctx, uint8_t **d_fs, int32_t **d_fs_hard);
+/* Deep fine sync (DESIGN.md section 2.4.6): with fine sync on, decode every candidate from three refined LLR sets instead of one, and
+ * with every retry decoder that is on.  Set a is fine sync's dB set; sets b and c are WSJT-X's nsym = 2 and 3 coherent metrics: the
+ * symbols of each half are grouped in pairs (nsym = 2: 14 and a single) or triples (nsym = 3: 9 and a pair), and a bit's LLR is the
+ * largest |sum of the group's complex tone amplitudes| over the 8^g tone patterns with the bit 1 minus that with the bit 0, normalised as
+ * set a.  The chain after set a's BP is OSD (when on) and AP (when on) on set a, then BP, OSD and AP on set b and on set c, each on what
+ * the steps before left at stage 1 or 2, with the acceptance rules of that decoder; a step's hard distance is counted against the set
+ * it decodes, and its cap is min(the decoder's own cap, max_hard_errors) -- the fine-sync cap for BP.  fs / fs_hard keep their meaning
+ * (fs = 2: decoded by any step; fs_hard: the accepted word's distance, otherwise set a's BP's).  on: 0 = off (default; nothing
+ * launched or allocated, every output as without this call), 1 = on; anything else is FT8B200_EINVAL.  It does nothing while fine sync
+ * is off.  The process_* calls (every pass) and the stage-wise ft8b200_finesync honour it.  max_hard_errors < 0 selects
+ * FT8B200_FINESYNC_DEEP_DEFAULT_MAX_HARD: the largest cap at which deep fine sync decoded no message at all on 4096 noise-only daemon
+ * slots (K = 120) with OSD {0, 2} x AP {0, 1} (tools/perf_finesync_deep.py; profiles/perf_finesync_deep.json).  Measured on a B200 at
+ * 1000 W: at cap 174 it decoded one message, by OSD on set c at hard distance 31 (with OSD order 2), and at cap 30 nothing, so the
+ * rule gives 30.  Decode time in ft8b200_stage_times includes it. */
+#define FT8B200_FINESYNC_DEEP_DEFAULT_MAX_HARD 30
+int ft8b200_set_finesync_deep(ft8b200_ctx_t *ctx, int on, int max_hard_errors);
+/* The front half of deep fine sync on its own, whatever the switches: for the candidates at stage 1 or 2 of the n_slots x
+ * max_candidates entries, fine sync's search (d_grid, as ft8b200_finesync's d_fs_grid) and the three refined LLR sets into d_llr_sets
+ * (float [3][n_slots][max_candidates][174]: set a, as ft8b200_finesync's d_fs_llr, then sets b and c); other entries are not written.
+ * Slots as ft8b200_finesync; any n_slots outside 1 ... 65535 or a float or int32 buffer not 4-byte aligned is FT8B200_EINVAL, and
+ * nothing is written.  tests/finesync_deep_ref.py is the float64 definition. */
+int ft8b200_finesync_sets(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, int n_slots, const candidate_t *d_cand, const int *d_ncand,
+                          const uint8_t *d_stage, int32_t *d_grid, float *d_llr_sets, void *stream);
+/* d_fs_how (uint8, n_slots x max_candidates) of pass 1 of the last process_* batch, or of the last stage-wise ft8b200_finesync, run with
+ * deep fine sync: 0 = not decoded by fine sync, else 1 + 3 set + decoder (set a, b, c = 0, 1, 2; BP, OSD, AP = 0, 1, 2); NULL before
+ * any deep run */
+int ft8b200_finesync_deep_workspace(ft8b200_ctx_t *ctx, uint8_t **d_fs_how);
 /* Multi-pass decoding (DESIGN.md section 2.4.2) on the daemon path -- every process_raw*, process_slots / process_conditioned call,
  * and through them the pipe, the cluster, the drop-in ft8_subsystem, the stream and .iq file paths.  passes = 1 (default) decodes
  * a slot once, exactly as without this call.  With 2 or 3, after each pass the messages the spot table accepted as new in that
@@ -506,6 +533,8 @@ int ft8b200_pipe_set_ap(ft8b200_pipe_t *p, int on, int max_hard_errors);
 int ft8b200_pipe_set_passes(ft8b200_pipe_t *p, int passes);
 /* ft8b200_set_finesync on every lane (a cluster's pipes through ft8b200_cluster_pipe).  FT8B200_EBUSY while batches are in flight. */
 int ft8b200_pipe_set_finesync(ft8b200_pipe_t *p, int on, int max_hard_errors);
+/* ft8b200_set_finesync_deep on every lane (a cluster's pipes through ft8b200_cluster_pipe).  FT8B200_EBUSY while batches are in flight. */
+int ft8b200_pipe_set_finesync_deep(ft8b200_pipe_t *p, int on, int max_hard_errors);
 int ft8b200_pipe_autotune(ft8b200_pipe_t *p, const uint8_t *d_iq, size_t bytes_per_stream, size_t stream_stride_bytes, int n_slots,
                           const int *candidates, int n_candidates, int batches, int *best_back_sms, int *best_comb_front, float *ms_out);
 void ft8b200_pipe_destroy(ft8b200_pipe_t *p);

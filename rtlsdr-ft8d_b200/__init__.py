@@ -329,6 +329,30 @@ class Context:
         self._chk(self.L.ft8b200_finesync_workspace(C.c_void_p(self.h), C.byref(a), C.byref(b)))
         return a.value or 0, b.value or 0
 
+    def set_finesync_deep(self, on: int, max_hard_errors: int = -1):
+        """Deep fine sync (sets a, b, c and OSD / AP on them; only while fine sync is on): 0 (off) or 1; max_hard_errors < 0 =
+        FT8B200_FINESYNC_DEEP_DEFAULT_MAX_HARD."""
+        self._chk(self.L.ft8b200_set_finesync_deep(C.c_void_p(self.h), int(on), int(max_hard_errors)))
+
+    def finesync_sets(self, d_i, d_q, cand, ncand, stage, stream: int | None = None):
+        """Deep fine sync's front half on slots d_i / d_q float32 [n, 48000] -> (grid int32[n, K, 2], llr float32[3, n, K, 174] of sets
+        a, b, c), written for the candidates at stage 1 or 2 only (zeros elsewhere)."""
+        import torch
+        n = d_i.shape[0]
+        dev = d_i.device
+        grid = torch.zeros((n, self.K, 2), dtype=torch.int32, device=dev)
+        llr = torch.zeros((3, n, self.K, 174), dtype=torch.float32, device=dev)
+        self._chk(self.L.ft8b200_finesync_sets(C.c_void_p(self.h), _p(d_i), _p(d_q), n, _p(cand), _p(ncand), _p(stage), _p(grid), _p(llr),
+                                               _st(stream)))
+        return grid, llr
+
+    def finesync_deep_workspace_ptrs(self):
+        """Device pointer of fs_how (uint8 [n, K]; 0 = not a fine-sync decode, else 1 + 3 set + decoder) of pass 1 of the last batch, or
+        stage-wise ft8b200_finesync, run with deep fine sync (0 before that)."""
+        a = C.c_void_p(0)
+        self._chk(self.L.ft8b200_finesync_deep_workspace(C.c_void_p(self.h), C.byref(a)))
+        return a.value or 0
+
     def set_passes(self, passes: int):
         """Multi-pass decoding with signal subtraction on the daemon path: 1 (default, one pass), 2 or 3 (ft8b200_set_passes)."""
         self._chk(self.L.ft8b200_set_passes(C.c_void_p(self.h), int(passes)))
@@ -600,6 +624,10 @@ class Pipe:
     def set_finesync(self, on: int, max_hard_errors: int = -1):
         """Context.set_finesync on every lane; not while batches are in flight."""
         self._chk(self.L.ft8b200_pipe_set_finesync(C.c_void_p(self.h), int(on), int(max_hard_errors)))
+
+    def set_finesync_deep(self, on: int, max_hard_errors: int = -1):
+        """Context.set_finesync_deep on every lane; not while batches are in flight."""
+        self._chk(self.L.ft8b200_pipe_set_finesync_deep(C.c_void_p(self.h), int(on), int(max_hard_errors)))
 
     def set_passes(self, passes: int):
         """Context.set_passes on every lane; not while batches are in flight."""

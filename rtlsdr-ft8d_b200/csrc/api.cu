@@ -8,6 +8,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
 #include <mutex>
 #include <string>
 #include <vector>
@@ -65,42 +66,44 @@ struct DevBuf {
 };
 
 // The per-candidate rows of one pass over S slots of K candidates: what find_sync and BP write, the codewords multi-pass decoding
-// subtracts (plain), the LLRs OSD and AP read, and the flag and hard-distance pair of each retry decoder (OSD, AP, fine sync).
-// A buffer whose option is off is not allocated.
+// subtracts (plain), the LLRs OSD and AP read, the flag and hard-distance pair of each retry decoder (OSD, AP, fine sync), and which
+// step of deep fine sync decoded a candidate (fs_how).  A buffer whose option is off is not allocated.
 struct Rows {
-    DevBuf mag, cand, ncand, ok, stage, status, msg, plain, llr, osd, osd_hard, ap, ap_hard, fs, fs_hard;
+    DevBuf mag, cand, ncand, ok, stage, status, msg, plain, llr, osd, osd_hard, ap, ap_hard, fs, fs_hard, fs_how;
     // the rows of slots s0...: every pointer moved to slot s0, nullptr for a buffer that does not exist or (llr, plain) is not used
     struct View {
         uint8_t *mag; candidate_t *cand; int *ncand; uint8_t *ok, *stage; decode_status_t *status; message_t *msg; uint8_t *plain; float *llr;
-        uint8_t *osd; int32_t *osd_hard; uint8_t *ap; int32_t *ap_hard; uint8_t *fs; int32_t *fs_hard;
+        uint8_t *osd; int32_t *osd_hard; uint8_t *ap; int32_t *ap_hard; uint8_t *fs; int32_t *fs_hard; uint8_t *fs_how;
     };
     // the LLRs and the pair of each retry decoder that is on
-    int ensure_retry(size_t S, size_t K, bool osd_on, bool ap_on, bool fs_on) {
+    int ensure_retry(size_t S, size_t K, bool osd_on, bool ap_on, bool fs_on, bool deep_on) {
         const size_t E = S * K;
         int rc;
         if ((osd_on || ap_on) && (rc = llr.ensure(E * kLdpcN * sizeof(float)))) return rc;
         if (osd_on && ((rc = osd.ensure(E)) || (rc = osd_hard.ensure(E * sizeof(int32_t))))) return rc;
         if (ap_on && ((rc = ap.ensure(E)) || (rc = ap_hard.ensure(E * sizeof(int32_t))))) return rc;
         if (fs_on && ((rc = fs.ensure(E)) || (rc = fs_hard.ensure(E * sizeof(int32_t))))) return rc;
+        if (deep_on && (rc = fs_how.ensure(E))) return rc;
         return 0;
     }
-    int ensure(size_t S, size_t K, bool osd_on, bool ap_on, bool fs_on, bool need_plain) {
+    int ensure(size_t S, size_t K, bool osd_on, bool ap_on, bool fs_on, bool deep_on, bool need_plain) {
         int rc;
         if ((rc = mag.ensure(S * kWfBytes)) || (rc = cand.ensure(S * K * sizeof(candidate_t))) || (rc = ncand.ensure(S * sizeof(int)))) return rc;
         if ((rc = ok.ensure(S * K)) || (rc = stage.ensure(S * K)) || (rc = status.ensure(S * K * sizeof(decode_status_t)))) return rc;
         if ((rc = msg.ensure(S * K * sizeof(message_t)))) return rc;
         if (need_plain && (rc = plain.ensure(S * K * kLdpcN))) return rc;
-        return ensure_retry(S, K, osd_on, ap_on, fs_on);
+        return ensure_retry(S, K, osd_on, ap_on, fs_on, deep_on);
     }
     void release() {
-        for (DevBuf *b : {&mag, &cand, &ncand, &ok, &stage, &status, &msg, &plain, &llr, &osd, &osd_hard, &ap, &ap_hard, &fs, &fs_hard}) b->release();
+        for (DevBuf *b : {&mag, &cand, &ncand, &ok, &stage, &status, &msg, &plain, &llr, &osd, &osd_hard, &ap, &ap_hard, &fs, &fs_hard, &fs_how})
+            b->release();
     }
     View at(int s0, size_t K, bool llr_on, bool plain_on) const {
         const size_t o = (size_t)s0 * K;
         return {mag.at<uint8_t>((size_t)s0 * kWfBytes), cand.at<candidate_t>(o), ncand.at<int>(s0), ok.at<uint8_t>(o), stage.at<uint8_t>(o),
                 status.at<decode_status_t>(o), msg.at<message_t>(o), plain_on ? plain.at<uint8_t>(o * kLdpcN) : nullptr,
                 llr_on ? llr.at<float>(o * kLdpcN) : nullptr, osd.at<uint8_t>(o), osd_hard.at<int32_t>(o), ap.at<uint8_t>(o),
-                ap_hard.at<int32_t>(o), fs.at<uint8_t>(o), fs_hard.at<int32_t>(o)};
+                ap_hard.at<int32_t>(o), fs.at<uint8_t>(o), fs_hard.at<int32_t>(o), fs_how.at<uint8_t>(o)};
     }
 };
 }  // namespace
@@ -128,6 +131,12 @@ struct ft8b200_ctx {
     int fs_on = 0;
     int fs_max_hard = FT8B200_FINESYNC_DEFAULT_MAX_HARD;
     DevBuf fs_llr, fs_grid;
+    // deep fine sync (ft8b200_set_finesync_deep), 0 = off: with fine sync on, the nsym = 2 and 3 sets and OSD / AP on the refined sets.
+    // Scratch, for slots s0 ... s0 + n at offset s0: sets b and c (deep_llr, [2][n][K][174]) and the flag / hard rows of the 8 extra
+    // retry steps (deep_flag, deep_hard, [8][n][K])
+    int fs_deep = 0;
+    int fs_deep_max_hard = FT8B200_FINESYNC_DEEP_DEFAULT_MAX_HARD;
+    DevBuf deep_llr, deep_flag, deep_hard;
     // multi-pass decoding (ft8b200_set_passes): 1 = off.  With passes > 1: the slot's log of accepted messages across passes
     // (ulog/ufreq/uscore/ucand, first = record count before the last pass), the refined grid points, the residual slots (ri/rq), and
     // the rows of the later passes
@@ -174,13 +183,17 @@ int ensure_slot_buffers(ft8b200_ctx_t *ctx, int n_slots) {
     const size_t K = (size_t)ctx->cfg.max_candidates, M = (size_t)ctx->cfg.max_messages, S = (size_t)n_slots;
     const bool multi = ctx->passes > 1;
     int rc;
-    if ((rc = ctx->pass1.ensure(S, K, ctx->osd_order, ctx->ap_on, ctx->fs_on, multi))) return rc;
+    const bool deep = ctx->fs_on && ctx->fs_deep;
+    if ((rc = ctx->pass1.ensure(S, K, ctx->osd_order, ctx->ap_on, ctx->fs_on, deep, multi))) return rc;
     if ((rc = ctx->results.ensure(S * M * sizeof(struct decoder_results)))) return rc;
     if ((rc = ctx->nresults.ensure(S * sizeof(int32_t)))) return rc;
     if ((rc = ctx->table.ensure(S * M * sizeof(int16_t)))) return rc;
     if (ctx->fs_on && ((rc = ctx->fs_llr.ensure(S * K * kLdpcN * sizeof(float))) || (rc = ctx->fs_grid.ensure(S * K * 2 * sizeof(int32_t))))) return rc;
+    if (deep && ((rc = ctx->deep_llr.ensure(2 * S * K * kLdpcN * sizeof(float))) || (rc = ctx->deep_flag.ensure(8 * S * K)) ||
+                 (rc = ctx->deep_hard.ensure(8 * S * K * sizeof(int32_t)))))
+        return rc;
     if (!multi) return 0;
-    if ((rc = ctx->later.ensure(S, K, ctx->osd_order, ctx->ap_on, ctx->fs_on, true))) return rc;
+    if ((rc = ctx->later.ensure(S, K, ctx->osd_order, ctx->ap_on, ctx->fs_on, deep, true))) return rc;
     if ((rc = ctx->ulog.ensure(S * M * sizeof(message_t))) || (rc = ctx->ufreq.ensure(S * M * sizeof(float)))) return rc;
     if ((rc = ctx->uscore.ensure(S * M * sizeof(int32_t))) || (rc = ctx->ucand.ensure(S * M * sizeof(int32_t)))) return rc;
     if ((rc = ctx->first.ensure(S * sizeof(int32_t))) || (rc = ctx->grid.ensure(S * M * 2 * sizeof(int32_t)))) return rc;
@@ -197,10 +210,44 @@ int ensure_scratch(ft8b200_ctx_t *ctx, int npos, int n_slots) {
     return 0;
 }
 
+// Deep fine sync (DESIGN.md section 2.4.6) after the BP on set a (llr[0]) of n slots: OSD and AP on set a, then BP, OSD and AP on sets
+// b and c, each where it is on and on what the steps before left at stage 1 or 2, capped at min(its own cap, the deep cap), their
+// outcomes into step i's rows of flag / hard ([8][n][K]); then the merge into fs / fs_hard / fs_how.  Every step walks its entries in
+// a fixed stride, so none needs a pull counter.
+int launch_deep(ft8b200_ctx_t *ctx, const Rows::View &r, int n, const float *const (&llr)[3], uint8_t *flag, int32_t *hard, uint8_t *fs,
+                int32_t *fs_hard, uint8_t *fs_how, const uint32_t *work, const unsigned int *total, int sms, cudaStream_t st) {
+    const int K = ctx->cfg.max_candidates, iters = ctx->cfg.ldpc_iterations, cap = ctx->fs_deep_max_hard;
+    const size_t nk = (size_t)n * K;
+    unsigned int steps = 0;
+    for (int set = 0; set < 3; ++set) {
+        for (int dec = set ? 0 : 1; dec < 3; ++dec) {   // BP, OSD, AP; set a's BP has run
+            const int i = 3 * set + dec - 1;
+            uint8_t *f = flag + i * nk;
+            int32_t *h = hard + i * nk;
+            if (dec == 0) {
+                CU(launch_rebp(n, K, PROTO_FT8, Hypothesis{}, 1, std::min(ctx->fs_max_hard, cap), iters, llr[set], r.ncand, r.ok, r.stage, r.status, r.msg,
+                               r.plain, f, h, work, total, nullptr, sms, st, &ctx->launches));
+            } else if (dec == 1) {
+                if (!ctx->osd_order) continue;
+                CU(launch_osd(n, K, PROTO_FT8, ctx->osd_order, std::min(ctx->osd_max_hard, cap), llr[set], r.ncand, r.ok, r.stage, r.status, r.msg, r.plain,
+                              f, h, nullptr, work, total, nullptr, sms, st, &ctx->launches));
+            } else {
+                if (!ctx->ap_on) continue;
+                CU(launch_rebp(n, K, PROTO_FT8, cq_hypothesis(PROTO_FT8), 1, std::min(ctx->ap_max_hard, cap), iters, llr[set], r.ncand, r.ok, r.stage,
+                               r.status, r.msg, r.plain, f, h, work, total, nullptr, sms, st, &ctx->launches));
+            }
+            steps |= 1u << i;
+        }
+    }
+    CU(launch_finesync_merge(nk, steps, flag, hard, fs, fs_hard, fs_how, sms, st, &ctx->launches));
+    return 0;
+}
+
 // What runs after BP on the rows r of n slots starting at slot s0: OSD, AP and fine sync, each where it is on, each on what the ones
 // before it left at stage 1 or 2.  With the work list (the whole path) they visit its entries and find_sync has zeroed their pull
 // counters, words [2] - [4] of work_total; without it (ft8b200_decode) they visit every entry and the counters they use are zeroed
-// here.  Fine sync demodulates the slot samples xi / xq (kSlot floats per slot); without samples it does not run.
+// here.  Fine sync demodulates the slot samples xi / xq (kSlot floats per slot); without samples it does not run.  Deep fine sync
+// (launch_deep) follows it where on.
 int launch_retries(ft8b200_ctx_t *ctx, int protocol, const Rows::View &r, int s0, int n, const float *xi, const float *xq, const uint32_t *work,
                    int sms, cudaStream_t st) {
     const int K = ctx->cfg.max_candidates, iters = ctx->cfg.ldpc_iterations;
@@ -218,11 +265,20 @@ int launch_retries(ft8b200_ctx_t *ctx, int protocol, const Rows::View &r, int s0
     }
     if (ctx->fs_on && xi) {  // (finesync_kernel demodulates FT8)
         float *fs_llr = ctx->fs_llr.as<float>() + (size_t)s0 * K * kLdpcN;
+        const bool deep = ctx->fs_deep;
+        float *deep_llr = deep ? ctx->deep_llr.as<float>() + 2 * (size_t)s0 * K * kLdpcN : nullptr;
+        const size_t set_floats = (size_t)n * K * kLdpcN;
         if (!work) CU(cudaMemsetAsync(counters + 4, 0, sizeof(unsigned int), st));
-        CU(launch_finesync(n, K, 1, xi, xq, r.cand, r.ncand, r.stage, fs_llr, ctx->fs_grid.as<int32_t>() + (size_t)s0 * K * 2, work, total,
-                           counters + 4, sms, st, &ctx->launches));
+        CU(launch_finesync(n, K, 1, deep, xi, xq, r.cand, r.ncand, r.stage, fs_llr, deep_llr, deep ? deep_llr + set_floats : nullptr,
+                           ctx->fs_grid.as<int32_t>() + (size_t)s0 * K * 2, work, total, counters + 4, sms, st, &ctx->launches));
         CU(launch_rebp(n, K, PROTO_FT8, Hypothesis{}, 1, ctx->fs_max_hard, iters, fs_llr, r.ncand, r.ok, r.stage, r.status, r.msg, r.plain, r.fs,
                        r.fs_hard, work, total, nullptr, sms, st, &ctx->launches));
+        if (deep) {
+            const float *const sets[3] = {fs_llr, deep_llr, deep_llr + set_floats};
+            if (int rc = launch_deep(ctx, r, n, sets, ctx->deep_flag.as<uint8_t>() + 8 * (size_t)s0 * K, ctx->deep_hard.as<int32_t>() + 8 * (size_t)s0 * K,
+                                     r.fs, r.fs_hard, r.fs_how, work, total, sms, st))
+                return rc;
+        }
     }
     return 0;
 }
@@ -326,8 +382,8 @@ void ft8b200_destroy(ft8b200_ctx_t *ctx) {
     cudaFree(ctx->tb.window1024); cudaFree(ctx->tb.twiddle1024); cudaFree(ctx->tb.db_thresholds); cudaFree(ctx->tb.wf_blob);
     cudaFree(ctx->tb.mon_window); cudaFree(ctx->tb.mon_twiddle); cudaFree(ctx->tb.mon_super);
     DevBuf *bufs[] = {&ctx->raw, &ctx->sums, &ctx->si, &ctx->sq, &ctx->peak, &ctx->count, &ctx->results, &ctx->nresults, &ctx->table, &ctx->lists,
-                      &ctx->scores, &ctx->work, &ctx->work_total, &ctx->fs_llr, &ctx->fs_grid, &ctx->ulog, &ctx->ufreq, &ctx->uscore, &ctx->ucand,
-                      &ctx->first, &ctx->grid, &ctx->ri, &ctx->rq, &ctx->sub_scratch};
+                      &ctx->scores, &ctx->work, &ctx->work_total, &ctx->fs_llr, &ctx->fs_grid, &ctx->deep_llr, &ctx->deep_flag, &ctx->deep_hard,
+                      &ctx->ulog, &ctx->ufreq, &ctx->uscore, &ctx->ucand, &ctx->first, &ctx->grid, &ctx->ri, &ctx->rq, &ctx->sub_scratch};
     for (DevBuf *b : bufs) b->release();
     ctx->pass1.release();
     ctx->later.release();
@@ -455,7 +511,7 @@ int decode_proto(ft8b200_ctx_t *ctx, int protocol, const uint8_t *d_mag, size_t 
     }
     // OSD's and AP's outputs go to pass 1's rows (ft8b200_osd_workspace, ft8b200_ap_workspace), and so do the LLRs when the caller
     // passes none; everything else is the caller's
-    if ((rc = ctx->pass1.ensure_retry((size_t)n_slots, (size_t)ctx->cfg.max_candidates, ctx->osd_order, ctx->ap_on, false))) return rc;
+    if ((rc = ctx->pass1.ensure_retry((size_t)n_slots, (size_t)ctx->cfg.max_candidates, ctx->osd_order, ctx->ap_on, false, false))) return rc;
     Rows::View r = ctx->pass1.at(0, ctx->cfg.max_candidates, ctx->osd_order || ctx->ap_on, false);
     r.cand = const_cast<candidate_t *>(d_cand);  // the retry decoders only read the candidates
     r.ncand = const_cast<int *>(d_ncand);
@@ -524,6 +580,15 @@ int ft8b200_set_finesync(ft8b200_ctx_t *ctx, int on, int max_hard_errors) {
     std::lock_guard<std::mutex> lk(ctx->mu);
     ctx->fs_on = on;
     ctx->fs_max_hard = max_hard_errors < 0 ? FT8B200_FINESYNC_DEFAULT_MAX_HARD : max_hard_errors;
+    return 0;
+}
+
+int ft8b200_set_finesync_deep(ft8b200_ctx_t *ctx, int on, int max_hard_errors) {
+    if (!ctx) return fail(FT8B200_EINVAL, "null context");
+    if (on != 0 && on != 1) return fail(FT8B200_EINVAL, "ft8b200_set_finesync_deep: on must be 0 (off, the default) or 1");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    ctx->fs_deep = on;
+    ctx->fs_deep_max_hard = max_hard_errors < 0 ? FT8B200_FINESYNC_DEEP_DEFAULT_MAX_HARD : max_hard_errors;
     return 0;
 }
 
@@ -610,19 +675,61 @@ int ft8b200_finesync(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, int
     if ((((size_t)d_i) | ((size_t)d_q) | ((size_t)d_fs_llr)) & 3) return fail(FT8B200_EINVAL, "ft8b200_finesync: float buffers must be 4-byte aligned");
     std::lock_guard<std::mutex> lk(ctx->mu);
     if ((rc = ctx->work_total.ensure(5 * sizeof(unsigned int)))) return rc;
+    const int K = ctx->cfg.max_candidates;
+    const size_t nk = (size_t)n_slots * K;
     if (!d_fs_llr) {
-        if ((rc = ctx->fs_llr.ensure((size_t)n_slots * ctx->cfg.max_candidates * kLdpcN * sizeof(float)))) return rc;
+        if ((rc = ctx->fs_llr.ensure(nk * kLdpcN * sizeof(float)))) return rc;
         d_fs_llr = ctx->fs_llr.as<float>();
     }
+    // deep mode: sets b and c and the extra steps' rows in the context's scratch, fs_how into pass 1's row (ft8b200_finesync_deep_workspace)
+    const bool deep = ctx->fs_on && ctx->fs_deep;
+    if (deep && ((rc = ctx->deep_llr.ensure(2 * nk * kLdpcN * sizeof(float))) || (rc = ctx->deep_flag.ensure(8 * nk)) ||
+                 (rc = ctx->deep_hard.ensure(8 * nk * sizeof(int32_t))) || (rc = ctx->pass1.fs_how.ensure(nk))))
+        return rc;
+    float *deep_llr = deep ? ctx->deep_llr.as<float>() : nullptr;
     cudaStream_t st = pick(ctx, stream);
     unsigned int *next = ctx->work_total.as<unsigned int>() + 4;
     CU(cudaMemsetAsync(next, 0, sizeof(unsigned int), st));
-    const int K = ctx->cfg.max_candidates;
-    CU(launch_finesync(n_slots, K, ctx->fs_on, d_i, d_q, d_cand, d_ncand, d_stage, d_fs_llr, d_fs_grid, nullptr, nullptr, next, ctx->sm_count, st,
-                       &ctx->launches));
+    CU(launch_finesync(n_slots, K, ctx->fs_on, deep, d_i, d_q, d_cand, d_ncand, d_stage, d_fs_llr, deep_llr, deep ? deep_llr + nk * kLdpcN : nullptr,
+                       d_fs_grid, nullptr, nullptr, next, ctx->sm_count, st, &ctx->launches));
     CU(launch_rebp(n_slots, K, PROTO_FT8, Hypothesis{}, ctx->fs_on, ctx->fs_max_hard, ctx->cfg.ldpc_iterations, d_fs_llr, d_ncand, d_ok, d_stage, d_status,
                    d_msg, d_plain, d_fs, d_fs_hard, nullptr, nullptr, nullptr, ctx->sm_count, st, &ctx->launches));
+    if (deep) {
+        Rows::View r = {};
+        r.ncand = const_cast<int *>(d_ncand);   // the retry decoders only read the counts
+        r.ok = d_ok; r.stage = d_stage; r.status = d_status; r.msg = d_msg; r.plain = d_plain;
+        const float *const sets[3] = {d_fs_llr, deep_llr, deep_llr + nk * kLdpcN};
+        if ((rc = launch_deep(ctx, r, n_slots, sets, ctx->deep_flag.as<uint8_t>(), ctx->deep_hard.as<int32_t>(), d_fs, d_fs_hard,
+                              ctx->pass1.fs_how.as<uint8_t>(), nullptr, nullptr, ctx->sm_count, st)))
+            return rc;
+    }
     tally(ctx);
+    return 0;
+}
+
+int ft8b200_finesync_sets(ft8b200_ctx_t *ctx, const float *d_i, const float *d_q, int n_slots, const candidate_t *d_cand, const int *d_ncand,
+                          const uint8_t *d_stage, int32_t *d_grid, float *d_llr_sets, void *stream) {
+    int rc = ctx_enter(ctx);
+    if (rc) return rc;
+    if (!d_i || !d_q || !d_cand || !d_ncand || !d_stage || !d_grid || !d_llr_sets || n_slots < 1 || n_slots > FT8B200_MAX_RAW_ROWS)
+        return fail(FT8B200_EINVAL, "ft8b200_finesync_sets: null buffer or n_slots outside 1 ... 65535");
+    if ((((size_t)d_i) | ((size_t)d_q) | ((size_t)d_grid) | ((size_t)d_llr_sets)) & 3)
+        return fail(FT8B200_EINVAL, "ft8b200_finesync_sets: d_i, d_q, d_grid and d_llr_sets must be 4-byte aligned");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    if ((rc = ctx->work_total.ensure(5 * sizeof(unsigned int)))) return rc;
+    cudaStream_t st = pick(ctx, stream);
+    unsigned int *next = ctx->work_total.as<unsigned int>() + 4;
+    CU(cudaMemsetAsync(next, 0, sizeof(unsigned int), st));
+    const size_t set_floats = (size_t)n_slots * ctx->cfg.max_candidates * kLdpcN;
+    CU(launch_finesync(n_slots, ctx->cfg.max_candidates, 1, 1, d_i, d_q, d_cand, d_ncand, d_stage, d_llr_sets, d_llr_sets + set_floats,
+                       d_llr_sets + 2 * set_floats, d_grid, nullptr, nullptr, next, ctx->sm_count, st, &ctx->launches));
+    tally(ctx);
+    return 0;
+}
+
+int ft8b200_finesync_deep_workspace(ft8b200_ctx_t *ctx, uint8_t **d_fs_how) {
+    if (!ctx) return fail(FT8B200_EINVAL, "null context");
+    if (d_fs_how) *d_fs_how = ctx->pass1.fs_how.as<uint8_t>();
     return 0;
 }
 

@@ -101,12 +101,18 @@ cudaError_t launch_rebp(int n_slots, int max_cand, int protocol, const Hypothesi
                         int sm_count, cudaStream_t st, int *launches);
 // fine-sync decoding, front half (finesync.cu): for the entries BP, OSD and AP left at stage 1 or 2 (on = 0: nothing attempted), the
 // Costas search on the slots d_xi / d_xq (kSlot floats per slot) and the refined LLRs into d_llr ([n_slots][max_cand][174]) and d_grid
-// ([n_slots][max_cand][2]), for the entries it attempts only; work list as launch_osd, *d_next: its pull counter, zeroed by the
-// caller.  launch_rebp on d_llr is the back half.
+// ([n_slots][max_cand][2]), for the entries it attempts only; deep = 1 also writes sets b and c (DESIGN.md section 2.4.6) into d_llr_b
+// and d_llr_c, laid out as d_llr.  Work list as launch_osd, *d_next: its pull counter, zeroed by the caller.  launch_rebp on d_llr is
+// the back half.
 cudaError_t upload_finesync_tables();
-cudaError_t launch_finesync(int n_slots, int max_cand, int on, const float *d_xi, const float *d_xq, const candidate_t *d_cand, const int *d_ncand,
-                            const uint8_t *d_stage, float *d_llr, int32_t *d_grid, const uint32_t *d_work, const unsigned int *d_work_total,
-                            unsigned int *d_next, int sm_count, cudaStream_t st, int *launches);
+cudaError_t launch_finesync(int n_slots, int max_cand, int on, int deep, const float *d_xi, const float *d_xq, const candidate_t *d_cand,
+                            const int *d_ncand, const uint8_t *d_stage, float *d_llr, float *d_llr_b, float *d_llr_c, int32_t *d_grid,
+                            const uint32_t *d_work, const unsigned int *d_work_total, unsigned int *d_next, int sm_count, cudaStream_t st,
+                            int *launches);
+// deep mode's last step: the n entries' flag / hard rows of retry step i (0 ... 7, at d_flag / d_hard + i * n; bit i of `steps` = it
+// ran) folded into d_fs / d_fs_hard, and d_how (0 = not decoded by fine sync, 1 + 3 set + decoder) written for every entry
+cudaError_t launch_finesync_merge(size_t n, unsigned int steps, const uint8_t *d_flag, const int32_t *d_hard, uint8_t *d_fs, int32_t *d_fs_hard,
+                                  uint8_t *d_how, int sm_count, cudaStream_t st, int *launches);
 cudaError_t launch_unpack77_batch(const uint8_t *d_payloads, int n, char *d_text32, int32_t *d_status, cudaStream_t st, int *launches);
 cudaError_t upload_ldpc_tables();
 void set_decode_variant(int v);  // 0 = node-centred belief propagation (default), 1 = edge-centred

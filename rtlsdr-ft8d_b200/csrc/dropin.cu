@@ -133,9 +133,10 @@ ft8b200_ctx_t *default_ctx() {
         // deeper decoding for a relinked program without code changes: FT8B200_OSD=<order>, FT8B200_OSD_MAX_HARD=<cap> (INTEGRATION.md)
         const char *osd = getenv("FT8B200_OSD"), *cap = getenv("FT8B200_OSD_MAX_HARD");
         if (osd && ft8b200_set_osd(g_ctx, atoi(osd), cap ? atoi(cap) : -1) != 0) die("FT8B200_OSD (0, 1 or 2)");
-        // a-priori decoding of CQ calls and fine-sync decoding (INTEGRATION.md)
+        // a-priori decoding of CQ calls, fine-sync decoding and its deep mode (INTEGRATION.md)
         set_from_env(g_ctx, "FT8B200_AP", ft8b200_set_ap);
         set_from_env(g_ctx, "FT8B200_FINESYNC", ft8b200_set_finesync);
+        set_from_env(g_ctx, "FT8B200_FINESYNC_DEEP", ft8b200_set_finesync_deep);
         // multi-pass decoding with signal subtraction: FT8B200_PASSES=<1, 2 or 3>
         const char *passes = getenv("FT8B200_PASSES");
         if (passes && ft8b200_set_passes(g_ctx, atoi(passes)) != 0) die("FT8B200_PASSES (1, 2 or 3)");

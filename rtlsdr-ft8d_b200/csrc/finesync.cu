@@ -10,6 +10,9 @@
 //   c[k][j] = sum_{m < 512} x[s* + 512 k + m] exp(-2 pi i (f* + 6.25 j) m / 3200), k < 79, j < 8; E = mean |c|^2;
 //   v = 10 log10(|c|^2 / E + 1e-12), the max-log bit metrics of extract_llrs over v, normalised as a10 (scale sqrt(24 / var)).
 // E = 0 (nothing of the span inside the slot, or a silent one) writes NaN LLRs: the back half then does not attempt the candidate.
+// Deep mode (finesync_kernel<true>, DESIGN.md section 2.4.6, tests/finesync_deep_ref.py) also writes sets b and c, the nsym = 2 and 3
+// coherent metrics: c'[k][j] = c[k][j] exp(-2 pi i f* 512 k / 3200) (one time origin for every symbol), and per group of g consecutive
+// data symbols of a half A(b) = |sum_t c'[sym_t][gray[b_t]]| over the 8^g patterns, bit LLR = max A (bit 1) - max A (bit 0).
 #include "common.cuh"
 #include "ft8_tables.h"
 #include "slot_search.cuh"
@@ -41,6 +44,7 @@ struct FsArgs {
     float *llr;                      // [n_slots][max_cand][174]
     int32_t *grid;                   // [n_slots][max_cand][2]: dt samples, df steps
     const uint32_t *work; const unsigned int *work_total; unsigned int *next;
+    float *llr_b, *llr_c;            // deep mode: sets b (nsym = 2) and c (nsym = 3), laid out as llr
 };
 
 // x[n] exp(-2 pi i f m / fs) needs the phase of f m / fs: formed in double, only its fractional cycle goes through sincospif
@@ -53,7 +57,74 @@ __device__ __forceinline__ float2 tone(double f_hz, int m) {
 
 __device__ __forceinline__ int costas_symbol(int q) { return q < 7 ? q : (q < 14 ? q + 29 : q + 58); }   // 0-6, 36-42, 72-78
 
+// Deep mode, one group of G consecutive data symbols starting at symbol sym0, on one warp: lane l takes the patterns l, l + 32 ...
+// (pattern p: symbol t carries Gray index (p >> 3 (G - 1 - t)) & 7, so bit q of the group is bit 3 G - 1 - q of p), keeps the
+// largest A with each bit 1 and 0, and the warp takes the maxima of those (max is exact, so the result does not depend on the order).
+// raw[q] = the group's unnormalised LLRs, written by lane 0.
+template <int G>
+__device__ __forceinline__ void group_llrs(const float2 *C, int sym0, int lane, float *raw) {
+    float m1[3 * G], m0[3 * G];
+#pragma unroll
+    for (int q = 0; q < 3 * G; ++q) m1[q] = m0[q] = 0.0f;
+    for (int p = lane; p < (1 << (3 * G)); p += 32) {
+        float re = 0.0f, im = 0.0f;
+#pragma unroll
+        for (int t = 0; t < G; ++t) {
+            const float2 z = C[(sym0 + t) * 8 + c_gray[(p >> (3 * (G - 1 - t))) & 7]];
+            re += z.x;
+            im += z.y;
+        }
+        const float A = sqrtf(re * re + im * im);
+#pragma unroll
+        for (int q = 0; q < 3 * G; ++q) {
+            if ((p >> (3 * G - 1 - q)) & 1) m1[q] = fmaxf(m1[q], A);
+            else m0[q] = fmaxf(m0[q], A);
+        }
+    }
+#pragma unroll
+    for (int q = 0; q < 3 * G; ++q) {   // A >= 0: its bit pattern orders as an unsigned integer
+        const float hi = __uint_as_float(__reduce_max_sync(0xffffffffu, __float_as_uint(m1[q])));
+        const float lo = __uint_as_float(__reduce_max_sync(0xffffffffu, __float_as_uint(m0[q])));
+        if (lane == 0) raw[q] = hi - lo;
+    }
+}
+
+// Deep mode: sets b and c of one candidate from the symbol-referenced spectra C [79][8] and the tone powers P (for E), the whole CTA.
+// The groups of a half start at its first data symbol; the last takes what remains (nsym = 2: 14 pairs and a single, nsym = 3: 9
+// triples and a pair).  The 30 + 20 groups go to the warps in turn, then warps 0 and 1 normalise sets b and c as set a is (a10).
+__device__ void deep_sets(const FsArgs &a, size_t oidx, const float2 *C, const float *P, float *raw) {
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    for (int task = warp; task < 50; task += kThreads / 32) {
+        const int set = task < 30 ? 0 : 1, nsym = 2 + set, u = task - 30 * set, per = set ? 10 : 15;
+        const int half = u / per, g = u - half * per;
+        const int s = 29 * half + nsym * g, G = min(nsym, 29 - nsym * g);   // first data symbol of the group, its size
+        const int sym0 = s + (s < 29 ? 7 : 14);
+        float *out = raw + set * kLdpcN + 3 * s;
+        if (G == 3) group_llrs<3>(C, sym0, lane, out);
+        else if (G == 2) group_llrs<2>(C, sym0, lane, out);
+        else group_llrs<1>(C, sym0, lane, out);
+    }
+    __syncthreads();
+    if (warp < 2) {
+        double e = 0.0;
+        for (int q = lane; q < kNsym * 8; q += 32) e += (double)P[q];
+        for (int o = 16; o > 0; o >>= 1) e += __shfl_xor_sync(0xffffffffu, e, o);
+        const float *l = raw + warp * kLdpcN;
+        double sum = 0.0, sum2 = 0.0;
+        for (int i = lane; i < kLdpcN; i += 32) { sum += l[i]; sum2 += (double)l[i] * l[i]; }
+        for (int o = 16; o > 0; o >>= 1) {
+            sum += __shfl_xor_sync(0xffffffffu, sum, o);
+            sum2 += __shfl_xor_sync(0xffffffffu, sum2, o);
+        }
+        const double var = (sum2 - sum * sum / 174.0) / 174.0;
+        const double scale = sqrt(24.0 / var);
+        float *dst = (warp ? a.llr_c : a.llr_b) + oidx * kLdpcN;
+        for (int i = lane; i < kLdpcN; i += 32) dst[i] = e > 0.0 ? (float)(l[i] * scale) : __int_as_float(0x7fc00000);
+    }
+}
+
 // one candidate, the whole CTA
+template <bool kDeep>
 __device__ void finesync_one(const FsArgs &a, size_t oidx, int slot, const float2 *w, float2 *xs, float2 *rs, float2 *bs, double *metric,
                              float *P, int *pick) {
     const int tid = threadIdx.x;
@@ -168,6 +239,7 @@ __device__ void finesync_one(const FsArgs &a, size_t oidx, int slot, const float
             float re = 0.0f, im = 0.0f;
             for (int c = 0; c < 32; ++c) { re += sp[tid * 32 + c].x; im += sp[tid * 32 + c].y; }
             P[k * 8 + tid] = (float)((double)re * re + (double)im * im);
+            if (kDeep) bs[kSym + 256 + k * 8 + tid] = cmul_conj(make_float2(re, im), tone(f, kSym * k));   // c'[k][tid]
         }
     }
     __syncthreads();
@@ -203,9 +275,12 @@ __device__ void finesync_one(const FsArgs &a, size_t oidx, int slot, const float
             for (int i = 0; i < 3; ++i) out[3 * s + i] = e > 0.0 ? (float)(l[r][i] * scale) : __int_as_float(0x7fc00000);
         }
     }
+    // c' sits behind tw and sp in bs, the raw LLRs of sets b and c in metric: both dead by now
+    if (kDeep) deep_sets(a, oidx, bs + kSym + 256, P, reinterpret_cast<float *>(metric));
 }
 
 // one CTA per candidate left at stage 1 or 2; a persistent grid whose CTAs pull entries from *a.next (zeroed by the caller)
+template <bool kDeep>
 __global__ void __launch_bounds__(kThreads) finesync_kernel(const FsArgs a) {
     __shared__ float2 w[kDfPoints * kRow];
     __shared__ float2 xs[kCoarseSpan + kCoarseSpan / 8];
@@ -223,10 +298,28 @@ __global__ void __launch_bounds__(kThreads) finesync_kernel(const FsArgs a) {
         const int slot = (int)(oidx / (size_t)a.max_cand), c = (int)(oidx - (size_t)slot * a.max_cand);
         const int stage = a.stage[oidx];
         __syncthreads();   // the previous item's shared state is no longer read; w is written
-        if (c < a.ncand[slot] && (stage == 1 || stage == 2)) finesync_one(a, oidx, slot, w, xs, rs, bs, metric, P, pick);
+        if (c < a.ncand[slot] && (stage == 1 || stage == 2)) finesync_one<kDeep>(a, oidx, slot, w, xs, rs, bs, metric, P, pick);
         if (threadIdx.x == 0) s_item = gridDim.x + atomicAdd(a.next, 1u);
         __syncthreads();
         item = s_item;
+    }
+}
+
+// Deep mode: folds the flag / hard rows of the retries on the refined sets into the candidate's fs / fs_hard and fs_how.  Step i
+// (0 ... 7: OSD and AP on set a, then BP, OSD and AP on set b and on set c) has its rows at flag / hard + i * n and ran when bit i of
+// `steps` is set.  At most one step accepts (each runs only on what the ones before left at stage 1 or 2).
+__global__ void finesync_merge_kernel(size_t n, unsigned int steps, const uint8_t *flag, const int32_t *hard, uint8_t *fs, int32_t *fs_hard,
+                                      uint8_t *how) {
+    for (size_t e = (size_t)blockIdx.x * blockDim.x + threadIdx.x; e < n; e += (size_t)gridDim.x * blockDim.x) {
+        uint8_t h = fs[e] == 2 ? 1 : 0;
+        for (int i = 0; i < 8; ++i) {
+            if (((steps >> i) & 1u) && flag[i * n + e] == 2) {
+                fs[e] = 2;
+                fs_hard[e] = hard[i * n + e];
+                h = (uint8_t)(2 + i);
+            }
+        }
+        how[e] = h;
     }
 }
 
@@ -240,14 +333,25 @@ cudaError_t upload_finesync_tables() {
     return e;
 }
 
-cudaError_t launch_finesync(int n_slots, int max_cand, int on, const float *d_xi, const float *d_xq, const candidate_t *d_cand, const int *d_ncand,
-                            const uint8_t *d_stage, float *d_llr, int32_t *d_grid, const uint32_t *d_work, const unsigned int *d_work_total,
-                            unsigned int *d_next, int sm_count, cudaStream_t st, int *launches) {
-    const FsArgs a = {n_slots, max_cand, on, d_xi, d_xq, d_cand, d_ncand, d_stage, d_llr, d_grid, d_work, d_work_total, d_next};
+cudaError_t launch_finesync(int n_slots, int max_cand, int on, int deep, const float *d_xi, const float *d_xq, const candidate_t *d_cand,
+                            const int *d_ncand, const uint8_t *d_stage, float *d_llr, float *d_llr_b, float *d_llr_c, int32_t *d_grid,
+                            const uint32_t *d_work, const unsigned int *d_work_total, unsigned int *d_next, int sm_count, cudaStream_t st,
+                            int *launches) {
+    const FsArgs a = {n_slots, max_cand, on, d_xi, d_xq, d_cand, d_ncand, d_stage, d_llr, d_grid, d_work, d_work_total, d_next, d_llr_b, d_llr_c};
     // persistent grid, 4 CTAs per SM it may use; a CTA skips the entries at stage 3 or 4 and pulls the next
     size_t blocks = (size_t)n_slots * max_cand;
     if (sm_count > 0 && blocks > (size_t)(4 * sm_count)) blocks = (size_t)(4 * sm_count);
-    finesync_kernel<<<(unsigned)blocks, kThreads, 0, st>>>(a);
+    if (deep) finesync_kernel<true><<<(unsigned)blocks, kThreads, 0, st>>>(a);
+    else finesync_kernel<false><<<(unsigned)blocks, kThreads, 0, st>>>(a);
+    ++*launches;
+    return cudaGetLastError();
+}
+
+cudaError_t launch_finesync_merge(size_t n, unsigned int steps, const uint8_t *d_flag, const int32_t *d_hard, uint8_t *d_fs, int32_t *d_fs_hard,
+                                  uint8_t *d_how, int sm_count, cudaStream_t st, int *launches) {
+    size_t blocks = (n + 255) / 256;
+    if (sm_count > 0 && blocks > (size_t)(8 * sm_count)) blocks = (size_t)(8 * sm_count);
+    finesync_merge_kernel<<<(unsigned)blocks, 256, 0, st>>>(n, steps, d_flag, d_hard, d_fs, d_fs_hard, d_how);
     ++*launches;
     return cudaGetLastError();
 }

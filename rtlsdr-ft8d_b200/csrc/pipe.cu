@@ -475,6 +475,11 @@ int ft8b200_pipe_set_finesync(ft8b200_pipe_t *p, int on, int max_hard_errors) {
     return set_lanes(p, __func__, [&](ft8b200_ctx_t *c) { return ft8b200_set_finesync(c, on, max_hard_errors); });
 }
 
+int ft8b200_pipe_set_finesync_deep(ft8b200_pipe_t *p, int on, int max_hard_errors) {
+    if (!p || (on != 0 && on != 1)) return FT8B200_BAD_ARG();
+    return set_lanes(p, __func__, [&](ft8b200_ctx_t *c) { return ft8b200_set_finesync_deep(c, on, max_hard_errors); });
+}
+
 int ft8b200_pipe_set_passes(ft8b200_pipe_t *p, int passes) {
     if (!p) return FT8B200_BAD_ARG();
     if (passes < 1 || passes > 3) return pfail(p, FT8B200_EINVAL, "ft8b200_pipe_set_passes: passes must be 1, 2 or 3");
